@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (libr2s.so through its C ABI)
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host cores (CPU oracle port)
+    python bench.py --gpus 1 --steps K --dump-outputs DIR     # also write the results of the last timed step to DIR/*.npy
 
 Workload (BASELINE.json configs[4], SURVEY.md 8d-5): synthetic n^3 HEX8 SIMP density field (n = 256), grid step h_e/2,
 rho_t = 0.5, remove_artifacts, rbf_interp, rbf_grid = :fine  ->  (2(2n+6)+1)^3 = 1037^3 fine voxels.
@@ -37,6 +38,21 @@ B_PER_FINE_VOXEL = 4.5          # fine evaluation: 4 B write + 1/8 * 4 B weight 
 FMA_PER_FINE_VOXEL = 79.75      # mean of the 8 polyphase tap counts (81 + 3*70 + 3*80 + 88) / 8
 B_PER_VOXEL_SIGN = 8.0
 B_PER_VOXEL_CC = 4 * 9.0 + 16.0  # 4 label passes x 9 B + the final sdf read-modify-write
+DUMP_BYTES = 48 << 20            # --dump-outputs: data bytes of all files together, well under 64 MB with the .npy headers
+DUMP_SEED = 20240517
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Write each result array of the timed path's last step as out_dir/<name>.npy (its own dtype, float64 or float32).  The arrays
+    share `budget` equally; an array larger than its share is written as the 1-D vector of its values at a fixed, seeded set of flat
+    indices (sorted; the same for every run with the same arguments), so that the outputs of two builds compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays)
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, a.size, share // a.itemsize))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -191,10 +207,12 @@ def run_reference(args):
     step, nt, g = cpu_pipeline(n)
     for _ in range(max(0, min(args.warmup, 1))):
         step()
-    ts = []
-    for _ in range(args.steps):
-        t, nv = step()
+    ts, last = [], {}
+    for k in range(args.steps):
+        t, nv = step(last if k == args.steps - 1 else None)
         ts.append(t)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sdf_dists": last["sdf"].reshape([int(v) + 1 for v in g.N[::-1]]), "fine_sdf": last["fine"]})
     t = float(np.mean(ts))
     sample = "n=%d^3 HEX8 SIMP replica of the workload (%d coarse points, %d fine voxels), full timed region" % (n, g.ngp, nv)
     line = {"impl": "reference", "metric": METRIC, "value": nv / t, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": min(args.warmup, 1),
@@ -333,6 +351,10 @@ def run_gpu(args):
         e1.record(stream)
         barrier()
         ms = e0.elapsed_time(e1)
+        if args.dump_outputs:      # the device results of the last timed step, through the pinned buffers before the e2e leg reuses them
+            c.check(c.lib.r2s_download_sdf(c.h, C.c_void_p(h_sdf.data_ptr())))
+            c.check(c.lib.r2s_download_fine_sdf(c.h, C.c_void_p(h_fine.data_ptr())))
+            dump_outputs(args.dump_outputs, {"sdf_dists": h_sdf.numpy().reshape([int(v) + 1 for v in grid.N[::-1]]), "fine_sdf": h_fine.numpy().reshape(fdims[::-1])})
         # ---- e2e: the same K steps through the host-buffer entry point ----
         step_e2e()
         barrier()
@@ -490,7 +512,13 @@ def main():
     ap.add_argument("--pipelined-e2e", action="store_true", default=True, help="also time the pipelined host-buffer calls (r2s_pipeline_slab_begin/_wait) -> e2e_pipelined (default)")
     ap.add_argument("--no-pipelined-e2e", action="store_true", help="skip the pipelined host-buffer leg")
     ap.add_argument("--no-balance", action="store_true", help="keep equal plane counts per slab (no cost-based re-cut during warm-up)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write sdf_dists.npy (float64) and fine_sdf.npy (float32) of the last timed step to DIR; "
+                    "an output too large for %d MiB in all is written as a fixed, seeded sample of its values" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1:
+        ap.error("--dump-outputs needs --gpus 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)
