@@ -14,6 +14,7 @@
 #include "r2s_common.cuh"
 #include "r2s_tables.cuh"
 #include "r2s_p2p.cuh"
+#include "r2s_volq.cuh"
 
 // ------------------------------------------------------------------------------------------------ process_vector (:15-22)
 __global__ void __launch_bounds__(256) k_to_f32(i64 n, i64 v0, int nx, int px, const double *__restrict__ sdf, float *__restrict__ s, unsigned *__restrict__ maxbits) {
@@ -378,52 +379,9 @@ __global__ void __launch_bounds__(256) k_minmax(i64 n, int nx, int px, const flo
 static inline float ordered_to_float(unsigned b) { b = (b & 0x80000000u) ? (b & 0x7fffffffu) : ~b; float f; memcpy(&f, &b, 4); return f; }
 
 // ------------------------------------------------------------------------------------------------ volume (CalcVolumeFromSDF.jl:26-125)
-// pass 1: classify cells of (sdf - th): full cells counted, cut cells appended to a list.  Grid-stride; counts are
-// aggregated per block (one atomic per block for the full cells, one per block-iteration for the list slots).
-__global__ void __launch_bounds__(256) k_vol_classify(int nx, int ny, int nz, int px, const float *__restrict__ sdf, float th, float iso, u64 *__restrict__ acc,
-                                                      int *__restrict__ cutlist, int cutcap) {
-  __shared__ int s_warp[8]; __shared__ int s_base;
-  const i64 ncell = (i64)(nx - 1) * (ny - 1) * (nz - 1), sxy = (i64)px * ny;      // px = row pitch of the field (>= nx)
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int nfull = 0;
-  for (i64 c0 = (i64)blockIdx.x * 256; c0 < ncell; c0 += (i64)gridDim.x * 256) {
-    i64 c = c0 + threadIdx.x; bool cut = false;
-    if (c < ncell) {
-      int i = (int)(c % (nx - 1)), j = (int)((c / (nx - 1)) % (ny - 1)), k = (int)(c / ((i64)(nx - 1) * (ny - 1)));
-      i64 b = ((i64)k * ny + j) * px + i;
-      float v0 = sdf[b] - th, v1 = sdf[b + 1] - th, v2 = sdf[b + px] - th, v3 = sdf[b + px + 1] - th;
-      float v4 = sdf[b + sxy] - th, v5 = sdf[b + sxy + 1] - th, v6 = sdf[b + sxy + px] - th, v7 = sdf[b + sxy + px + 1] - th;
-      float mn = fminf(fminf(fminf(v0, v1), fminf(v2, v3)), fminf(fminf(v4, v5), fminf(v6, v7)));
-      float mx = fmaxf(fmaxf(fmaxf(v0, v1), fmaxf(v2, v3)), fmaxf(fmaxf(v4, v5), fmaxf(v6, v7)));
-      if (!(mx < iso)) { if (mn >= iso) nfull++; else cut = true; }
-    }
-    unsigned mc = __ballot_sync(0xffffffffu, cut);
-    if (__syncthreads_or(mc != 0)) {
-      if (lane == 0) s_warp[warp] = __popc(mc);
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        int tot = 0;
-        for (int w = 0; w < 8; w++) { int t = s_warp[w]; s_warp[w] = tot; tot += t; }
-        s_base = (int)atomicAdd(&acc[1], (u64)tot);
-      }
-      __syncthreads();
-      if (cut) { int slot = s_base + s_warp[warp] + __popc(mc & ((1u << lane) - 1)); if (slot < cutcap) cutlist[slot] = (int)c; }
-      __syncthreads();
-    }
-  }
-  for (int o = 16; o > 0; o >>= 1) nfull += __shfl_down_sync(0xffffffffu, nfull, o);
-  __syncthreads();
-  if (lane == 0) s_warp[warp] = nfull;
-  __syncthreads();
-  if (threadIdx.x == 0) { int tot = 0; for (int w = 0; w < 8; w++) tot += s_warp[w]; if (tot) atomicAdd(&acc[0], (u64)tot); }
-}
 // pass 2: ONE THREAD per cut cell (grid-stride over the list; the count is read from device memory so that no host round
-// trip separates the two passes).  The two inner Gauss loops are fully unrolled with the abscissae / weights as kernel-parameter
-// (constant-bank) operands: 4 lerps per xi, 2 per (xi, eta), then per point one lerp, one compare and one predicated add --
-// about 3 instructions per Gauss point.  The point values follow the reference's lerp order (xi, then eta, then zeta;
-// CalcVolumeFromSDF.jl:88-103).  The cell's Float32 sum of w_i w_j w_k over inside points (iq outer, kq
-// inner, a fixed order) is accumulated across cells as a 2^-37 fixed-point integer (deterministic).
-struct GaussF { float x[9]; float w[9]; };
+// trip separates the two passes); cut_cell_quad9 (r2s_volq.cuh) does the 729 points.  The cell's Float32 sum is accumulated across
+// cells as a 2^-37 fixed-point integer (deterministic).
 __global__ void __launch_bounds__(128) k_vol_cut(int nx, int ny, int px, const float *__restrict__ sdf, float th, float iso, const int *__restrict__ cutlist, int cutcap,
                                                  GaussF G, u64 *__restrict__ acc) {
   const int ncut = (int)min((u64)cutcap, acc[1]);
@@ -436,29 +394,9 @@ __global__ void __launch_bounds__(128) k_vol_cut(int nx, int ny, int px, const f
       const i64 c = cutlist[idx];
       const int i = (int)(c % (nx - 1)), j = (int)((c / (nx - 1)) % (ny - 1)), k = (int)(c / ((i64)(nx - 1) * (ny - 1)));
       const i64 b = ((i64)k * ny + j) * px + i;
-      const float c000 = sdf[b] - th, c100 = sdf[b + 1] - th, c010 = sdf[b + px] - th, c110 = sdf[b + px + 1] - th;
-      const float c001 = sdf[b + sxy] - th, c101 = sdf[b + sxy + 1] - th, c011 = sdf[b + sxy + px] - th, c111 = sdf[b + sxy + px + 1] - th;
-      float part = 0.0f;
-#pragma unroll 1      // the 81-point inner body stays unrolled; unrolling all 729 points (60 KB of code) thrashed the instruction cache
-      for (int iq = 0; iq < 9; iq++) {
-        const float xi = (G.x[iq] + 1) / 2, xm = 1.0f - xi;
-        const float c00 = c000 * xm + c100 * xi, c01 = c001 * xm + c101 * xi;
-        const float c10 = c010 * xm + c110 * xi, c11 = c011 * xm + c111 * xi;
-#pragma unroll
-        for (int jq = 0; jq < 9; jq++) {
-          const float eta = (G.x[jq] + 1) / 2, em = 1.0f - eta;
-          const float c0 = c00 * em + c10 * eta, c1 = c01 * em + c11 * eta;
-          const float wij = G.w[iq] * G.w[jq], dc = c1 - c0;
-#pragma unroll
-          for (int kq = 0; kq < 9; kq++) {
-            const float zeta = (G.x[kq] + 1) / 2;
-            // the zeta lerp c0 (1 - zeta) + c1 zeta as ONE fma, c0 + (c1 - c0) zeta: 2 FMA-pipe operations per Gauss point instead
-            // of 3 (this kernel is FMA-pipe bound); the two forms differ by Float32 round-off only
-            const float ps = fmaf(dc, zeta, c0);
-            if (ps >= iso) part += wij * G.w[kq];
-          }
-        }
-      }
+      const float cv[8] = {sdf[b] - th, sdf[b + 1] - th, sdf[b + px] - th, sdf[b + px + 1] - th,
+                           sdf[b + sxy] - th, sdf[b + sxy + 1] - th, sdf[b + sxy + px] - th, sdf[b + sxy + px + 1] - th};
+      const float part = cut_cell_quad9<false>(cv, G, iso, nullptr);
       local += (u64)llrint((double)part * 137438953472.0);      // part in [0,8]; 2^37 per unit, exact for a float
     }
   }
@@ -513,8 +451,104 @@ __global__ void __launch_bounds__(128) k_vol_cut_n(int nx, int ny, int px, const
 }
 static GaussF gauss9f() { GaussTab t = gauss_legendre_host(9); GaussF g; for (int i = 0; i < 9; i++) { g.x[i] = (float)t.x[i]; g.w[i] = (float)t.w[i]; } return g; }
 
-// volume of {sdf - th >= iso}; edge = cell edge length (Float32 like the reference)
-static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, int px, float th, float edge, float iso, int order, double *vol) {
+// active cell of the threshold search: id, min / max of its corner values, index of its quadrature record (-1: none yet)
+struct VAct { int id; float mn, mx; int rec; };
+// Whole-grid classification (bisection steps 1-3, the final fine-grid volume, r2s_dev_volume_from_sdf) by PLANE MARCHING: a warp owns a
+// tile of VM_R cell rows x (32 VM_V - 1) cells and marches through VM_Z cell planes.  Lane l holds the values of columns
+// x0 + VM_V l .. x0 + VM_V l + VM_V - 1 of the VM_R + 1 rows; per plane it forms the y-pair min / max of each column, and a cell's
+// min / max over its 8 corners is that of its two columns (the right one of the lane's last cell comes from lane + 1 by shuffle) in
+// planes k and k + 1.  Plane k + 1 of one layer is plane k of the next, so every value is loaded once per tile (rows shared by two
+// tiles twice) and the next plane is loaded while the current one is classified.  The last lane's last cell has no right column: tiles
+// overlap by one column.  Cell ids, counts and lists are those of a cell-by-cell pass; only the order of the lists differs.
+// Cells of planes [kc0, kc1) are classified (values of plane kc1 are read: the halo plane of a slab).  Cut cells go to cutlist, (EMIT) cells
+// the remaining bracket [lo, hi] can still cut go to the active list; cells that are full for every threshold still to come are counted in
+// acc[3].
+#define VM_V 2
+#define VM_R 4
+#define VM_Z 32
+template <bool EMIT>
+__global__ void __launch_bounds__(256) k_vol_march(int nx, int ny, int px, int kc0, int kc1, const float *__restrict__ sdf, float lo, float hi, float th, VAct *__restrict__ list_out,
+                                                   u64 *__restrict__ n_out_ptr, i64 list_cap, u64 *__restrict__ acc, int *__restrict__ cutlist, int cutcap) {
+  __shared__ int s_cut[8][WS_CAP];
+  __shared__ VAct s_keep[EMIT ? 8 : 1][EMIT ? WS_CAP : 1];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  constexpr int TXC = 32 * VM_V - 1;
+  const int ntx = (nx - 2 + TXC) / TXC, nty = (ny - 2 + VM_R) / VM_R, ntz = (kc1 - kc0 + VM_Z - 1) / VM_Z;
+  const i64 ntile = (i64)ntx * nty * ntz, pl = (i64)px * ny;
+  int nfull = 0, nperm = 0, ncq = 0, nkq = 0;
+  for (i64 tile = (i64)blockIdx.x * 8 + warp; tile < ntile; tile += (i64)gridDim.x * 8) {      // warp-uniform
+    const int tx = (int)(tile % ntx), ty = (int)((tile / ntx) % nty), tz = (int)(tile / ((i64)ntx * nty));
+    const int x0 = tx * TXC, xl = x0 + VM_V * lane, j0 = ty * VM_R, k0 = kc0 + tz * VM_Z, k1 = min(k0 + VM_Z, kc1);
+    bool vin[VM_R + 1][VM_V];
+    int off[VM_R + 1][VM_V];
+#pragma unroll
+    for (int r = 0; r <= VM_R; r++)
+#pragma unroll
+      for (int u = 0; u < VM_V; u++) { vin[r][u] = xl + u < nx && j0 + r < ny; off[r][u] = (j0 + r) * px + xl + u; }
+    auto load = [&](int k, float (&v)[VM_R + 1][VM_V]) {
+      const float *p = sdf + (i64)k * pl;
+#pragma unroll
+      for (int r = 0; r <= VM_R; r++)
+#pragma unroll
+        for (int u = 0; u < VM_V; u++) v[r][u] = vin[r][u] ? p[off[r][u]] : 0.0f;
+    };
+    float v[VM_R + 1][VM_V], amn[VM_R][VM_V], amx[VM_R][VM_V];
+    load(k0, v);
+#pragma unroll
+    for (int r = 0; r < VM_R; r++)
+#pragma unroll
+      for (int u = 0; u < VM_V; u++) { amn[r][u] = fminf(v[r][u], v[r + 1][u]); amx[r][u] = fmaxf(v[r][u], v[r + 1][u]); }
+    load(k0 + 1, v);
+    for (int k = k0; k < k1; k++) {
+      float bmn[VM_R][VM_V], bmx[VM_R][VM_V];
+#pragma unroll
+      for (int r = 0; r < VM_R; r++)
+#pragma unroll
+        for (int u = 0; u < VM_V; u++) { bmn[r][u] = fminf(v[r][u], v[r + 1][u]); bmx[r][u] = fmaxf(v[r][u], v[r + 1][u]); }
+      if (k + 2 <= k1) load(k + 2, v);      // plane k + 2 is in flight while plane k's cells are classified
+#pragma unroll
+      for (int r = 0; r < VM_R; r++) {
+        const int j = j0 + r;
+        float cmn[VM_V + 1], cmx[VM_V + 1];      // column min / max over the cell layer's 4 values; [VM_V] = lane + 1's first column
+#pragma unroll
+        for (int u = 0; u < VM_V; u++) { cmn[u] = fminf(amn[r][u], bmn[r][u]); cmx[u] = fmaxf(amx[r][u], bmx[r][u]); }
+        cmn[VM_V] = __shfl_down_sync(0xffffffffu, cmn[0], 1); cmx[VM_V] = __shfl_down_sync(0xffffffffu, cmx[0], 1);
+        const int cbase = (k * (ny - 1) + j) * (nx - 1);
+#pragma unroll
+        for (int u = 0; u < VM_V; u++) {
+          const int i = xl + u;
+          bool cut = false, keep = false;
+          const float mn = fminf(cmn[u], cmn[u + 1]), mx = fmaxf(cmx[u], cmx[u + 1]);
+          if (i < nx - 1 && j < ny - 1 && (lane < 31 || u < VM_V - 1)) {
+            if (EMIT && mn >= hi) nperm++;
+            else if (EMIT && mx < lo) {}
+            else {
+              keep = EMIT;
+              if (!(mx < th)) { if (mn >= th) nfull++; else cut = true; }
+            }
+          }
+          ws_push<int>(s_cut[warp], ncq, cut, cbase + i, cutlist, &acc[1], (i64)cutcap, lane);
+          if (EMIT) { VAct e; e.id = cbase + i; e.mn = mn; e.mx = mx; e.rec = -1; ws_push<VAct>(s_keep[warp], nkq, keep, e, list_out, n_out_ptr, list_cap, lane); }
+        }
+#pragma unroll
+        for (int u = 0; u < VM_V; u++) { amn[r][u] = bmn[r][u]; amx[r][u] = bmx[r][u]; }
+      }
+    }
+  }
+  ws_flush<int>(s_cut[warp], ncq, cutlist, &acc[1], (i64)cutcap, lane);
+  if (EMIT) ws_flush<VAct>(s_keep[warp], nkq, list_out, n_out_ptr, list_cap, lane);
+  for (int o = 16; o > 0; o >>= 1) { nfull += __shfl_down_sync(0xffffffffu, nfull, o); nperm += __shfl_down_sync(0xffffffffu, nperm, o); }
+  if (lane == 0) { if (nfull) atomicAdd(&acc[0], (u64)nfull); if (nperm) atomicAdd(&acc[3], (u64)nperm); }
+}
+template <bool EMIT>
+static void vol_march(cudaStream_t st, int nx, int ny, int px, int kc0, int kc1, const float *sdf, float lo, float hi, float th, VAct *list_out, u64 *n_out_ptr, i64 list_cap, u64 *acc,
+                      int *cutlist, int cutcap) {
+  const i64 ntile = (i64)((nx - 2 + 32 * VM_V - 1) / (32 * VM_V - 1)) * ((ny - 2 + VM_R) / VM_R) * ((kc1 - kc0 + VM_Z - 1) / VM_Z);
+  const int grid = (int)std::min<i64>(std::max<i64>(cdiv(ntile, 8), 1), 148 * 16);
+  k_vol_march<EMIT><<<grid, 256, 0, st>>>(nx, ny, px, kc0, kc1, sdf, lo, hi, th, list_out, n_out_ptr, list_cap, acc, cutlist, cutcap);
+}
+// volume of {sdf >= iso}; edge = cell edge length (Float32 like the reference)
+static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, int px, float edge, float iso, int order, double *vol) {
   cudaStream_t st = ctx->stream;
   i64 ncell = (i64)(nx - 1) * (ny - 1) * (nz - 1);
   if (ncell >= (1ll << 31)) FAIL("calculate_volume_from_sdf: grid too large for 32-bit cell ids");
@@ -524,12 +558,12 @@ static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, in
   for (int attempt = 0; attempt < 2; attempt++) {
     int cutcap = (int)(ctx->cutlist.cap / sizeof(int));
     CK(cudaMemsetAsync(acc, 0, sizeof(u64) * 4, st));
-    k_vol_classify<<<min(cdiv(ncell, 256), 148 * 16), 256, 0, st>>>(nx, ny, nz, px, sdf, th, iso, acc, ctx->cutlist.as<int>(), cutcap); LAUNCH_CHECK();
-    if (order == 9) k_vol_cut<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, th, iso, ctx->cutlist.as<int>(), cutcap, G9, acc);
+    vol_march<false>(st, nx, ny, px, 0, nz - 1, sdf, iso, iso, iso, nullptr, nullptr, 0, acc, ctx->cutlist.as<int>(), cutcap); LAUNCH_CHECK();
+    if (order == 9) k_vol_cut<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, 0.0f, iso, ctx->cutlist.as<int>(), cutcap, G9, acc);
     else {
       GaussTab t = gauss_legendre_host(order); GaussNF G; G.n = order;
       for (int q = 0; q < 32; q++) { G.x[q] = q < order ? (float)t.x[q] : 0.0f; G.w[q] = q < order ? (float)t.w[q] : 0.0f; }
-      k_vol_cut_n<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, th, iso, ctx->cutlist.as<int>(), cutcap, G, acc);
+      k_vol_cut_n<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, 0.0f, iso, ctx->cutlist.as<int>(), cutcap, G, acc);
     }
     LAUNCH_CHECK();
     u64 h[3];
@@ -544,63 +578,18 @@ static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, in
   }
   FAIL("calculate_volume_from_sdf: cut-cell list overflow");
 }
-// active cell of the threshold search: id, min / max of its corner values, index of its quadrature record (-1: none yet)
-struct VAct { int id; float mn, mx; int rec; };
-// Whole-grid classification (bisection steps 1-3 and the final fine-grid volume): a warp owns cell ROWS; per 31-cell segment every lane
-// loads the 4 values of its x-column (coalesced) and takes the neighbouring column's min / max from lane + 1, so a cell costs 4 loads
-// instead of 8; the row index arithmetic is done once per row.  Cut cells go to cutlist, (EMIT) cells the remaining bracket [lo, hi]
-// can still cut go to the active list; cells that are full for every threshold still to come are counted in acc[3].
-template <bool EMIT>
-__global__ void __launch_bounds__(256) k_vol_rows(int nx, int ny, int px, int kc0, int kc1, const float *__restrict__ sdf, float lo, float hi, float th, VAct *__restrict__ list_out,
-                                                  u64 *__restrict__ n_out_ptr, i64 list_cap, u64 *__restrict__ acc, int *__restrict__ cutlist, int cutcap) {
-  __shared__ int s_cut[8][WS_CAP];
-  __shared__ VAct s_keep[EMIT ? 8 : 1][EMIT ? WS_CAP : 1];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int nrow = (ny - 1) * (kc1 - kc0);
-  const i64 sxy = (i64)px * ny;
-  int nfull = 0, nperm = 0, ncq = 0, nkq = 0;
-  for (int row = blockIdx.x * 8 + warp; row < nrow; row += gridDim.x * 8) {      // warp-uniform
-    const int j = row % (ny - 1), k = kc0 + row / (ny - 1);
-    const i64 b0 = ((i64)k * ny + j) * px; const int c0 = (k * (ny - 1) + j) * (nx - 1);
-    for (int i0 = 0; i0 < nx - 1; i0 += 31) {
-      const int i = i0 + lane;
-      bool cut = false, keep = false;
-      float cmn = INFINITY, cmx = -INFINITY;
-      if (i < nx) {
-        const i64 b = b0 + i;
-        const float v0 = sdf[b], v1 = sdf[b + px], v2 = sdf[b + sxy], v3 = sdf[b + sxy + px];
-        cmn = fminf(fminf(v0, v1), fminf(v2, v3)); cmx = fmaxf(fmaxf(v0, v1), fmaxf(v2, v3));
-      }
-      const float nmn = __shfl_down_sync(0xffffffffu, cmn, 1), nmx = __shfl_down_sync(0xffffffffu, cmx, 1);
-      float mn = 0.f, mx = 0.f;
-      if (lane < 31 && i < nx - 1) {
-        mn = fminf(cmn, nmn); mx = fmaxf(cmx, nmx);
-        if (EMIT && mn >= hi) nperm++;
-        else if (EMIT && mx < lo) {}
-        else {
-          keep = EMIT;
-          if (!(mx < th)) { if (mn >= th) nfull++; else cut = true; }
-        }
-      }
-      ws_push<int>(s_cut[warp], ncq, cut, c0 + i, cutlist, &acc[1], (i64)cutcap, lane);
-      if (EMIT) { VAct e; e.id = c0 + i; e.mn = mn; e.mx = mx; e.rec = -1; ws_push<VAct>(s_keep[warp], nkq, keep, e, list_out, n_out_ptr, list_cap, lane); }
-    }
-  }
-  ws_flush<int>(s_cut[warp], ncq, cutlist, &acc[1], (i64)cutcap, lane);
-  if (EMIT) ws_flush<VAct>(s_keep[warp], nkq, list_out, n_out_ptr, list_cap, lane);
-  for (int o = 16; o > 0; o >>= 1) { nfull += __shfl_down_sync(0xffffffffu, nfull, o); nperm += __shfl_down_sync(0xffffffffu, nperm, o); }
-  if (lane == 0) { if (nfull) atomicAdd(&acc[0], (u64)nfull); if (nperm) atomicAdd(&acc[3], (u64)nperm); }
-}
 // ---- bisection steps >= 4: the ACTIVE list carries everything a cell needs ------------------------------------------------------
 // After three whole-grid steps only the cells that the remaining bracket [lo, hi] can still cut are active (a thin shell around the
 // level set).  The active list holds 16 bytes per cell (id, min / max of its corners, record index); a cell that is cut for the first time
-// gets a 48-byte RECORD: its eight corner values (gathered once) and a CACHE of its last quadrature: part (the Float32 sum of w_i w_j w_k over the inside Gauss points),
-// the threshold it was computed at and a margin = the smallest |value| over the 729 Gauss points minus a bound on the Float32
+// gets a RECORD: its eight corner values (32 bytes, gathered once, read only by k_vl_eval) and, in a separate 16-byte array with the same
+// index, a CACHE of its last quadrature: part (the Float32 sum of w_i w_j w_k over the inside Gauss points), the threshold it was
+// computed at and a margin = the smallest |value| over the 729 Gauss points minus a bound on the Float32
 // round-off of those values.  While |th - th_cached| stays below the margin no Gauss value can change sign, the inside set -- and
 // with it the cell's Float32 sum, bit for bit -- is the same, and the cached sum is added without re-evaluating the cell.  As the
 // bracket halves, almost every cell freezes: the 40 bisections cost about a dozen full quadratures instead of 40.  The total is an
 // exact integer sum, so the result is bit-identical to re-evaluating every cut cell at every step (R2S_VOL_CACHE=0 does that).
-struct VRec { float c[8]; float part, th_e, margin; int pad; };
+struct VRec { float c[8]; };
+struct VCache { float part, th_e, margin; int pad; };      // one 16-byte load in k_vl_step
 // State of the bisection on the DEVICE (steps >= 4): the bracket update is a one-thread kernel, so the host enqueues all remaining steps
 // without waiting for any of them and reads the result once.  A step whose threshold repeats the previous one (lo and hi adjacent floats)
 // and every step after the stopping rule has fired are skipped by all kernels of the step (skip / skipf).
@@ -627,9 +616,12 @@ __device__ __forceinline__ void bis_end(BisState *S, const u64 *acc, const u64 *
   S->nb++; S->have_prev = 1; S->th_prev = S->th;
   if (!(S->nb < 40 && S->eps > 1.0e-4)) S->done = 1;
 }
-// one thread per active cell: retire / keep (compaction into `out`), classify at th from (mn, mx), use the cached quadrature of the cell's
-// record or queue the cell for k_vl_eval.  acc[6] = records handed out so far.
-__global__ void __launch_bounds__(256) k_vl_step(const BisState *__restrict__ S, VAct *l0, VAct *l1, i64 out_cap, int use_cache, u64 *__restrict__ acc, const VRec *__restrict__ recs,
+// active cells: retire / keep (compaction into `out`), classify at th from (mn, mx), use the cached quadrature of the cell's record or queue
+// the cell for k_vl_eval.  acc[6] = records handed out so far.  The kernel moves little data per cell and is bound by the latency of its
+// two dependent loads (list entry, then cache): a warp takes VL_U x 32 consecutive entries per trip and issues all list loads, then all
+// cache loads, then the appends.
+#define VL_U 4
+__global__ void __launch_bounds__(256) k_vl_step(const BisState *__restrict__ S, VAct *l0, VAct *l1, i64 out_cap, int use_cache, u64 *__restrict__ acc, const VCache *__restrict__ cache,
                                                  int2 *__restrict__ evlist, i64 ev_cap) {
   if (S->skip) return;
   const int icur = S->cur;
@@ -641,45 +633,59 @@ __global__ void __launch_bounds__(256) k_vl_step(const BisState *__restrict__ S,
   const i64 n_in = (i64)*n_in_ptr;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int nfull = 0, nperm = 0, nkq = 0, neq = 0; u64 local = 0;
-  for (i64 t0 = ((i64)blockIdx.x * blockDim.x + (threadIdx.x & ~31)); t0 < n_in; t0 += (i64)gridDim.x * blockDim.x) {      // warp-uniform
-    const i64 t = t0 + lane; bool keep = false, miss = false, fresh = false; VAct e; e.id = 0; e.mn = e.mx = 0.f; e.rec = -1;
-    if (t < n_in) {
-      e = in[t];
-      if (e.mn >= hi) nperm++;                        // full for every threshold still to come
-      else if (e.mx < lo) {}                          // empty for every threshold still to come
-      else {
-        keep = true;
-        if (!(e.mx < th)) {
-          if (e.mn >= th) nfull++;
-          else if (e.rec < 0) { miss = true; fresh = true; }
-          else {
-            const VRec &r = recs[e.rec];
-            if (use_cache && fabsf(th - r.th_e) * 1.00001f < r.margin) local += (u64)llrint((double)r.part * 137438953472.0);
+  for (i64 t0 = ((i64)blockIdx.x * blockDim.x + (threadIdx.x & ~31)) * VL_U; t0 < n_in; t0 += (i64)gridDim.x * blockDim.x * VL_U) {      // warp-uniform
+    VAct e[VL_U];
+#pragma unroll
+    for (int u = 0; u < VL_U; u++) {
+      const i64 t = t0 + u * 32 + lane;
+      if (t < n_in) { const int4 q = __ldcs(reinterpret_cast<const int4 *>(in) + t); e[u].id = q.x; e[u].mn = __int_as_float(q.y); e[u].mx = __int_as_float(q.z); e[u].rec = q.w; }
+      else { e[u].id = 0; e[u].mn = INFINITY; e[u].mx = INFINITY; e[u].rec = -1; }      // beyond the list: counted as permanently full below, then masked
+    }
+    float4 r[VL_U];
+#pragma unroll
+    for (int u = 0; u < VL_U; u++) {
+      r[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+      const bool cached = use_cache && e[u].rec >= 0 && !(e[u].mn >= hi) && !(e[u].mx < lo) && !(e[u].mx < th) && !(e[u].mn >= th);      // the tests below, in the same form
+      if (cached) r[u] = __ldg(reinterpret_cast<const float4 *>(cache) + e[u].rec);
+    }
+#pragma unroll
+    for (int u = 0; u < VL_U; u++) {
+      const bool valid = t0 + u * 32 + lane < n_in;
+      bool keep = false, miss = false, fresh = false;
+      if (valid) {
+        if (e[u].mn >= hi) nperm++;                     // full for every threshold still to come
+        else if (e[u].mx < lo) {}                       // empty for every threshold still to come
+        else {
+          keep = true;
+          if (!(e[u].mx < th)) {
+            if (e[u].mn >= th) nfull++;
+            else if (e[u].rec < 0) { miss = true; fresh = true; }
+            else if (use_cache && fabsf(th - r[u].y) * 1.00001f < r[u].z) local += (u64)llrint((double)r[u].x * 137438953472.0);
             else miss = true;
           }
         }
       }
+      // new records: one claim per warp round (only cells that are cut for the first time)
+      const unsigned mf = __ballot_sync(0xffffffffu, fresh);
+      if (mf) {
+        int base = 0;
+        if (lane == 0) base = (int)atomicAdd(&acc[6], (u64)__popc(mf));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (fresh) e[u].rec = base + __popc(mf & ((1u << lane) - 1));
+      }
+      ws_push<VAct>(s_keep[warp], nkq, keep, e[u], out, n_out_ptr, out_cap, lane);
+      ws_push<int2>(s_ev[warp], neq, miss, make_int2(e[u].rec | (fresh ? (int)0x80000000 : 0), e[u].id), evlist, &acc[1], ev_cap, lane);
     }
-    // new records: one claim per warp round (only cells that are cut for the first time)
-    const unsigned mf = __ballot_sync(0xffffffffu, fresh);
-    if (mf) {
-      int base = 0;
-      if (lane == 0) base = (int)atomicAdd(&acc[6], (u64)__popc(mf));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      if (fresh) e.rec = base + __popc(mf & ((1u << lane) - 1));
-    }
-    ws_push<VAct>(s_keep[warp], nkq, keep, e, out, n_out_ptr, out_cap, lane);
-    ws_push<int2>(s_ev[warp], neq, miss, make_int2(e.rec | (fresh ? (int)0x80000000 : 0), e.id), evlist, &acc[1], ev_cap, lane);
   }
   ws_flush<VAct>(s_keep[warp], nkq, out, n_out_ptr, out_cap, lane);
   ws_flush<int2>(s_ev[warp], neq, evlist, &acc[1], ev_cap, lane);
   for (int o = 16; o > 0; o >>= 1) { nfull += __shfl_down_sync(0xffffffffu, nfull, o); nperm += __shfl_down_sync(0xffffffffu, nperm, o); local += __shfl_down_sync(0xffffffffu, local, o); }
   if (lane == 0) { if (nfull) atomicAdd(&acc[0], (u64)nfull); if (nperm) atomicAdd(&acc[3], (u64)nperm); if (local) atomicAdd(&acc[2], local); }
 }
-// quadrature of the queued cells at th (same point values, same order of the Float32 sum as k_vol_cut) + their new cache entries; a cell
-// that is cut for the first time gathers its corner values into its record
-__global__ void __launch_bounds__(128) k_vl_eval(const BisState *__restrict__ S, VRec *__restrict__ recs, const int2 *__restrict__ evlist, int nx, int ny, int px, const float *__restrict__ sdf,
-                                                 GaussF G, u64 *__restrict__ acc) {
+// quadrature of the queued cells at th (cut_cell_quad9, as k_vol_cut) + their new cache entries; a cell that is cut for the first time
+// gathers its corner values into its record
+__global__ void __launch_bounds__(128) k_vl_eval(const BisState *__restrict__ S, VRec *__restrict__ recs, VCache *__restrict__ cache, const int2 *__restrict__ evlist, int nx, int ny,
+                                                 int px, const float *__restrict__ sdf, GaussF G, u64 *__restrict__ acc) {
   if (S->skip) return;
   const float th = S->th;
   const int nev = (int)acc[1];
@@ -697,37 +703,21 @@ __global__ void __launch_bounds__(128) k_vl_eval(const BisState *__restrict__ S,
         const i64 b = ((i64)k * ny + j) * px + i;
         c[0] = sdf[b]; c[1] = sdf[b + 1]; c[2] = sdf[b + px]; c[3] = sdf[b + px + 1];
         c[4] = sdf[b + sxy]; c[5] = sdf[b + sxy + 1]; c[6] = sdf[b + sxy + px]; c[7] = sdf[b + sxy + px + 1];
-#pragma unroll
-        for (int a = 0; a < 8; a++) e.c[a] = c[a];
+        float4 *d = reinterpret_cast<float4 *>(e.c);
+        d[0] = make_float4(c[0], c[1], c[2], c[3]); d[1] = make_float4(c[4], c[5], c[6], c[7]);
       } else {
-#pragma unroll
-        for (int a = 0; a < 8; a++) c[a] = e.c[a];
+        const float4 *d = reinterpret_cast<const float4 *>(e.c), a = d[0], b = d[1];
+        c[0] = a.x; c[1] = a.y; c[2] = a.z; c[3] = a.w; c[4] = b.x; c[5] = b.y; c[6] = b.z; c[7] = b.w;
       }
-      const float c000 = c[0] - th, c100 = c[1] - th, c010 = c[2] - th, c110 = c[3] - th;
-      const float c001 = c[4] - th, c101 = c[5] - th, c011 = c[6] - th, c111 = c[7] - th;
-      const float amax = fmaxf(fmaxf(fmaxf(fabsf(c000), fabsf(c100)), fmaxf(fabsf(c010), fabsf(c110))), fmaxf(fmaxf(fabsf(c001), fabsf(c101)), fmaxf(fabsf(c011), fabsf(c111))));
-      float part = 0.0f, m = INFINITY;
-#pragma unroll 1
-      for (int iq = 0; iq < 9; iq++) {
-        const float xi = (G.x[iq] + 1) / 2, xm = 1.0f - xi;
-        const float c00 = c000 * xm + c100 * xi, c01 = c001 * xm + c101 * xi;
-        const float c10 = c010 * xm + c110 * xi, c11 = c011 * xm + c111 * xi;
 #pragma unroll
-        for (int jq = 0; jq < 9; jq++) {
-          const float eta = (G.x[jq] + 1) / 2, em = 1.0f - eta;
-          const float c0 = c00 * em + c10 * eta, c1 = c01 * em + c11 * eta;
-          const float wij = G.w[iq] * G.w[jq], dc = c1 - c0;
-#pragma unroll
-          for (int kq = 0; kq < 9; kq++) {
-            const float ps = fmaf(dc, (G.x[kq] + 1) / 2, c0);
-            if (ps >= 0.0f) part += wij * G.w[kq];
-            m = fminf(m, fabsf(ps));
-          }
-        }
-      }
+      for (int a = 0; a < 8; a++) c[a] = c[a] - th;
+      const float amax = fmaxf(fmaxf(fmaxf(fabsf(c[0]), fabsf(c[1])), fmaxf(fabsf(c[2]), fabsf(c[3]))), fmaxf(fmaxf(fabsf(c[4]), fabsf(c[5])), fmaxf(fabsf(c[6]), fabsf(c[7]))));
+      float m;
+      const float part = cut_cell_quad9<true>(c, G, 0.0f, &m);
       // a Gauss value moves by (th_cached - th) plus Float32 round-off of the corner subtractions and the three lerps: a few ulp of the
       // corner magnitude, bounded generously by 1e-5 * amax (the step test applies the same factor to the threshold difference)
-      e.part = part; e.th_e = th; e.margin = m - 1.0e-5f * amax;
+      VCache w; w.part = part; w.th_e = th; w.margin = m - 1.0e-5f * amax; w.pad = 0;
+      cache[q.x & 0x7fffffff] = w;
       local += (u64)llrint((double)part * 137438953472.0);
     }
   }
@@ -766,7 +756,7 @@ static int vol_bisect_step(r2s_ctx *ctx, VolBisect &vb, float lo, float hi, floa
   static const GaussF G9 = gauss9f();
   const i64 n_all = (i64)(vb.nx - 1) * (vb.ny - 1) * (i64)(vb.kc1 - vb.kc0);
   vb.step++;
-  const bool emit = vb.step == 3;      // steps 1-3 classify the whole grid (k_vol_rows); step 3 also emits the active list (into list 0)
+  const bool emit = vb.step == 3;      // steps 1-3 classify the whole grid (k_vol_march); step 3 also emits the active list (into list 0)
   if (emit) CK(ctx->vent[0].reserve(sizeof(VAct) * (size_t)(n_all + 1)));
   u64 h[6];
   for (int attempt = 0; attempt < 2; attempt++) {
@@ -775,10 +765,8 @@ static int vol_bisect_step(r2s_ctx *ctx, VolBisect &vb, float lo, float hi, floa
     u64 *nout = vb.acc + 4;
     // (a second attempt follows a cut-list overflow: the list has been grown, the step is repeated from scratch)
     if (emit) { CK(cudaMemsetAsync(nout, 0, sizeof(u64), st)); CK(cudaMemsetAsync(vb.acc + 3, 0, sizeof(u64), st)); }      // step 3 is the first step that retires cells
-    const int nrow = (vb.ny - 1) * (vb.kc1 - vb.kc0);
-    const int rgrid = (int)std::min<i64>(std::max<i64>(cdiv(nrow, 8), 1), 148 * 8);
-    if (!emit) k_vol_rows<false><<<rgrid, 256, 0, st>>>(vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, nullptr, nullptr, 0, vb.acc, ctx->cutlist.as<int>(), cutcap);
-    else k_vol_rows<true><<<rgrid, 256, 0, st>>>(vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, ctx->vent[0].as<VAct>(), nout, n_all + 1, vb.acc, ctx->cutlist.as<int>(), cutcap);
+    if (!emit) vol_march<false>(st, vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, nullptr, nullptr, 0, vb.acc, ctx->cutlist.as<int>(), cutcap);
+    else vol_march<true>(st, vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, ctx->vent[0].as<VAct>(), nout, n_all + 1, vb.acc, ctx->cutlist.as<int>(), cutcap);
     LAUNCH_CHECK();
     k_vol_cut<<<148 * 16, 128, 0, st>>>(vb.nx, vb.ny, vb.px, vb.sdf, th, 0.0f, ctx->cutlist.as<int>(), cutcap, G9, vb.acc); LAUNCH_CHECK();
     // cross-rank sum of (full cells, overflow flag, cut sum); integers, so the total does not depend on the slab count
@@ -797,7 +785,7 @@ static int vol_bisect_step(r2s_ctx *ctx, VolBisect &vb, float lo, float hi, floa
     }
     if (emit) {      // step 3: list 0 holds the active cells; room for one record per active cell (only cells that get cut use one)
       vb.cur = 0; vb.n_cur = (i64)h[4];
-      CK(ctx->vrec.reserve(sizeof(VRec) * (size_t)(vb.n_cur + 1)));
+      CK(ctx->vrec.reserve((sizeof(VRec) + sizeof(VCache)) * (size_t)(vb.n_cur + 1)));      // corner records, then the caches
     }
     vb.n_eval += (i64)h[1];
     float ev = vb.edge * vb.edge * vb.edge, jac = ev / 8.0f;
@@ -819,15 +807,16 @@ static int vol_bisect_finish(r2s_ctx *ctx, VolBisect &vb, float &lo, float &hi, 
   h.ev = vb.edge * vb.edge * vb.edge; h.jac = h.ev / 8.0f;
   BisState *S = ctx->bis_state.as<BisState>();
   CK(cudaMemcpyAsync(S, &h, sizeof(h), cudaMemcpyHostToDevice, st));
-  const int grid = (int)std::min<i64>(std::max<i64>(cdiv(vb.n_cur, 256), 1), 148 * 8);
+  const int grid = (int)std::min<i64>(std::max<i64>(cdiv(vb.n_cur, 256 * VL_U), 1), 148 * 8);
+  VRec *recs = ctx->vrec.as<VRec>(); VCache *cache = reinterpret_cast<VCache *>(recs + (vb.n_cur + 1));
   u64 *red = vb.acc + 8;
   ctx->skip_flag = &S->skipf;      // the peer-memory all-reduce of a skipped step skips itself (same flag value on every rank)
   const bool single = ctx->nranks == 1;
   k_bis_turn<<<1, 1, 0, st>>>(S, vb.acc, red, 1); LAUNCH_CHECK();
   for (int step = nb; step < 40; step++) {
     const int next = step + 1 < 40 ? 1 : 0;
-    k_vl_step<<<grid, 256, 0, st>>>(S, ctx->vent[0].as<VAct>(), ctx->vent[1].as<VAct>(), vb.n_cur + 1, ctx->knobs.vol_cache, vb.acc, ctx->vrec.as<VRec>(), ctx->vlist[1].as<int2>(), vb.n_cur + 1); LAUNCH_CHECK();
-    k_vl_eval<<<148 * 16, 128, 0, st>>>(S, ctx->vrec.as<VRec>(), ctx->vlist[1].as<int2>(), vb.nx, vb.ny, vb.px, vb.sdf, G9, vb.acc); LAUNCH_CHECK();
+    k_vl_step<<<grid, 256, 0, st>>>(S, ctx->vent[0].as<VAct>(), ctx->vent[1].as<VAct>(), vb.n_cur + 1, ctx->knobs.vol_cache, vb.acc, cache, ctx->vlist[1].as<int2>(), vb.n_cur + 1); LAUNCH_CHECK();
+    k_vl_eval<<<148 * 16, 128, 0, st>>>(S, recs, cache, ctx->vlist[1].as<int2>(), vb.nx, vb.ny, vb.px, vb.sdf, G9, vb.acc); LAUNCH_CHECK();
     if (single) { k_bis_turn<<<1, 1, 0, st>>>(S, vb.acc, red, 4 | 2 | next); LAUNCH_CHECK(); }
     else {
       k_bis_turn<<<1, 1, 0, st>>>(S, vb.acc, red, 4); LAUNCH_CHECK();
@@ -843,7 +832,7 @@ static int vol_bisect_finish(r2s_ctx *ctx, VolBisect &vb, float &lo, float &hi, 
 int r2s_dev_volume_from_sdf(r2s_ctx *ctx, const float *sdf_dev, i64 nx, i64 ny, i64 nz, float edge, float iso, int order, double *vol) {
   if (order < 1 || order > 32) FAIL("calculate_volume_from_sdf: detailed_quad_order must be between 1 and 32");
   CK(ctx->cutlist.reserve(sizeof(int) * 1024));
-  return volume_dev(ctx, sdf_dev, (int)nx, (int)ny, (int)nz, (int)nx, 0.0f, edge, iso, order, vol);
+  return volume_dev(ctx, sdf_dev, (int)nx, (int)ny, (int)nz, (int)nx, edge, iso, order, vol);
 }
 
 // ------------------------------------------------------------------------------------------------ fine-grid evaluation (:363)
