@@ -6,7 +6,7 @@
 //   * a shared-memory tiled stencil mat-vec fused with the CG vector updates and dot products (HBM-bound),
 //   * an 8-phase polyphase stencil for the evaluation on the :fine grid (taps with |d|^2 <= ln(1000) in half cells),
 //   * a two-pass cut-cell quadrature for the volume-matching bisection (LS_Threshold, :265-300).
-// Sums are deterministic: block partials in fixed slots (double) or 64-bit fixed-point integer atomics.
+// Sums are deterministic: block partials in fixed slots (double) or fixed-point integer atomics (vol_cell_add, r2s_volq.cuh).
 #include <float.h>
 #include <stdlib.h>
 #include <algorithm>
@@ -381,11 +381,26 @@ static inline float ordered_to_float(unsigned b) { b = (b & 0x80000000u) ? (b & 
 // ------------------------------------------------------------------------------------------------ volume (CalcVolumeFromSDF.jl:26-125)
 // pass 2: ONE THREAD per cut cell (grid-stride over the list; the count is read from device memory so that no host round
 // trip separates the two passes); cut_cell_quad9 (r2s_volq.cuh) does the 729 points.  The cell's Float32 sum is accumulated across
-// cells as a 2^-37 fixed-point integer (deterministic).
+// cells as a 2^-37 fixed-point integer (vol_cell_add; deterministic); vol_sum_flush adds the low 32 bits and the rest of the thread sums
+// into acc[2] and acc[7].  One pair of atomics per CTA, not per warp: same-address atomics retire about one per clock, and a second
+// per-warp atomic cost ~10 us per launch of k_vl_step / k_vl_eval (B200).  Called by every thread of the CTA (at most 8 warps).
+__device__ __forceinline__ void vol_sum_flush(u64 local, u64 *__restrict__ acc) {
+  __shared__ u64 s_w[2][8];
+  u64 s[2] = {local & 0xffffffffull, local >> 32};
+  for (int o = 16; o > 0; o >>= 1) { s[0] += __shfl_down_sync(0xffffffffu, s[0], o); s[1] += __shfl_down_sync(0xffffffffu, s[1], o); }
+  if ((threadIdx.x & 31) == 0) { s_w[0][threadIdx.x >> 5] = s[0]; s_w[1][threadIdx.x >> 5] = s[1]; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    u64 a = 0, b = 0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); w++) { a += s_w[0][w]; b += s_w[1][w]; }
+    if (a) atomicAdd(&acc[2], a);
+    if (b) atomicAdd(&acc[7], b);
+  }
+}
 __global__ void __launch_bounds__(128) k_vol_cut(int nx, int ny, int px, const float *__restrict__ sdf, float th, float iso, const int *__restrict__ cutlist, int cutcap,
                                                  GaussF G, u64 *__restrict__ acc) {
   const int ncut = (int)min((u64)cutcap, acc[1]);
-  const int lane = threadIdx.x & 31, nthr = gridDim.x * blockDim.x;
+  const int nthr = gridDim.x * blockDim.x;
   const i64 sxy = (i64)px * ny;
   u64 local = 0;
   for (int base = blockIdx.x * blockDim.x; base < ncut; base += nthr) {      // warp-uniform trip count
@@ -396,12 +411,10 @@ __global__ void __launch_bounds__(128) k_vol_cut(int nx, int ny, int px, const f
       const i64 b = ((i64)k * ny + j) * px + i;
       const float cv[8] = {sdf[b] - th, sdf[b + 1] - th, sdf[b + px] - th, sdf[b + px + 1] - th,
                            sdf[b + sxy] - th, sdf[b + sxy + 1] - th, sdf[b + sxy + px] - th, sdf[b + sxy + px + 1] - th};
-      const float part = cut_cell_quad9<false>(cv, G, iso, nullptr);
-      local += (u64)llrint((double)part * 137438953472.0);      // part in [0,8]; 2^37 per unit, exact for a float
+      vol_cell_add(local, cut_cell_quad9<false>(cv, G, iso, nullptr));
     }
   }
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
-  if (lane == 0 && local) atomicAdd(&acc[2], local);
+  vol_sum_flush(local, acc);
 }
 // ---- LS_Threshold bisection (RBFs4Smoothing.jl:265-300): volume of {lsf - th >= 0} for a SEQUENCE of thresholds ----------
 // V(th) is a sum over cells; a cell's class depends only on (cmin, cmax) = (min, max) of its 8 corner values: full iff
@@ -410,14 +423,15 @@ __global__ void __launch_bounds__(128) k_vol_cut(int nx, int ny, int px, const f
 // cmax < lo stays empty for the rest of the search: such cells are retired (full ones into a permanent counter) and only the
 // remaining "active" cells are carried to the next step in a compacted list.  The sum is accumulated in integers, so the
 // result is bit-identical to re-classifying every cell at every step, at ~3 full passes instead of 40.
-// acc: [0] full cells of this step  [1] cut count  [2] cut fixed-point sum  [3] permanently full  [4],[5] list sizes (ping-pong)
+// acc: [0] full cells of this step  [1] cut count  [2], [7] cut fixed-point sum (vol_sum_flush's two words)  [3] permanently full
+//      [4],[5] list sizes (ping-pong)  [6] records handed out
 // any quadrature order 1..32 (calculate_volume_from_sdf's detailed_quad_order; the convergence tests of the reference use 20): same
 // organisation as k_vol_cut, loops not unrolled, abscissae / weights read from the kernel-parameter bank with uniform indices
 struct GaussNF { float x[32]; float w[32]; int n; };
 __global__ void __launch_bounds__(128) k_vol_cut_n(int nx, int ny, int px, const float *__restrict__ sdf, float th, float iso, const int *__restrict__ cutlist, int cutcap,
                                                    GaussNF G, u64 *__restrict__ acc) {
   const int ncut = (int)min((u64)cutcap, acc[1]);
-  const int lane = threadIdx.x & 31, nthr = gridDim.x * blockDim.x;
+  const int nthr = gridDim.x * blockDim.x;
   const i64 sxy = (i64)px * ny;
   u64 local = 0;
   for (int base = blockIdx.x * blockDim.x; base < ncut; base += nthr) {
@@ -443,11 +457,10 @@ __global__ void __launch_bounds__(128) k_vol_cut_n(int nx, int ny, int px, const
           }
         }
       }
-      local += (u64)llrint((double)part * 137438953472.0);
+      vol_cell_add(local, part);
     }
   }
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
-  if (lane == 0 && local) atomicAdd(&acc[2], local);
+  vol_sum_flush(local, acc);
 }
 static GaussF gauss9f() { GaussTab t = gauss_legendre_host(9); GaussF g; for (int i = 0; i < 9; i++) { g.x[i] = (float)t.x[i]; g.w[i] = (float)t.w[i]; } return g; }
 
@@ -557,7 +570,7 @@ static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, in
   static const GaussF G9 = gauss9f();
   for (int attempt = 0; attempt < 2; attempt++) {
     int cutcap = (int)(ctx->cutlist.cap / sizeof(int));
-    CK(cudaMemsetAsync(acc, 0, sizeof(u64) * 4, st));
+    CK(cudaMemsetAsync(acc, 0, sizeof(u64) * 8, st));
     vol_march<false>(st, nx, ny, px, 0, nz - 1, sdf, iso, iso, iso, nullptr, nullptr, 0, acc, ctx->cutlist.as<int>(), cutcap); LAUNCH_CHECK();
     if (order == 9) k_vol_cut<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, 0.0f, iso, ctx->cutlist.as<int>(), cutcap, G9, acc);
     else {
@@ -566,14 +579,14 @@ static int volume_dev(r2s_ctx *ctx, const float *sdf, int nx, int ny, int nz, in
       k_vol_cut_n<<<148 * 16, 128, 0, st>>>(nx, ny, px, sdf, 0.0f, iso, ctx->cutlist.as<int>(), cutcap, G, acc);
     }
     LAUNCH_CHECK();
-    u64 h[3];
+    u64 h[8];
     if (r2s_readback(ctx, h, acc, sizeof(h))) return 1;
     if ((i64)h[1] > cutcap) {     // the cut list was too small: grow it and redo both passes
       CK(ctx->cutlist.reserve(sizeof(int) * (size_t)(h[1] + h[1] / 2 + 1024)));
       continue;
     }
     float ev = edge * edge * edge, jac = ev / 8.0f;
-    *vol = (double)h[0] * (double)ev + ((double)h[2] / 137438953472.0 /* 2^37 */) * (double)jac;
+    *vol = (double)h[0] * (double)ev + vol_fixed_value(h[2], h[7]) * (double)jac;
     return 0;
   }
   FAIL("calculate_volume_from_sdf: cut-cell list overflow");
@@ -602,12 +615,13 @@ __device__ __forceinline__ void bis_begin(BisState *S, u64 *acc) {
   S->th = th;
   const int skip = (S->have_prev && th == S->th_prev) ? 1 : 0;      // the volume of an identical threshold is not recomputed
   S->skip = skip; S->skipf = skip ? 1.0f : 0.0f;
-  if (!skip) { acc[0] = 0; acc[1] = 0; acc[2] = 0; acc[4 + (1 - S->cur)] = 0; }
+  if (!skip) { acc[0] = 0; acc[1] = 0; acc[2] = 0; acc[7] = 0; acc[4 + (1 - S->cur)] = 0; }
 }
 __device__ __forceinline__ void bis_end(BisState *S, const u64 *acc, const u64 *red) {      // LS_Threshold's loop body after the volume (RBFs4Smoothing.jl:286-296)
   if (S->done) return;
   if (!S->skip) {
-    S->v = (double)red[0] * (double)S->ev + ((double)red[2] / 137438953472.0 /* 2^37 */) * (double)S->jac;
+    // the contraction nvcc chose for the plain expression (full * ev + sum * jac), written out
+    S->v = fma((double)red[0], (double)S->ev, __dmul_rn(vol_fixed_value(red[2], red[3]), (double)S->jac));
     S->cur = 1 - S->cur; S->n_eval += acc[1];
   }
   const float cur = (float)S->v;
@@ -660,7 +674,7 @@ __global__ void __launch_bounds__(256) k_vl_step(const BisState *__restrict__ S,
           if (!(e[u].mx < th)) {
             if (e[u].mn >= th) nfull++;
             else if (e[u].rec < 0) { miss = true; fresh = true; }
-            else if (use_cache && fabsf(th - r[u].y) * 1.00001f < r[u].z) local += (u64)llrint((double)r[u].x * 137438953472.0);
+            else if (use_cache && fabsf(th - r[u].y) * 1.00001f < r[u].z) vol_cell_add(local, r[u].x);
             else miss = true;
           }
         }
@@ -679,8 +693,9 @@ __global__ void __launch_bounds__(256) k_vl_step(const BisState *__restrict__ S,
   }
   ws_flush<VAct>(s_keep[warp], nkq, out, n_out_ptr, out_cap, lane);
   ws_flush<int2>(s_ev[warp], neq, evlist, &acc[1], ev_cap, lane);
-  for (int o = 16; o > 0; o >>= 1) { nfull += __shfl_down_sync(0xffffffffu, nfull, o); nperm += __shfl_down_sync(0xffffffffu, nperm, o); local += __shfl_down_sync(0xffffffffu, local, o); }
-  if (lane == 0) { if (nfull) atomicAdd(&acc[0], (u64)nfull); if (nperm) atomicAdd(&acc[3], (u64)nperm); if (local) atomicAdd(&acc[2], local); }
+  for (int o = 16; o > 0; o >>= 1) { nfull += __shfl_down_sync(0xffffffffu, nfull, o); nperm += __shfl_down_sync(0xffffffffu, nperm, o); }
+  if (lane == 0) { if (nfull) atomicAdd(&acc[0], (u64)nfull); if (nperm) atomicAdd(&acc[3], (u64)nperm); }
+  vol_sum_flush(local, acc);
 }
 // quadrature of the queued cells at th (cut_cell_quad9, as k_vol_cut) + their new cache entries; a cell that is cut for the first time
 // gathers its corner values into its record
@@ -689,7 +704,7 @@ __global__ void __launch_bounds__(128) k_vl_eval(const BisState *__restrict__ S,
   if (S->skip) return;
   const float th = S->th;
   const int nev = (int)acc[1];
-  const int lane = threadIdx.x & 31, nthr = gridDim.x * blockDim.x;
+  const int nthr = gridDim.x * blockDim.x;
   u64 local = 0;
   for (int base = blockIdx.x * blockDim.x; base < nev; base += nthr) {      // warp-uniform trip count
     const int idx = base + threadIdx.x;
@@ -718,16 +733,15 @@ __global__ void __launch_bounds__(128) k_vl_eval(const BisState *__restrict__ S,
       // corner magnitude, bounded generously by 1e-5 * amax (the step test applies the same factor to the threshold difference)
       VCache w; w.part = part; w.th_e = th; w.margin = m - 1.0e-5f * amax; w.pad = 0;
       cache[q.x & 0x7fffffff] = w;
-      local += (u64)llrint((double)part * 137438953472.0);
+      vol_cell_add(local, part);
     }
   }
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_down_sync(0xffffffffu, local, o);
-  if (lane == 0 && local) atomicAdd(&acc[2], local);
+  vol_sum_flush(local, acc);
 }
-// acc -> red for the cross-rank sum: [0] full + permanently full, [1] 1 if this rank's cut list overflowed, [2] cut sum
+// acc -> red for the cross-rank sum: [0] full + permanently full, [1] 1 if this rank's cut list overflowed, [2], [3] cut sum (two words)
 __device__ __forceinline__ void vol_pack(const u64 *__restrict__ acc, int cutcap, u64 *__restrict__ red, const BisState *S) {
   if (S && S->skip) return;
-  red[0] = acc[0] + acc[3]; red[1] = acc[1] > (u64)cutcap ? 1 : 0; red[2] = acc[2]; red[3] = 0;
+  red[0] = acc[0] + acc[3]; red[1] = acc[1] > (u64)cutcap ? 1 : 0; red[2] = acc[2]; red[3] = acc[7];
 }
 __global__ void k_vol_pack(const u64 *__restrict__ acc, int cutcap, u64 *__restrict__ red, const BisState *S) { vol_pack(acc, cutcap, red, S); }
 // the one-thread kernels between two bisection steps, fused: what = 1 begin, 2 end, 4 pack (pack -> [all-reduce] -> end -> begin of the next step)
@@ -761,15 +775,16 @@ static int vol_bisect_step(r2s_ctx *ctx, VolBisect &vb, float lo, float hi, floa
   u64 h[6];
   for (int attempt = 0; attempt < 2; attempt++) {
     int cutcap = (int)(ctx->cutlist.cap / sizeof(int));
-    CK(cudaMemsetAsync(vb.acc, 0, sizeof(u64) * 3, st));
+    // acc[3..6] only come into use at step 3 (it is the first step that retires cells and emits the active list) and after it, in
+    // vol_bisect_finish: all eight words start from zero at every step.  (A second attempt follows a cut-list overflow: the list has been
+    // grown, the step is repeated from scratch.)
+    CK(cudaMemsetAsync(vb.acc, 0, sizeof(u64) * 8, st));
     u64 *nout = vb.acc + 4;
-    // (a second attempt follows a cut-list overflow: the list has been grown, the step is repeated from scratch)
-    if (emit) { CK(cudaMemsetAsync(nout, 0, sizeof(u64), st)); CK(cudaMemsetAsync(vb.acc + 3, 0, sizeof(u64), st)); }      // step 3 is the first step that retires cells
     if (!emit) vol_march<false>(st, vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, nullptr, nullptr, 0, vb.acc, ctx->cutlist.as<int>(), cutcap);
     else vol_march<true>(st, vb.nx, vb.ny, vb.px, vb.kc0, vb.kc1, vb.sdf, lo, hi, th, ctx->vent[0].as<VAct>(), nout, n_all + 1, vb.acc, ctx->cutlist.as<int>(), cutcap);
     LAUNCH_CHECK();
     k_vol_cut<<<148 * 16, 128, 0, st>>>(vb.nx, vb.ny, vb.px, vb.sdf, th, 0.0f, ctx->cutlist.as<int>(), cutcap, G9, vb.acc); LAUNCH_CHECK();
-    // cross-rank sum of (full cells, overflow flag, cut sum); integers, so the total does not depend on the slab count
+    // cross-rank sum of (full cells, overflow flag, the two words of the cut sum); integers, so the total does not depend on the slab count
     u64 *red = vb.acc + 8, hr[4];
     k_vol_pack<<<1, 1, 0, st>>>(vb.acc, cutcap, red, nullptr); LAUNCH_CHECK();
     if (r2s_allreduce(ctx, red, 4, 1)) return 1;
@@ -789,7 +804,7 @@ static int vol_bisect_step(r2s_ctx *ctx, VolBisect &vb, float lo, float hi, floa
     }
     vb.n_eval += (i64)h[1];
     float ev = vb.edge * vb.edge * vb.edge, jac = ev / 8.0f;
-    *vol = (double)hr[0] * (double)ev + ((double)hr[2] / 137438953472.0 /* 2^37 */) * (double)jac;
+    *vol = (double)hr[0] * (double)ev + vol_fixed_value(hr[2], hr[3]) * (double)jac;
     return 0;
   }
   FAIL("LS_Threshold: cut-cell list overflow");

@@ -101,3 +101,21 @@ R2S_HD float cut_cell_quad9(const float c[8], const GaussF &G, float iso, float 
   if (MARGIN) *mabs = m;
   return part;
 }
+
+// The cut-cell sum in fixed point.  A cell's Float32 sum part (in [0, 8]) enters the volume as q = llrint(part * 2^37) < 2^40 (exact for
+// a sum of 9-point Gauss weight products).  A thread adds its cells' q into one 64-bit word (vol_cell_add: fewer than 2^24 cells per
+// thread in every kernel, so it cannot wrap); the kernels then add the low 32 bits and the rest of the thread sums into two separate
+// 64-bit words s0, s1 (vol_sum_flush in r2s_rbf.cu), neither of which wraps below 2^31 cells (s0 < 2^63, s1 < 2^39).  A single word
+// wrapped once the parts added up to 2^27.  The integer sum S = s1 * 2^32 + s0 does not depend on the order of the cells.
+R2S_HD void vol_cell_add(unsigned long long &local, float part) {
+  local += (unsigned long long)llrint((double)part * 137438953472.0 /* 2^37 */);
+}
+// S / 2^37 as a double, rounded once (to nearest, ties to even).  Below 2^64 this is (double)S / 2^37, the value of the single-word sum.
+R2S_HD double vol_fixed_value(unsigned long long s0w, unsigned long long s1w) {
+  const unsigned long long lo = s0w + (s1w << 32), hi = (s1w >> 32) + (lo < s0w ? 1ull : 0ull);      // S = hi * 2^64 + lo
+  if (hi == 0) return (double)lo / 137438953472.0;
+  int sh = 0;
+  while (sh < 64 && (hi >> sh) != 0) sh++;      // S < 2^(64 + sh): keep its top 64 bits, the bits shifted out as a sticky bit
+  const unsigned long long t = (lo >> sh) | (hi << (64 - sh)) | ((lo & ((1ull << sh) - 1)) != 0 ? 1ull : 0ull);
+  return ldexp((double)t, sh - 37);
+}

@@ -524,3 +524,17 @@ def test_threshold_search_cache_is_exact(r2s, monkeypatch):
     for name in ("nocache", "debug"):
         assert res[name][2].th == res["cache"][2].th and res[name][2].volume == res["cache"][2].volume and res[name][2].bisections == res["cache"][2].bisections
         assert np.array_equal(res[name][0], res["cache"][0]) and np.array_equal(res[name][1], res["cache"][1])
+    # a 400^3-cell field on which every cell is cut and the fixed-point sum exceeds 2^64 (tests/test_volume_exact.py), approximation mode
+    from test_volume_exact import rbf_on_grid, wrap_field
+    f, n = wrap_field(400), 400
+    big = {}
+    for name, env in (("cache", {}), ("nocache", {"R2S_VOL_CACHE": "0"})):
+        for k, v in env.items():
+            monkeypatch.setenv(k, v)
+        ctx = r2s.Context()
+        fine, th, vol, rep, _ = rbf_on_grid(r2s, ctx, f, [n, n, n], 1.0, 1, False, 0.5 * n ** 3)
+        big[name] = (fine, th, vol, rep.bisections)
+        ctx.close()
+        for k in env:
+            monkeypatch.delenv(k)
+    assert big["nocache"][1:] == big["cache"][1:] and np.array_equal(big["nocache"][0], big["cache"][0])

@@ -6,6 +6,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import volume_ref
 from fixtures import load_mesh, simp_hex8
 
 pytestmark = pytest.mark.gpu
@@ -20,16 +21,18 @@ def _device_lists():
     return lists
 
 
-@pytest.mark.parametrize("case", ["simp24", "chapadlo"])
+@pytest.mark.parametrize("case", ["simp24", "chapadlo", "simp24_approx"])
 def test_multi_pipeline_matches_single_device(r2s, case, tmp_path):
-    if case == "simp24":
+    if case.startswith("simp24"):
         X, IEN, rho = simp_hex8(24)
-        opts = dict(threshold_density=0.5, sdf_grid_setup="manual", grid_step=0.5, rbf_interp=True, rbf_grid="fine", remove_artifacts=True, artifact_min_component_ratio=0.3)
+        opts = dict(threshold_density=0.5, sdf_grid_setup="manual", grid_step=0.5, rbf_interp=case == "simp24", rbf_grid="fine", remove_artifacts=True,
+                    artifact_min_component_ratio=0.3)
     else:
         X, IEN, rho = load_mesh("chapadlo")
         opts = dict(sdf_grid_setup="automatic", rbf_interp=True, rbf_grid="fine", remove_artifacts=True)
     fine1, fg1, grid1, sdf1, rep1 = r2s.rho2sdf(case, X, IEN, rho, options=r2s.Rho2sdfOptions(**opts), return_report=True)
     scale = max(1.0, float(np.abs(fine1).max()))
+    assert rep1["volume"] == np.float32(volume_ref.reference(fine1, volume_ref.fine_edge(grid1, 2))[2])
     for devs in _device_lists():
         base = str(tmp_path / ("out%d" % len(devs)))
         fine, fg, grid, sdf, rep = r2s.rho2sdf(case, X, IEN, rho, options=r2s.Rho2sdfOptions(**opts), return_report=True, devices=devs, export_vti=base)
@@ -39,6 +42,10 @@ def test_multi_pipeline_matches_single_device(r2s, case, tmp_path):
         # Float32 smoothing: the CG dot products are summed slab by slab, so the fields agree to round-off, not bit for bit
         assert np.max(np.abs(fine - fine1)) <= 1e-5 * scale and abs(rep["th"] - rep1["th"]) <= 1e-5 * scale
         assert abs(rep["volume"] - rep1["volume"]) <= 1e-5 * abs(rep1["volume"]) and rep["collectives"] > 0
+        # the final volume is exact for the field each layout returns: the slabs' cell ranges (kf0 / kf1, the halo plane) add up to the grid
+        assert rep["volume"] == np.float32(volume_ref.reference(fine, volume_ref.fine_edge(grid, 2))[2])
+        if not opts["rbf_interp"]:      # no CG: the threshold search is an integer sum and the evaluation is per point, so nothing may differ
+            assert np.array_equal(fine, fine1) and rep["th"] == rep1["th"] and rep["volume"] == rep1["volume"]
         # exportSdfToVTI of a result that lives on several slabs: pieces + index reassemble to the returned field
         dims, origin, spacing, label, arr = r2s.read_pvti(base + ".pvti")
         assert label == "distance" and arr.shape == fine.shape and np.array_equal(arr, fine)
