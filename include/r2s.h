@@ -171,6 +171,31 @@ int r2s_export_pvti(r2s_ctx *ctx, const char *path, const char *label, int which
 int r2s_write_vti_host(const char *path, const char *label, const void *values, int is_f64, int64_t nx, int64_t ny, int64_t nz, const double origin[3],
                        const double spacing[3]);
 
+/* ---- zero surface of the smoothed SDF (csrc/r2s_surf.cu; replaces the isosurface step the reference leaves to src/Visualizations) ------- */
+/* Marching cubes with a face rule that separates the two inside corners of an ambiguous face: a closed, consistently oriented mesh of
+ * {value = iso}, a corner inside iff value >= iso.  One vertex per grid edge that crosses iso, ordered by (linear id of the edge's lower
+ * point, axis x < y < z); coordinate origin[d] + spacing[d] * (p_d [+ t on the edge's axis]), t = (iso - va) / (vb - va) in double, rounded
+ * to float once.  Triangles (int32 vertex ids, 0-based) ordered by linear cell id, then by case-table order; counter-clockwise seen from
+ * outside the solid {value >= iso}.  The result is a function of the field and iso alone (no atomics decide the order), the same on one
+ * context and on several slabs.  Unpaired mesh edges can only lie in the grid's boundary faces.  Rejected with an error: a non-finite value
+ * or iso, fewer than 2 points on an axis, 2^31 or more cells or vertices.  The mesh stays on the device until it is downloaded or exported;
+ * r2s_set_grid / r2s_set_mesh / r2s_set_slab drop it. */
+/* surface {fine_sdf = iso} of the device-resident fine_sdf of the last pipeline / smoothing call: kept on the device; frame of
+ * r2s_export_vti (origin AABB_min, spacing cell_size / smooth).  Fails on a slab rank of the NCCL communicator (use r2s_multi). */
+int r2s_isosurface(r2s_ctx *ctx, float iso, int64_t *n_vertices, int64_t *n_triangles);
+/* the same for a host field sdf[nx*ny*nz] (x fastest) in the given frame; does not touch the pipeline's resident results */
+int r2s_isosurface_from_sdf(r2s_ctx *ctx, const float *sdf, int64_t nx, int64_t ny, int64_t nz, const double origin[3],
+                            const double spacing[3], float iso, int64_t *n_vertices, int64_t *n_triangles);
+/* vertices[3*nv] (x y z per vertex), triangles[3*nt] */
+int r2s_download_isosurface(r2s_ctx *ctx, float *vertices, int32_t *triangles);
+/* format 0: binary STL (unit facet normals from a double cross product, 0 0 0 for a degenerate triangle); 1: binary little-endian PLY
+ * (shared vertices).  The mesh is downloaded to host memory once and written from there. */
+int r2s_export_isosurface(r2s_ctx *ctx, const char *path, int format);
+/* the fine_sdf of the last r2s_multi_pipeline, on all slabs: the same mesh as one context on the same field */
+int r2s_multi_isosurface(r2s_multi *m, float iso, int64_t *n_vertices, int64_t *n_triangles);
+int r2s_multi_download_isosurface(r2s_multi *m, float *vertices, int32_t *triangles);
+int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format);
+
 /* ---- measurement helper (bench.py): FMA-pipe peak of the device in TFLOP/s, fp64 != 0 -> double, else float -------- */
 int r2s_measure_fma_peak(r2s_ctx *ctx, int fp64, double *tflops);
 

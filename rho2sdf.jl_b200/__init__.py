@@ -9,6 +9,8 @@ image, so this module carries the same names, argument meaning and error behavio
     find_threshold_for_volume, calculate_isocontour_volume                  (src/MeshGrid/*)
     evalDistances, Sign_Detection, remove_sdf_artifacts                     (src/SignedDistances/*)
     RBFs_smoothing, calculate_volume_from_sdf                               (src/SdfSmoothing/*)
+    isosurface, isosurface_from_sdf, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}; the reference leaves it to
+                                                                             src/Visualizations / ParaView)
 
 Array conventions: X is (nnp, 3) float64 (== Julia's 3 x nnp column-major), IEN is (nel, nen) int64 holding 1-BASED node
 ids (== Julia's nen x nel), grid fields are indexed [k, j, i] (x fastest, == Julia's (i, j, k) column-major).
@@ -24,7 +26,8 @@ import numpy as np
 __all__ = ["HEX8", "TET4", "Rho2sdfOptions", "Mesh", "Grid", "getMesh_AABB", "generateGridPoints", "noninteractive_sdf_grid_setup",
            "DenseInNodes", "find_threshold_for_volume", "calculate_isocontour_volume", "evalDistances", "Sign_Detection",
            "remove_sdf_artifacts", "RBFs_smoothing", "calculate_volume_from_sdf", "rho2sdf", "rho2sdf_hex8", "rho2sdf_tet4",
-           "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
+           "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti",
+           "isosurface", "isosurface_from_sdf", "export_isosurface", "read_stl", "read_ply", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -129,6 +132,13 @@ def load_library():
     L.r2s_unpin_host.argtypes = [vp]
     L.r2s_write_vti_host.argtypes = [C.c_char_p, C.c_char_p, vp, C.c_int, C.c_int64, C.c_int64, C.c_int64, vp, vp]
     L.r2s_measure_fma_peak.argtypes = [vp, C.c_int, dp]
+    L.r2s_isosurface.argtypes = [vp, C.c_float, ip, ip]
+    L.r2s_isosurface_from_sdf.argtypes = [vp, vp, C.c_int64, C.c_int64, C.c_int64, vp, vp, C.c_float, ip, ip]
+    L.r2s_download_isosurface.argtypes = [vp, vp, vp]
+    L.r2s_export_isosurface.argtypes = [vp, C.c_char_p, C.c_int]
+    L.r2s_multi_isosurface.argtypes = [vp, C.c_float, ip, ip]
+    L.r2s_multi_download_isosurface.argtypes = [vp, vp, vp]
+    L.r2s_multi_export_isosurface.argtypes = [vp, C.c_char_p, C.c_int]
     _LIB = L
     return L
 
@@ -598,6 +608,96 @@ def read_pvti(path):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+# Isosurface: the zero surface of the smoothed SDF (csrc/r2s_surf.cu)
+# ---------------------------------------------------------------------------------------------------------------------
+def _surface_format(path):
+    low = str(path).lower()
+    if low.endswith(".stl"):
+        return 0
+    if low.endswith(".ply"):
+        return 1
+    raise R2SError("export_isosurface: the file name must end in .stl (binary STL) or .ply (binary PLY): %s" % path)
+
+
+def _download_surface(obj, download, nv, nt):
+    V = np.empty((nv, 3), dtype=np.float32)
+    T = np.empty((nt, 3), dtype=np.int32)
+    obj.check(download(obj.h, _ptr(V), _ptr(T)))
+    return V, T
+
+
+def _extract(mesh, iso):
+    nv, nt = C.c_int64(), C.c_int64()
+    if mesh.multi is not None:
+        m = mesh.multi
+        m.check(m.lib.r2s_multi_isosurface(m.h, float(iso), C.byref(nv), C.byref(nt)))
+        return m, m.lib.r2s_multi_download_isosurface, nv.value, nt.value
+    c = mesh.ctx
+    c.check(c.lib.r2s_isosurface(c.h, float(iso), C.byref(nv), C.byref(nt)))
+    return c, c.lib.r2s_download_isosurface, nv.value, nt.value
+
+
+def isosurface(mesh, iso=0.0):
+    """Triangle mesh of {fine_sdf = iso} for the fine_sdf the last pipeline / smoothing call left on the device(s) of `mesh` (slab 0,
+    or all slabs of a multi-GPU mesh).  Returns (V (nv, 3) float32, T (nt, 3) int32, 0-based): one vertex per grid edge that crosses
+    iso (a point is inside iff value >= iso), triangles counter-clockwise seen from outside, in the frame of export_device_result_to_vti
+    (origin AABB_min, spacing cell_size / smooth).  The mesh is closed wherever the field is below iso on the grid's border."""
+    obj, dl, nv, nt = _extract(mesh, iso)
+    return _download_surface(obj, dl, nv, nt)
+
+
+def isosurface_from_sdf(fine_sdf, origin, spacing, iso=0.0, ctx=None):
+    """The same mesh for a host field fine_sdf[k, j, i] (float32, x fastest) with grid origin and spacing (3 values each)."""
+    a = np.ascontiguousarray(fine_sdf, dtype=np.float32)
+    if a.ndim != 3:
+        raise R2SError("isosurface_from_sdf: fine_sdf must be a 3-D array [k, j, i]")
+    nz, ny, nx = a.shape
+    o = _f64(np.broadcast_to(np.asarray(origin, dtype=np.float64), (3,)))
+    h = _f64(np.broadcast_to(np.asarray(spacing, dtype=np.float64), (3,)))
+    c = ctx or Context()
+    nv, nt = C.c_int64(), C.c_int64()
+    c.check(c.lib.r2s_isosurface_from_sdf(c.h, _ptr(a), nx, ny, nz, _ptr(o), _ptr(h), float(iso), C.byref(nv), C.byref(nt)))
+    return _download_surface(c, c.lib.r2s_download_isosurface, nv.value, nt.value)
+
+
+def export_isosurface(mesh, path, iso=0.0):
+    """Extract {fine_sdf = iso} on the device(s) of `mesh` and write it to `path`: binary STL (.stl) or binary little-endian PLY (.ply)."""
+    fmt = _surface_format(path)
+    obj, _, _, _ = _extract(mesh, iso)
+    if mesh.multi is not None:
+        obj.check(obj.lib.r2s_multi_export_isosurface(obj.h, str(path).encode(), fmt))
+    else:
+        obj.check(obj.lib.r2s_export_isosurface(obj.h, str(path).encode(), fmt))
+    return str(path)
+
+
+def read_stl(path):
+    """Minimal reader of binary STL files: returns (normals (nt, 3), corners (nt, 3, 3)) float32."""
+    raw = open(path, "rb").read()
+    nt = int(np.frombuffer(raw[80:84], dtype="<u4")[0])
+    if len(raw) != 84 + 50 * nt:
+        raise R2SError("read_stl: %s is not a binary STL file of %d triangles" % (path, nt))
+    rec = np.frombuffer(raw[84:], dtype=np.dtype([("n", "<f4", 3), ("v", "<f4", (3, 3)), ("attr", "<u2")]), count=nt)
+    return rec["n"].copy(), rec["v"].copy()
+
+
+def read_ply(path):
+    """Minimal reader of the binary little-endian PLY files written above: returns (V (nv, 3) float32, T (nt, 3) int32)."""
+    raw = open(path, "rb").read()
+    end = raw.index(b"end_header\n") + len(b"end_header\n")
+    head = raw[:end].decode()
+    if "format binary_little_endian 1.0" not in head or "property list uchar int vertex_indices" not in head:
+        raise R2SError("read_ply: unsupported PLY layout in %s" % path)
+    nv = int(head.split("element vertex ")[1].split()[0])
+    nt = int(head.split("element face ")[1].split()[0])
+    V = np.frombuffer(raw, dtype="<f4", count=3 * nv, offset=end).reshape(nv, 3)
+    F = np.frombuffer(raw, dtype=np.dtype([("n", "u1"), ("i", "<i4", 3)]), count=nt, offset=end + 12 * nv)
+    if nt and not (F["n"] == 3).all():
+        raise R2SError("read_ply: only triangles are supported")
+    return V.astype(np.float32), F["i"].astype(np.int32)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
 # RhoToSDF
 # ---------------------------------------------------------------------------------------------------------------------
 class Rho2sdfOptions:
@@ -631,10 +731,11 @@ class Rho2sdfOptions:
         self.grid_step = grid_step      # stands in for the stdin prompt of interactive_sdf_grid_setup (:manual)
 
 
-def rho2sdf(taskName, X, IEN, rho, options=None, device=0, stream=None, return_report=False, devices=None, export_vti=None):
+def rho2sdf(taskName, X, IEN, rho, options=None, device=0, stream=None, return_report=False, devices=None, export_vti=None, export_surface=None):
     """src/RhoToSDF.jl:116-242 -> (fine_sdf, fine_grid, sdf_grid, sdf_dists).  `devices=[0, 1, ...]`: the timed region runs as z-slabs on
     all listed GPUs from this one call (r2s_multi_pipeline).  `export_vti=base`: the fine SDF is streamed from the device(s) to
-    base.vti (one GPU) or base.pvti + pieces (RhoToSDF.jl:230-238, :267-273); VTU / JLD2 exports are out of scope."""
+    base.vti (one GPU) or base.pvti + pieces (RhoToSDF.jl:230-238, :267-273); VTU / JLD2 exports are out of scope.  `export_surface=path`:
+    the zero surface of the fine SDF is extracted on the device(s) and written as one .stl or .ply file (export_isosurface)."""
     options = options or Rho2sdfOptions()
     mesh = Mesh(X, IEN, rho, None, element_type=options.element_type, device=device, stream=stream, devices=devices)
     if options.sdf_grid_setup == "manual":
@@ -667,6 +768,8 @@ def rho2sdf(taskName, X, IEN, rho, options=None, device=0, stream=None, return_r
         c.check(c.lib.r2s_pipeline(c.h, C.byref(p), _ptr(rn), _ptr(sdf_dists), _ptr(fine), C.byref(rep)))
         if export_vti:
             export_device_result_to_vti(mesh, str(export_vti), "distance", fine=True)
+    if export_surface:
+        export_isosurface(mesh, export_surface, 0.0)
     out = (fine.reshape(dims[2], dims[1], dims[0]), FineGrid(sdf_grid, p.smooth), sdf_grid, sdf_dists)
     if return_report:
         return out + ({"rho_t": rho_t, "rho_n": rho_n, "V_domain": mesh.V_domain, "V_frac": mesh.V_frac, **rep.asdict()},)
@@ -675,11 +778,11 @@ def rho2sdf(taskName, X, IEN, rho, options=None, device=0, stream=None, return_r
 
 def rho2sdf_hex8(taskName, X, IEN, rho, **kwargs):
     """src/RhoToSDF.jl:284-293."""
-    extra = {k: kwargs.pop(k) for k in ("device", "stream", "return_report", "devices", "export_vti") if k in kwargs}
+    extra = {k: kwargs.pop(k) for k in ("device", "stream", "return_report", "devices", "export_vti", "export_surface") if k in kwargs}
     return rho2sdf(taskName, X, IEN, rho, options=Rho2sdfOptions(element_type=HEX8, **kwargs), **extra)
 
 
 def rho2sdf_tet4(taskName, X, IEN, rho, **kwargs):
     """src/RhoToSDF.jl:295-304."""
-    extra = {k: kwargs.pop(k) for k in ("device", "stream", "return_report", "devices", "export_vti") if k in kwargs}
+    extra = {k: kwargs.pop(k) for k in ("device", "stream", "return_report", "devices", "export_vti", "export_surface") if k in kwargs}
     return rho2sdf(taskName, X, IEN, rho, options=Rho2sdfOptions(element_type=TET4, **kwargs), **extra)

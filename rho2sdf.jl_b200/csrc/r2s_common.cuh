@@ -128,6 +128,14 @@ struct r2s_ctx {
 
   // volumes
   DevBuf v_part;
+
+  // isosurface (r2s_surf.cu): per-row counts / bases, the mesh part of this context (vertices from global id surf_vglob on); have_surface is
+  // cleared by r2s_set_grid / r2s_set_mesh / r2s_set_slab; surf_part = the mesh is one slab's part of an r2s_multi mesh
+  DevBuf surf_rows, surf_V, surf_T;
+  bool have_surface = false, surf_part = false;
+  const float *surf_f = nullptr; i64 surf_nx = 0, surf_ny = 0, surf_nz = 0, surf_z0 = 0, surf_z1 = 0; float surf_iso = 0.0f;
+  double surf_origin[3] = {0, 0, 0}, surf_spacing[3] = {0, 0, 0};
+  i64 surf_nv = 0, surf_nt = 0, surf_vglob = 0, surf_nv_all = 0, surf_nt_all = 0;
 };
 
 #define CK(call)                                                                                   \
@@ -194,6 +202,11 @@ int r2s_halo_exchange_f32(r2s_ctx *ctx, float *a, i64 plane_elems, int k0, int k
 extern "C" int r2s_comm_destroy(r2s_ctx *ctx);
 extern "C" int r2s_export_vti(r2s_ctx *ctx, const char *path, const char *label, int which);
 extern "C" int r2s_export_pvti(r2s_ctx *ctx, const char *path, const char *label, int which, const char *piece_base);
+// r2s_surf.cu: isosurface passes of one slab, for r2s_multi.cu
+int r2s_surf_count_slab(r2s_ctx *ctx, float iso, i64 *nv, i64 *nt);       // pass 1 + scans on the resident fine field (collective: halo planes)
+int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);                  // pass 2 with this slab's first global vertex id
+int r2s_surf_download_slab(r2s_ctx *ctx, float *V, int32_t *T, i64 tglob, bool staging);   // this slab's part into the whole arrays
+int r2s_surf_write_file(const char *path, int format, const float *V, i64 nv, const int *T, i64 nt, std::string *err);
 // in-process groups (r2s_multi.cu drives them): one context per slab, one host thread per context
 LocalGroup *r2s_local_group_create(r2s_ctx **ctxs, int n, std::string *err);
 void r2s_local_group_destroy(LocalGroup *g);

@@ -25,6 +25,8 @@ struct r2s_multi {
   std::vector<double> plane_cost;  // per coarse plane, from the last pipeline call (empty = even cut)
   bool has_grid = false, rebalance = true, recut_pending = false;      // a re-cut is applied at the START of the next pipeline call (the resident results stay valid for export)
   int nz = 0;
+  bool have_surface = false;        // an r2s_multi_isosurface result is resident on the slabs
+  std::vector<i64> surf_vb, surf_tb;  // n + 1 global vertex / triangle bases of the slabs' parts
 };
 
 // runs fn(rank) on one host thread per slab; a failing rank wakes the others out of their host barriers
@@ -102,7 +104,7 @@ r2s_ctx *r2s_multi_context(r2s_multi *m, int slab) { return (m && slab >= 0 && s
 
 int r2s_multi_set_mesh(r2s_multi *m, int nen, int64_t nnp, const double *X, int64_t nel, const int64_t *IEN) {
   if (!m) return 1;
-  m->has_grid = false;
+  m->has_grid = false; m->have_surface = false;
   return run_all(m, [&](int r) { return r2s_set_mesh(m->ctx[(size_t)r], nen, nnp, X, nel, IEN); });
 }
 int r2s_multi_set_grid(r2s_multi *m, const double amin[3], const double amax[3], const int64_t N[3], double cell) {
@@ -110,7 +112,7 @@ int r2s_multi_set_grid(r2s_multi *m, const double amin[3], const double amax[3],
   if (N[2] + 1 < 3 * (int64_t)m->n) { m->err = "r2s_multi_set_grid: fewer than 3 coarse planes per slab"; return 1; }
   // r2s_set_grid resets a context to the whole grid; the slabs are set (collectively) right after
   for (int r = 0; r < m->n; r++) if (r2s_set_grid(m->ctx[(size_t)r], amin, amax, N, cell)) { m->err = m->ctx[(size_t)r]->err; return 1; }
-  m->nz = (int)N[2] + 1; m->plane_cost.clear(); m->has_grid = true; m->recut_pending = false;
+  m->nz = (int)N[2] + 1; m->plane_cost.clear(); m->has_grid = true; m->recut_pending = false; m->have_surface = false;
   even_cut(m);
   return m->n > 1 ? apply_cut(m) : 0;
 }
@@ -125,7 +127,8 @@ int r2s_multi_set_rebalance(r2s_multi *m, int on) { if (!m) return 1; m->rebalan
 int r2s_multi_pipeline(r2s_multi *m, const r2s_params *p, const double *rho_n, double *sdf_dists, float *fine_sdf, r2s_report *rep) {
   if (!m || !p) return 1;
   if (!m->has_grid) { m->err = "r2s_multi_set_grid has not been called"; return 1; }
-  if (m->n == 1) { int rc = r2s_pipeline(m->ctx[0], p, rho_n, sdf_dists, fine_sdf, rep); if (rc) m->err = m->ctx[0]->err; return rc; }
+  if (m->n == 1) { m->have_surface = false; int rc = r2s_pipeline(m->ctx[0], p, rho_n, sdf_dists, fine_sdf, rep); if (rc) m->err = m->ctx[0]->err; return rc; }
+  m->have_surface = false;
   if (m->recut_pending) { m->recut_pending = false; m->cut = m->next_cut; if (apply_cut(m)) return 1; }
   const GridDev &g = m->ctx[0]->g;
   const size_t pl = (size_t)g.np[0] * g.np[1];
@@ -188,5 +191,45 @@ int r2s_multi_export_vti(r2s_multi *m, const char *base, const char *label, int 
   rc = r2s_export_pvti(m->ctx[0], (b + ".pvti").c_str(), label, which, base);
   if (rc) m->err = m->ctx[0]->err;
   return rc;
+}
+
+// Zero surface of the fine field that lives on the slabs (r2s_surf.cu): every slab counts its planes, the host scans the slab counts,
+// every slab emits its part with its global bases.  The concatenation of the parts in slab order equals one context's mesh of the field.
+int r2s_multi_isosurface(r2s_multi *m, float iso, int64_t *n_vertices, int64_t *n_triangles) {
+  if (!m) return 1;
+  if (!m->has_grid) { m->err = "r2s_multi_set_grid has not been called"; return 1; }
+  m->have_surface = false;
+  std::vector<i64> nv((size_t)m->n, 0), nt((size_t)m->n, 0);
+  if (m->n == 1) {
+    int64_t a = 0, b = 0;
+    if (r2s_isosurface(m->ctx[0], iso, &a, &b)) { m->err = m->ctx[0]->err; return 1; }
+    nv[0] = a; nt[0] = b;
+  } else {
+    if (run_all(m, [&](int r) { return r2s_surf_count_slab(m->ctx[(size_t)r], iso, &nv[(size_t)r], &nt[(size_t)r]); })) return 1;
+  }
+  m->surf_vb.assign((size_t)m->n + 1, 0); m->surf_tb.assign((size_t)m->n + 1, 0);
+  for (int r = 0; r < m->n; r++) { m->surf_vb[(size_t)r + 1] = m->surf_vb[(size_t)r] + nv[(size_t)r]; m->surf_tb[(size_t)r + 1] = m->surf_tb[(size_t)r] + nt[(size_t)r]; }
+  if (m->n > 1 && run_all(m, [&](int r) { return r2s_surf_emit(m->ctx[(size_t)r], m->surf_vb[(size_t)r], m->surf_vb[(size_t)m->n]); })) return 1;
+  m->have_surface = true;
+  if (n_vertices) *n_vertices = m->surf_vb[(size_t)m->n];
+  if (n_triangles) *n_triangles = m->surf_tb[(size_t)m->n];
+  return 0;
+}
+// vertices[3 * nv], triangles[3 * nt]: the whole mesh, every slab writes its part
+static int multi_download(r2s_multi *m, float *vertices, int32_t *triangles, bool staging) {
+  if (!m->have_surface) { m->err = "isosurface: no surface on this handle (call r2s_multi_isosurface first)"; return 1; }
+  return run_all(m, [&](int r) { return r2s_surf_download_slab(m->ctx[(size_t)r], vertices, triangles, m->surf_tb[(size_t)r], staging); });
+}
+int r2s_multi_download_isosurface(r2s_multi *m, float *vertices, int32_t *triangles) { return m ? multi_download(m, vertices, triangles, false) : 1; }
+// one file for the whole mesh (format 0 binary STL, 1 binary little-endian PLY)
+int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format) {
+  if (!m) return 1;
+  if (!path) { m->err = "r2s_multi_export_isosurface: path is required"; return 1; }
+  if (!m->have_surface) { m->err = "isosurface: no surface on this handle (call r2s_multi_isosurface first)"; return 1; }
+  const i64 nv = m->surf_vb[(size_t)m->n], nt = m->surf_tb[(size_t)m->n];
+  std::vector<float> V((size_t)(3 * nv));
+  std::vector<int32_t> T((size_t)(3 * nt));
+  if (multi_download(m, V.data(), T.data(), true)) return 1;
+  return r2s_surf_write_file(path, format, V.data(), nv, T.data(), nt, &m->err);
 }
 }  // extern "C"

@@ -11,7 +11,7 @@ using Rho2sdf.MeshGrid: Mesh, Grid
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
-       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf
+       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface
 
 const LIB = get(ENV, "R2S_LIBRARY", joinpath(@__DIR__, "..", "libr2s.so"))
 
@@ -164,9 +164,43 @@ end
 export_device_vti(mesh::Mesh, filename::String; label::String="distance", fine::Bool=true) =
   (c = context(mesh); check(c, ccall((:r2s_export_vti, LIB), Cint, (Ptr{Cvoid}, Cstring, Cstring, Cint), c.h, filename, label, fine ? 1 : 0)); filename)
 
+# ---- the zero surface of the smoothed SDF (csrc/r2s_surf.cu; the reference leaves it to src/Visualizations / ParaView) -----------------
+# Vertices 3 x nv Float32, triangles 3 x nt Int32 with 1-BASED vertex ids, counter-clockwise seen from outside {fine_sdf >= iso}.
+surface_format(path::String) = endswith(lowercase(path), ".stl") ? 0 : endswith(lowercase(path), ".ply") ? 1 :
+                               error("export_isosurface: the file name must end in .stl (binary STL) or .ply (binary PLY): $path")
+function download_surface(c::Context, nv::Int64, nt::Int64)
+  V = Matrix{Float32}(undef, 3, nv); T = Matrix{Int32}(undef, 3, nt)
+  check(c, ccall((:r2s_download_isosurface, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Int32}), c.h, V, T))
+  return V, T .+ Int32(1)
+end
+"surface of the fine_sdf the last RBFs_smoothing call on `mesh` left on the device (frame: AABB_min, cell_size / smooth)"
+function isosurface(mesh::Mesh; iso::Float32=0f0)
+  c = context(mesh); nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+  check(c, ccall((:r2s_isosurface, LIB), Cint, (Ptr{Cvoid}, Cfloat, Ref{Int64}, Ref{Int64}), c.h, iso, nv, nt))
+  return download_surface(c, nv[], nt[])
+end
+"surface of a host field; the frame is read off fine_grid (its first point and its steps along the three axes)"
+function isosurface(fine_sdf::Array{Float32,3}, fine_grid::AbstractArray{Vector{Float32},3}; iso::Float32=0f0, ctx::Context=Context())
+  nx, ny, nz = size(fine_sdf)
+  size(fine_grid) == (nx, ny, nz) || error("Dimensions of fine_sdf and fine_grid must match")
+  p0 = Float64.(fine_grid[1, 1, 1])
+  h = [Float64(fine_grid[2, 1, 1][1]) - p0[1], Float64(fine_grid[1, 2, 1][2]) - p0[2], Float64(fine_grid[1, 1, 2][3]) - p0[3]]
+  nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+  check(ctx, ccall((:r2s_isosurface_from_sdf, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Int64, Int64, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Cfloat, Ref{Int64}, Ref{Int64}),
+                   ctx.h, fine_sdf, nx, ny, nz, p0, h, iso, nv, nt))
+  return download_surface(ctx, nv[], nt[])
+end
+"extract the surface on the device of `mesh` and write it as binary STL (.stl) or binary little-endian PLY (.ply)"
+function export_isosurface(mesh::Mesh, path::String; iso::Float32=0f0)
+  c = context(mesh); fmt = surface_format(path); nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+  check(c, ccall((:r2s_isosurface, LIB), Cint, (Ptr{Cvoid}, Cfloat, Ref{Int64}, Ref{Int64}), c.h, iso, nv, nt))
+  check(c, ccall((:r2s_export_isosurface, LIB), Cint, (Ptr{Cvoid}, Cstring, Cint), c.h, path, fmt))
+  return path
+end
+
 # ---- src/RhoToSDF.jl:116-242: same preamble as the reference, the timed region (:164-227) is ONE library call ---------------
 function rho2sdf(taskName::String, X::Vector{Vector{Float64}}, IEN::Vector{Vector{Int64}}, rho::Vector{Float64}; options::Rho2sdfOptions=Rho2sdfOptions(),
-                 devices::Vector{Int}=devices_from_env())
+                 devices::Vector{Int}=devices_from_env(), export_surface::Union{String,Nothing}=nothing)
   element_type = options.element_type
   mesh = Mesh(X, IEN, rho, Rho2sdf.ShapeFunctions.shape_functions; element_type=element_type)                  # :128
   sdf_grid = options.sdf_grid_setup == :manual ? Rho2sdf.MeshGrid.interactive_sdf_grid_setup(mesh) : Rho2sdf.MeshGrid.noninteractive_sdf_grid_setup(mesh)   # :141-145
@@ -183,10 +217,16 @@ function rho2sdf(taskName::String, X::Vector{Vector{Float64}}, IEN::Vector{Vecto
     mcheck(m, ccall((:r2s_multi_set_grid, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Cdouble),
                     m.h, Vector{Float64}(sdf_grid.AABB_min), Vector{Float64}(sdf_grid.AABB_max), Vector{Int64}(sdf_grid.N), sdf_grid.cell_size))
     mcheck(m, ccall((:r2s_multi_pipeline, LIB), Cint, (Ptr{Cvoid}, Ref{R2SParams}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cfloat}, Ref{R2SReport}), m.h, p, ρₙ, sdf_dists, fine_sdf, rep))
+    if export_surface !== nothing      # the zero surface of the fine SDF, extracted on all slabs, one file
+      fmt = surface_format(export_surface); nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+      mcheck(m, ccall((:r2s_multi_isosurface, LIB), Cint, (Ptr{Cvoid}, Cfloat, Ref{Int64}, Ref{Int64}), m.h, 0f0, nv, nt))
+      mcheck(m, ccall((:r2s_multi_export_isosurface, LIB), Cint, (Ptr{Cvoid}, Cstring, Cint), m.h, export_surface, fmt))
+    end
     finalize(m)
   else
     c = context(mesh); use_grid(c, sdf_grid)
     check(c, ccall((:r2s_pipeline, LIB), Cint, (Ptr{Cvoid}, Ref{R2SParams}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cfloat}, Ref{R2SReport}), c.h, p, ρₙ, sdf_dists, fine_sdf, rep))
+    export_surface === nothing || export_isosurface(mesh, export_surface)      # before release!(mesh): the field is on that context
   end
   fine_grid = fine_grid_of(sdf_grid, smooth)
   Rho2sdf.export_sdf_results_with_element_type(fine_sdf, fine_grid, sdf_grid, taskName, smooth, options.rbf_interp, element_type)   # :230-238 (unchanged, Julia)
