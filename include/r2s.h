@@ -196,6 +196,40 @@ int r2s_multi_isosurface(r2s_multi *m, float iso, int64_t *n_vertices, int64_t *
 int r2s_multi_download_isosurface(r2s_multi *m, float *vertices, int32_t *triangles);
 int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format);
 
+/* ---- the smoothed SDF as a continuous function (csrc/r2s_sample.cu, r2s_sample.cuh; rbf_interpolation_kdtree, RBFs4Smoothing.jl:219-248) -- */
+/* The last pipeline / smoothing call leaves the field
+ *     fine_sdf(x) = th + sum_c w_c exp(-(|x - c| / sigma)^2)   over the coarse grid points c with |x - c| <= maxd
+ * on the device: weights w (the CG solution, or the processed Float32 SDF in approximation mode), th (the offset added to fine_sdf),
+ * sigma = cell_size, maxd = float(sqrt(-ln(rbf_cut) cell_size^2)).  It lives as long as fine_sdf does: r2s_set_grid / r2s_set_mesh /
+ * r2s_set_slab drop it (and a failed smoothing call), and sampling without it fails with an error.  For one query point:
+ *   1. p = float(x) per coordinate, rounded once; points are double, x y z per point (Julia's 3 x n column-major)
+ *   2. C_d[i] = range(Float32(amin_d), Float32(amax_d), length = N_d + 1) with a Float64 intermediate (the reference's coarse coordinates)
+ *   3. e_d = C_d[i] - p_d in Float32; d2 = (e_x e_x + e_y e_y) + e_z e_z, every operation rounded; coarse point included iff
+ *      sqrtf(d2) <= maxd, tested as d2 <= t2 with t2 the largest float whose correctly rounded square root is <= maxd
+ *   4. phi = (a_x[i] a_y[j]) a_z[k], a_d = exp_f32(-(kappa (e_d e_d))), kappa = float(1 / cell_size^2); exp_f32 is the library's own
+ *      Float32 exponential (relative error <= 1.5 2^-24); phi is within Float32 round-off of exp(-kappa d2)
+ *   5. value = (fmaf(w, phi, acc) over the included points in ascending (k, j, i), from 0) + th
+ *   6. gradient (optional) = (kappa + kappa) * sum fmaf(w phi, e_d, g_d) per axis, same order (d/dx of th + sum w phi)
+ *   7. lattice points: p_d = float(origin_d) + float(i_d) * float(spacing_d) in Float32 (origin = AABB_min, spacing = cell_size / k gives
+ *      the points of the reference's create_smooth_grid for smooth = k)
+ * The reference sums the 124 nearest coarse points within maxd; no ball of radius maxd (ln(1/cut) <= 8) holds more than 124 grid points
+ * (tests/test_sample_host.py proves it), so the sets are equal and only the order of summation differs.  Points outside the grid are
+ * legal: missing neighbours contribute nothing, far away the value is th.  The results are a function of the point alone: the same
+ * for any order or chunking of the points, on one context and on several slabs (given the same weights).  Rejected with an error:
+ * non-finite coordinates, n > 0 with a NULL array, lattice dims < 1; the single-context calls fail on a slab rank of the NCCL
+ * communicator (use r2s_multi).  Host arrays pass through a bounded device buffer in chunks: n is limited by host memory only. */
+/* values[n]; gradients: NULL or 3 * n (x y z per point) */
+int r2s_sample_sdf(r2s_ctx *ctx, const double *points, int64_t n, float *values, float *gradients);
+/* values[dims[0] * dims[1] * dims[2]], x fastest; the coordinates are generated on the device (none are stored) */
+int r2s_sample_sdf_lattice(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float *values);
+/* the field's definition: weights[(N1+1)(N2+1)(N3+1)] (x fastest, unpitched) and th; either may be NULL */
+int r2s_download_rbf_weights(r2s_ctx *ctx, float *weights, float *th);
+/* the field the last r2s_multi_pipeline left on the slabs: every point goes to the slab owning its floor plane (the largest z-table
+ * entry <= p_z, clamped to the grid), results come back in input order */
+int r2s_multi_sample_sdf(r2s_multi *m, const double *points, int64_t n, float *values, float *gradients);
+int r2s_multi_sample_sdf_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float *values);
+int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th);
+
 /* ---- measurement helper (bench.py): FMA-pipe peak of the device in TFLOP/s, fp64 != 0 -> double, else float -------- */
 int r2s_measure_fma_peak(r2s_ctx *ctx, int fp64, double *tflops);
 

@@ -11,6 +11,8 @@ image, so this module carries the same names, argument meaning and error behavio
     RBFs_smoothing, calculate_volume_from_sdf                               (src/SdfSmoothing/*)
     isosurface, isosurface_from_sdf, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}; the reference leaves it to
                                                                              src/Visualizations / ParaView)
+    sample_sdf, sample_sdf_lattice, rbf_weights                             (the smoothed SDF as a continuous function:
+                                                                             rbf_interpolation_kdtree, RBFs4Smoothing.jl:219-248)
 
 Array conventions: X is (nnp, 3) float64 (== Julia's 3 x nnp column-major), IEN is (nel, nen) int64 holding 1-BASED node
 ids (== Julia's nen x nel), grid fields are indexed [k, j, i] (x fastest, == Julia's (i, j, k) column-major).
@@ -27,7 +29,8 @@ __all__ = ["HEX8", "TET4", "Rho2sdfOptions", "Mesh", "Grid", "getMesh_AABB", "ge
            "DenseInNodes", "find_threshold_for_volume", "calculate_isocontour_volume", "evalDistances", "Sign_Detection",
            "remove_sdf_artifacts", "RBFs_smoothing", "calculate_volume_from_sdf", "rho2sdf", "rho2sdf_hex8", "rho2sdf_tet4",
            "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti",
-           "isosurface", "isosurface_from_sdf", "export_isosurface", "read_stl", "read_ply", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
+           "isosurface", "isosurface_from_sdf", "export_isosurface", "read_stl", "read_ply",
+           "sample_sdf", "sample_sdf_lattice", "rbf_weights", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -139,6 +142,10 @@ def load_library():
     L.r2s_multi_isosurface.argtypes = [vp, C.c_float, ip, ip]
     L.r2s_multi_download_isosurface.argtypes = [vp, vp, vp]
     L.r2s_multi_export_isosurface.argtypes = [vp, C.c_char_p, C.c_int]
+    for pre in ("r2s_", "r2s_multi_"):
+        getattr(L, pre + "sample_sdf").argtypes = [vp, vp, C.c_int64, vp, vp]
+        getattr(L, pre + "sample_sdf_lattice").argtypes = [vp, vp, vp, vp, vp]
+        getattr(L, pre + "download_rbf_weights").argtypes = [vp, vp, fp]
     _LIB = L
     return L
 
@@ -695,6 +702,59 @@ def read_ply(path):
     if nt and not (F["n"] == 3).all():
         raise R2SError("read_ply: only triangles are supported")
     return V.astype(np.float32), F["i"].astype(np.int32)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# The smoothed SDF as a continuous function (csrc/r2s_sample.cu)
+# ---------------------------------------------------------------------------------------------------------------------
+def _sampler(mesh):
+    """(handle object, function prefix): all slabs of a multi-GPU mesh, else the mesh's context"""
+    return (mesh.multi, "r2s_multi_") if mesh.multi is not None else (mesh.ctx, "r2s_")
+
+
+def sample_sdf(mesh, points, gradient=False):
+    """The reference's rbf_interpolation_kdtree(points, coarse_grid, weights, kernel) (RBFs4Smoothing.jl:219-248) for the field the last
+    pipeline / smoothing call left on the device(s) of `mesh`: th + sum_c w_c exp(-(|x - c| / cell)^2) over the coarse points within the
+    kernel's cut radius, evaluated on the GPU at arbitrary points (outside the grid too; far away the value is th).  points: (n, 3)
+    float64.  Returns float32 values (n,), and with gradient=True also the analytic gradients (n, 3) float32.  The exact arithmetic is
+    stated in include/r2s.h; a point's result does not depend on the other points or their order."""
+    p = np.ascontiguousarray(points, dtype=np.float64)
+    if p.ndim != 2 or p.shape[1] != 3:
+        raise R2SError("sample_sdf: points must be an (n, 3) array")
+    n = p.shape[0]
+    val = np.empty(n, dtype=np.float32)
+    g = np.empty((n, 3), dtype=np.float32) if gradient else None
+    obj, pre = _sampler(mesh)
+    obj.check(getattr(obj.lib, pre + "sample_sdf")(obj.h, _ptr(p) if n else None, n, _ptr(val) if n else None, _ptr(g) if (gradient and n) else None))
+    return (val, g) if gradient else val
+
+
+def sample_sdf_lattice(mesh, origin, spacing, shape):
+    """rbf_interpolation_kdtree on the lattice origin + i * spacing (i = 0 .. shape - 1 per axis, Float32 arithmetic, no coordinates
+    stored): returns float32 [k, j, i] of shape (shape[2], shape[1], shape[0]).  origin = AABB_min, spacing = cell_size / k gives the
+    points of the reference's create_smooth_grid for smooth = k, i.e. resampling at any resolution."""
+    o = _f64(np.broadcast_to(np.asarray(origin, dtype=np.float64), (3,)))
+    h = _f64(np.broadcast_to(np.asarray(spacing, dtype=np.float64), (3,)))
+    dims = np.ascontiguousarray(np.broadcast_to(np.asarray(shape, dtype=np.int64), (3,)))
+    if (dims < 1).any():
+        raise R2SError("sampling: lattice dims must be >= 1")
+    out = np.empty((int(dims[2]), int(dims[1]), int(dims[0])), dtype=np.float32)
+    obj, pre = _sampler(mesh)
+    obj.check(getattr(obj.lib, pre + "sample_sdf_lattice")(obj.h, _ptr(o), _ptr(h), _ptr(dims), _ptr(out)))
+    return out
+
+
+def rbf_weights(mesh):
+    """The definition of the continuous field: (w[k, j, i] float32 on the coarse grid, th float32), the weights and offset that
+    rbf_interpolation_kdtree sums (the CG solution, or the processed SDF in approximation mode)."""
+    obj, pre = _sampler(mesh)
+    if mesh._grid_id is None:
+        raise R2SError("r2s_set_grid has not been called")
+    np_ = [v + 1 for v in mesh._grid_id[2]]
+    w = np.empty((np_[2], np_[1], np_[0]), dtype=np.float32)
+    th = C.c_float()
+    obj.check(getattr(obj.lib, pre + "download_rbf_weights")(obj.h, _ptr(w), C.byref(th)))
+    return w, np.float32(th.value)
 
 
 # ---------------------------------------------------------------------------------------------------------------------

@@ -42,7 +42,7 @@ void r2s_destroy(r2s_ctx *ctx) {
                    &ctx->counters, &ctx->box_rec, &ctx->plist, &ctx->dist, &ctx->xp, &ctx->sdf, &ctx->signs, &ctx->s_rng, &ctx->s_el, &ctx->s_cnt, &ctx->s_keys, &ctx->s_keys_alt, &ctx->s_tile_ptr,
                    &ctx->cc_label, &ctx->cc_size, &ctx->cc_scal, &ctx->cc_bits, &ctx->cc_bits_all, &ctx->cc_gsz, &ctx->cc_seen, &ctx->f_s, &ctx->f_w, &ctx->f_r, &ctx->f_u, &ctx->f_c, &ctx->f_lsf, &ctx->f_fine, &ctx->f_part,
                    &ctx->f_scal, &ctx->cutlist, &ctx->slablist, &ctx->v_part, &ctx->vlist[0], &ctx->vlist[1], &ctx->vent[0], &ctx->vent[1], &ctx->vrec, &ctx->bis_state, &ctx->lat_xs, &ctx->lat_cell, &ctx->lat_map, &ctx->lat_info, &ctx->lat_pt,
-                   &ctx->surf_rows, &ctx->surf_V, &ctx->surf_T};
+                   &ctx->surf_rows, &ctx->surf_V, &ctx->surf_T, &ctx->rbf_tab, &ctx->smp_in, &ctx->smp_out};
   for (DevBuf *b : all) b->release();
   for (int i = 0; i < 16; i++) cudaEventDestroy(ctx->ev[i]);
   for (int i = 0; i < 5; i++) { cudaEventDestroy(ctx->ev_probe[i]); cudaEventDestroy(ctx->ev_k[i]); }
@@ -68,7 +68,7 @@ int r2s_set_mesh(r2s_ctx *ctx, int nen, int64_t nnp, const double *X, int64_t ne
   if (nel * nen >= (1ll << 31) || nnp >= (1ll << 31)) FAIL("r2s_set_mesh: mesh too large for 32-bit connectivity");
   CK(cudaSetDevice(ctx->device));
   for (i64 t = 0; t < nel * nen; t++) if (IEN[t] < 1 || IEN[t] > nnp) FAIL("r2s_set_mesh: IEN entry out of range (expected 1-based node ids)");
-  ctx->have_sdf = ctx->have_fine = ctx->have_surface = false;
+  ctx->have_sdf = ctx->have_fine = ctx->have_rbf = ctx->have_surface = false;
   ctx->nen = nen; ctx->nes = nen == 8 ? 6 : 4; ctx->nsn = nen == 8 ? 4 : 3; ctx->nnp = nnp; ctx->nel = nel;
   CK(ctx->X.reserve(sizeof(double) * 3 * (size_t)nnp));
   CK(ctx->IEN32.reserve(sizeof(int) * (size_t)(nel * nen)));
@@ -122,7 +122,7 @@ int r2s_set_grid(r2s_ctx *ctx, const double amin[3], const double amax[3], const
   CK(cudaStreamSynchronize(ctx->stream));
   g.pc = ctx->gtab_d.as<double>(); g.cellof = ctx->gtab_i.as<int>(); g.cstart = ctx->gtab_i.as<int>() + tot_p;
   ctx->has_grid = true; ctx->k0 = 0; ctx->k1 = g.np[2];
-  ctx->have_sdf = ctx->have_fine = ctx->have_surface = false; ctx->slab_k0.clear();
+  ctx->have_sdf = ctx->have_fine = ctx->have_rbf = ctx->have_surface = false; ctx->slab_k0.clear();
   return 0;
 }
 int r2s_set_slab(r2s_ctx *ctx, int64_t k0, int64_t k1) {
@@ -131,7 +131,7 @@ int r2s_set_slab(r2s_ctx *ctx, int64_t k0, int64_t k1) {
   if (k0 < 0 || k1 > ctx->g.np[2] || k0 >= k1) FAIL("r2s_set_slab: invalid plane range");
   if (ctx->nranks > 1 && k1 - k0 < 3) FAIL("r2s_set_slab: a slab needs at least 3 planes (smoothing halo)");
   ctx->k0 = k0; ctx->k1 = k1;
-  ctx->slab_k0.clear(); ctx->have_sdf = ctx->have_fine = ctx->have_surface = false;
+  ctx->slab_k0.clear(); ctx->have_sdf = ctx->have_fine = ctx->have_rbf = ctx->have_surface = false;
   if (ctx->nranks > 1) {
     // every rank learns the whole partition (collective: all ranks call r2s_set_slab); slabs must tile [0, N3+1) in rank order
     CK(cudaSetDevice(ctx->device));

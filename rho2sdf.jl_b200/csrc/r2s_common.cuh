@@ -125,6 +125,11 @@ struct r2s_ctx {
   DevBuf f_s, f_w, f_r, f_u, f_c, f_lsf, f_fine, f_part, f_scal, cutlist, slablist, vlist[2], vent[2], vrec, bis_state;
   int smooth_last = 1;
   bool have_sdf = false, have_fine = false;      // ctx->sdf / ctx->f_fine hold a result of the CURRENT grid (cleared by r2s_set_grid / r2s_set_mesh)
+  // the continuous field of the last smoothing call (r2s_sample.cu): weights rbf_w (f_w after the CG, f_s in approximation mode; row
+  // pitch rbf_px, whole-grid plane indexing, owned planes + 2 below / 3 above valid), offset rbf_th, the Float32 coordinate tables (host
+  // rbf_c, device rbf_tab).  have_rbf is cleared with have_fine; nothing but r2s_dev_rbf writes f_w / f_s.
+  bool have_rbf = false; const float *rbf_w = nullptr; int rbf_px = 0; float rbf_th = 0.0f; double rbf_cut = 0.0;
+  std::vector<float> rbf_c[3]; DevBuf rbf_tab, smp_in, smp_out;
 
   // volumes
   DevBuf v_part;
@@ -207,6 +212,14 @@ int r2s_surf_count_slab(r2s_ctx *ctx, float iso, i64 *nv, i64 *nt);       // pas
 int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);                  // pass 2 with this slab's first global vertex id
 int r2s_surf_download_slab(r2s_ctx *ctx, float *V, int32_t *T, i64 tglob, bool staging);   // this slab's part into the whole arrays
 int r2s_surf_write_file(const char *path, int format, const float *V, i64 nv, const int *T, i64 nt, std::string *err);
+// r2s_sample.cu: the sampler of the continuous field, for r2s_rbf.cu (record) and r2s_multi.cu (one slab's share, no rank check)
+struct SampleGrid;
+int r2s_sample_record(r2s_ctx *ctx, const float *w, int px, float th, double rbf_cut);
+int r2s_sample_grid(r2s_ctx *ctx, SampleGrid *G, bool dev);
+int r2s_sample_points_ctx(r2s_ctx *ctx, const double *pts, i64 n, float *val, float *grad);
+int r2s_sample_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float o[3], float h[3]);
+int r2s_sample_lattice_planes(r2s_ctx *ctx, const float o[3], const float h[3], const int64_t dims[3], i64 ka, i64 kb, float *out);
+int r2s_sample_download_weights(r2s_ctx *ctx, float *w, float *th, i64 k0, i64 k1);
 // in-process groups (r2s_multi.cu drives them): one context per slab, one host thread per context
 LocalGroup *r2s_local_group_create(r2s_ctx **ctxs, int n, std::string *err);
 void r2s_local_group_destroy(LocalGroup *g);

@@ -7,6 +7,7 @@
 // path (that is how the multi-slab logic is tested on a one-GPU box).  After every call the slabs are re-cut by measured cost (the
 // planes next to the mesh boundary carry the boundary-face work).
 #include <math.h>
+#include <cmath>
 #include <string.h>
 #include <algorithm>
 #include <functional>
@@ -14,6 +15,7 @@
 #include <thread>
 #include <vector>
 #include "r2s_common.cuh"
+#include "r2s_sample.cuh"
 
 struct r2s_multi {
   int n = 0;
@@ -222,6 +224,79 @@ static int multi_download(r2s_multi *m, float *vertices, int32_t *triangles, boo
 }
 int r2s_multi_download_isosurface(r2s_multi *m, float *vertices, int32_t *triangles) { return m ? multi_download(m, vertices, triangles, false) : 1; }
 // one file for the whole mesh (format 0 binary STL, 1 binary little-endian PLY)
+// ---- sampling the continuous field (r2s_sample.cu): a point whose floor plane in the Float32 z-table is c needs weight planes c - 2 .. c + 3;
+// a slab keeps its owned planes [k0, k1) plus 2 below and 3 above valid (the fine evaluation reads the same), so the slab owning c has them
+static int multi_sample_ready(r2s_multi *m, SampleGrid *G) {
+  if (!m->has_grid) { m->err = "r2s_multi_set_grid has not been called"; return 1; }
+  for (int r = 0; r < m->n; r++)
+    if (r2s_sample_grid(m->ctx[(size_t)r], G, false)) { m->err = "slab " + std::to_string(r) + ": " + m->ctx[(size_t)r]->err; return 1; }
+  return 0;
+}
+static int owner_of(const r2s_multi *m, const SampleGrid &G, float z) {
+  const int c = smp_floor(G.C[2], G.n[2], G.c0[2], G.inv[2], z);
+  return (int)(std::upper_bound(m->cut.begin() + 1, m->cut.end(), (i64)c) - m->cut.begin()) - 1;
+}
+int r2s_multi_sample_sdf(r2s_multi *m, const double *points, int64_t n, float *values, float *gradients) {
+  if (!m) return 1;
+  if (m->n == 1) { int rc = r2s_sample_sdf(m->ctx[0], points, n, values, gradients); if (rc) m->err = m->ctx[0]->err; return rc; }
+  if (n < 0) { m->err = "sampling: negative point count"; return 1; }
+  if (n > 0 && (!points || !values)) { m->err = "sampling: points and values are required when n > 0"; return 1; }
+  SampleGrid G;
+  if (multi_sample_ready(m, &G)) return 1;
+  std::vector<std::vector<i64>> idx((size_t)m->n);
+  for (i64 t = 0; t < n; t++) {
+    const double *p = points + 3 * t;
+    if (!std::isfinite(p[0]) || !std::isfinite(p[1]) || !std::isfinite(p[2])) { m->err = "sampling: a point coordinate is NaN or infinite"; return 1; }
+    idx[(size_t)owner_of(m, G, (float)p[2])].push_back(t);
+  }
+  return run_all(m, [&](int r) {
+    const std::vector<i64> &id = idx[(size_t)r];
+    const size_t k = id.size();
+    std::vector<double> p(3 * k);
+    std::vector<float> v(k), g(gradients ? 3 * k : 0);
+    for (size_t q = 0; q < k; q++) for (int d = 0; d < 3; d++) p[3 * q + d] = points[3 * id[q] + d];
+    if (r2s_sample_points_ctx(m->ctx[(size_t)r], p.data(), (i64)k, v.data(), gradients ? g.data() : nullptr)) return 1;
+    for (size_t q = 0; q < k; q++) {
+      values[id[q]] = v[q];
+      if (gradients) for (int d = 0; d < 3; d++) gradients[3 * id[q] + d] = g[3 * q + d];
+    }
+    return 0;
+  });
+}
+int r2s_multi_sample_sdf_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float *values) {
+  if (!m) return 1;
+  if (m->n == 1) { int rc = r2s_sample_sdf_lattice(m->ctx[0], origin, spacing, dims, values); if (rc) m->err = m->ctx[0]->err; return rc; }
+  float o[3], h[3];
+  if (r2s_sample_lattice_check(m->ctx[0], origin, spacing, dims, o, h)) { m->err = m->ctx[0]->err; return 1; }
+  SampleGrid G;
+  if (multi_sample_ready(m, &G)) return 1;
+  if (!values) { m->err = "sampling: values are required"; return 1; }
+  // runs of consecutive lattice planes with the same owner (a plane's z is o_z + float(k) h_z, the same formula as the kernel)
+  std::vector<std::vector<std::pair<i64, i64>>> runs((size_t)m->n);
+  int prev = -1;
+  for (i64 k = 0; k < dims[2]; k++) {
+    const int r = owner_of(m, G, smp_add(o[2], smp_mul((float)k, h[2])));
+    if (r == prev) runs[(size_t)r].back().second = k + 1;
+    else runs[(size_t)r].push_back({k, k + 1});
+    prev = r;
+  }
+  const i64 pl = dims[0] * dims[1];
+  return run_all(m, [&](int r) {
+    for (const auto &ab : runs[(size_t)r])
+      if (r2s_sample_lattice_planes(m->ctx[(size_t)r], o, h, dims, ab.first, ab.second, values + ab.first * pl)) return 1;
+    return 0;
+  });
+}
+// every slab writes its owned weight planes; th is the same on all slabs (the threshold search is collective)
+int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th) {
+  if (!m) return 1;
+  if (m->n == 1) { int rc = r2s_download_rbf_weights(m->ctx[0], weights, th); if (rc) m->err = m->ctx[0]->err; return rc; }
+  if (!weights && !th) { m->err = "r2s_download_rbf_weights: weights or th is required"; return 1; }
+  SampleGrid G;
+  if (multi_sample_ready(m, &G)) return 1;
+  return run_all(m, [&](int r) { return r2s_sample_download_weights(m->ctx[(size_t)r], weights, r == 0 ? th : nullptr, m->cut[(size_t)r], m->cut[(size_t)r + 1]); });
+}
+
 int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format) {
   if (!m) return 1;
   if (!path) { m->err = "r2s_multi_export_isosurface: path is required"; return 1; }

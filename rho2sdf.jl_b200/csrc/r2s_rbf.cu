@@ -1037,6 +1037,7 @@ int r2s_dev_rbf(r2s_ctx *ctx, int is_interp, int smooth, double rbf_cut, double 
   const int kf0 = smooth * k0, kf1 = (k1 < nz) ? smooth * k1 : fz;       // fine planes of this slab
   // the stencil form needs the reference's cut to sit strictly between lattice shells (true for the default 1e-3)
   StencilW W; { double L = -log(rbf_cut); if (!(L > 6.0 && L < 8.0)) FAIL("rbf: only kernel cut-offs with 6 < ln(1/cut) < 8 (81-point stencil) are supported"); for (int m = 0; m < 8; m++) W.w[m] = (float)exp(-(double)m); }
+  ctx->have_rbf = false;      // f_s / f_w are rewritten below
   CK(cudaEventRecord(ctx->ev[4], st));
   CK(ctx->f_s.reserve(sizeof(float) * (size_t)n)); CK(ctx->f_lsf.reserve(sizeof(float) * (size_t)n));
   CK(ctx->f_fine.reserve(sizeof(float) * (size_t)nf));
@@ -1224,6 +1225,7 @@ int r2s_dev_rbf(r2s_ctx *ctx, int is_interp, int smooth, double rbf_cut, double 
   CK(cudaEventRecord(ctx->ev[15], st));
   CK(cudaStreamSynchronize(st));
   ctx->smooth_last = smooth; ctx->have_fine = true;
+  if (r2s_sample_record(ctx, wgt, px, tho, rbf_cut)) return 1;
   *th_out = tho; *vol_out = volf;
   CK(cudaEventElapsedTime(&ctx->rep.ms_rbf_prep, ctx->ev[4], ctx->ev[5]));
   CK(cudaEventElapsedTime(&ctx->rep.ms_cg, ctx->ev[5], ctx->ev[6]));

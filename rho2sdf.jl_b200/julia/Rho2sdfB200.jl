@@ -11,7 +11,7 @@ using Rho2sdf.MeshGrid: Mesh, Grid
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
-       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface
+       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, sample_sdf, sample_sdf_lattice, rbf_weights
 
 const LIB = get(ENV, "R2S_LIBRARY", joinpath(@__DIR__, "..", "libr2s.so"))
 
@@ -196,6 +196,32 @@ function export_isosurface(mesh::Mesh, path::String; iso::Float32=0f0)
   check(c, ccall((:r2s_isosurface, LIB), Cint, (Ptr{Cvoid}, Cfloat, Ref{Int64}, Ref{Int64}), c.h, iso, nv, nt))
   check(c, ccall((:r2s_export_isosurface, LIB), Cint, (Ptr{Cvoid}, Cstring, Cint), c.h, path, fmt))
   return path
+end
+
+# ---- the smoothed SDF as a continuous function: rbf_interpolation_kdtree (src/SdfSmoothing/RBFs4Smoothing.jl:219-248) on the GPU ----------
+# th + sum_c w_c exp(-(|x - c| / cell_size)^2) over the coarse points within the cut radius, for the field the last RBFs_smoothing call on
+# `mesh` left on the device (exact arithmetic: include/r2s.h)
+"values (Float32, n) at the columns of points (3 x n); with gradient=true also the analytic gradients (3 x n Float32)"
+function sample_sdf(mesh::Mesh, points::Matrix{Float64}; gradient::Bool=false)
+  size(points, 1) == 3 || error("sample_sdf: points must be a 3 x n matrix")
+  c = context(mesh); n = size(points, 2)
+  values = Vector{Float32}(undef, n); grads = gradient ? Matrix{Float32}(undef, 3, n) : nothing
+  check(c, ccall((:r2s_sample_sdf, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Int64, Ptr{Cfloat}, Ptr{Cfloat}),
+                 c.h, points, n, values, gradient ? grads : C_NULL))
+  return gradient ? (values, grads) : values
+end
+"values on the lattice origin + (i - 1) .* spacing, i = 1 .. dims per axis (Float32 arithmetic), as an Array{Float32,3} of size dims"
+function sample_sdf_lattice(mesh::Mesh, origin::AbstractVector{<:Real}, spacing::AbstractVector{<:Real}, dims::NTuple{3,Int})
+  c = context(mesh); out = Array{Float32,3}(undef, dims)
+  check(c, ccall((:r2s_sample_sdf_lattice, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Ptr{Cfloat}),
+                 c.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], out))
+  return out
+end
+"(weights on the coarse grid of `grid`, th): the definition of the continuous field"
+function rbf_weights(mesh::Mesh, grid)
+  c = context(mesh); w = Array{Float32,3}(undef, Tuple(Int.(grid.N .+ 1))); th = Ref{Cfloat}(0f0)
+  check(c, ccall((:r2s_download_rbf_weights, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ref{Cfloat}), c.h, w, th))
+  return w, th[]
 end
 
 # ---- src/RhoToSDF.jl:116-242: same preamble as the reference, the timed region (:164-227) is ONE library call ---------------
