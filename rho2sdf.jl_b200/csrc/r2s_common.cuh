@@ -116,7 +116,7 @@ struct r2s_ctx {
   std::vector<double> h_pc[3];
 
   // distance / sign work buffers
-  DevBuf cls, act_flag, act_idx, act_rec, cnt_a, cnt_b, keys, keys_alt, tile_ptr, tile_faces, face_tiles, fc_list, tri_cnt, tri_rec, pairbuf, pairxp, cubtmp, counters, box_rec, plist;
+  DevBuf cls, act_flag, act_idx, act_rec, cnt_a, cnt_b, keys, keys_alt, tile_ptr, tile_faces, face_tiles, fc_list, tri_cnt, tri_rec, pairbuf, pairxp, cubtmp, counters, box_rec, plist, pseed;
   DevBuf dist, xp, sdf, signs;
   DevBuf s_rng, s_el, s_cnt, s_keys, s_keys_alt, s_tile_ptr;
   // connected components

@@ -15,6 +15,7 @@
 #include "r2s_tables.cuh"
 #include "r2s_exact.cuh"
 #include "r2s_iso.cuh"
+#include "r2s_bound.cuh"
 
 // ------------------------------------------------------------------------------------------------ binning
 // [zlo, zhi]: z-extent of the slab's planes grown by a safe margin; elements entirely outside cannot reach a plane of this rank
@@ -175,16 +176,19 @@ __global__ void __launch_bounds__(128, WANT_XP ? (BOX ? 4 : 2) : 4) k_project_he
 
 // ---- pair-list path for box elements (the headline workload: every voxel-type SIMP mesh) ----------------------------------------
 // evalDistances keeps, per grid point, the MINIMUM over the crossing elements whose candidate range holds the point
-// (sdfOnDensityField.jl:606-621).  A pair whose lower bound -- the distance from the point to a box that contains the element's
+// (sdfOnDensityField.jl:606-621).  A pair whose lower bound -- the distance from the point to a set that contains the element's
 // iso-patch -- is not below the point's current minimum cannot change the result, so it is never projected (exact: the result is a
 // minimum).  Organisation:
-//   k_box_records  per crossing box element: solver constants (iso::HexBox in element-local coordinates), phase 1, and the TIGHT box
-//                  of its iso-patch: per axis the hull of the slices xi_d = s whose four corner densities straddle rho_t (a bilinear
-//                  field takes its extrema over a slice at the corners; the candidates for the hull's ends are s = +-1 and the iso
-//                  crossings of the four edges along d)
-//   k_pair_scan<0> pass A: pairs whose point lies inside the element's closed AABB (bound 0, always needed) and every pair of a tile
-//                  with boundary-face elements (those go to the pair buffer un-pruned: k_assemble replays them in element order)
-//   k_pair_scan<1> pass B, after pass A has been projected: the other pairs, kept only if their bound is below dist[] so far
+//   k_box_records  per crossing box element: solver constants (iso::HexBox in element-local coordinates), phase 1, the TIGHT box of its
+//                  iso-patch and a slab that holds the patch (r2s_bound.cuh); the bound of a pair is the distance to box /\ slab
+//   k_pair_scan<0> seed: for every pair that does not go to the pair buffer, atomicMin of (float tight-box distance rounded down) << 32
+//                  | element on a per-point key -- each point's nearest element box, ties to the smaller active index (the seed only
+//                  chooses which pair pass A solves; seeding by box /\ slab solved 0.7 % of the pairs fewer on the replica of
+//                  tools/prune_study.py and cost an exact bound for every pair)
+//   k_pair_scan<1> pass A: every pair of a tile with boundary-face elements (those go to the pair buffer un-pruned: k_assemble replays
+//                  them in element order) and, for each other point, the one pair its key names
+//   k_pair_scan<2> pass B, after pass A has been projected: the other pairs, kept only if their bound is below dist[] so far (the cheap
+//                  tight-box bound first, then box distance + slab gap (lb2_box_gap), box /\ slab only for the pairs both leave)
 //   k_project_list one LANE per listed pair (dense warps whatever was pruned), result by atomicMin / into the pair buffer.
 struct __align__(16) BoxRec {      // 16-byte aligned: the projection kernel reads its doubles two at a time
   double R[8];               // monomial coefficients of rho
@@ -193,6 +197,7 @@ struct __align__(16) BoxRec {      // 16-byte aligned: the projection kernel rea
   double xi0[3];             // phase 1: Newton projection of xi = 0 onto the iso-surface
   double gs;                 // scale of the tolerances
   double tlo[3], thi[3];     // tight box of the iso-patch, GLOBAL coordinates (slightly widened)
+  double sn[3], sA, sB;      // slab sA <= sn.y <= sB that holds the iso-patch, GLOBAL coordinates (r2s_bound.cuh; sn = 0: unbounded)
   i64 pair_off;
   int ps[3], nx, ny, vol, ok0, el;
   int ftile, pad_;           // 1 = some tile overlapped by the candidate range holds boundary-face elements (its pairs may go to the pair buffer)
@@ -234,37 +239,11 @@ __global__ void k_box_records(i64 nact, const ActRec *__restrict__ rec, const in
       for (int ty = r.ps[1] / TILE_Y; ty <= (r.pe[1] - 1) / TILE_Y; ty++)
         for (int tx = r.ps[0] / TILE_X; tx <= (r.pe[0] - 1) / TILE_X; tx++)
           if (tile_faces[((i64)tz * g.nt[1] + ty) * g.nt[0] + tx]) B.ftile = 1;
-  // tight box per axis: corner pairs (lo end, hi end) of the four edges along the axis, node order of hex8_shape.jl:27-34
-  const int ea[3][4] = {{0, 3, 4, 7}, {0, 1, 4, 5}, {0, 1, 2, 3}}, eb[3][4] = {{1, 2, 5, 6}, {3, 2, 7, 6}, {4, 5, 6, 7}};
-#pragma unroll
-  for (int d = 0; d < 3; d++) {
-    double va[4], vb[4], cand[6]; int nc = 0;
-    cand[nc++] = -1.0; cand[nc++] = 1.0;
-#pragma unroll
-    for (int q = 0; q < 4; q++) {
-      va[q] = nv[3][ea[d][q]] - rho_t; vb[q] = nv[3][eb[d][q]] - rho_t;
-      if ((va[q] < 0.0) != (vb[q] < 0.0) && va[q] != vb[q]) cand[nc++] = fmin(1.0, fmax(-1.0, -1.0 + 2.0 * va[q] / (va[q] - vb[q])));
-    }
-    double smin = 1.0, smax = -1.0; bool any = false;
-    for (int t = 0; t < nc; t++) {
-      const double s = cand[t], w = 0.5 * (s + 1.0);
-      double mn = 1e300, mx = -1e300;
-#pragma unroll
-      for (int q = 0; q < 4; q++) { const double val = va[q] + (vb[q] - va[q]) * w; mn = fmin(mn, val); mx = fmax(mx, val); }
-      const double tol = 1e-12 * B.gs;
-      if (mn <= tol && mx >= -tol) { smin = fmin(smin, s); smax = fmax(smax, s); any = true; }
-    }
-    if (!any) { smin = -1.0; smax = 1.0; }      // cannot happen for a crossing element; stay safe
-    const double pad = 1e-9;                    // widen in xi: the bound only has to be a lower bound
-    smin = fmax(-1.0, smin - pad); smax = fmin(1.0, smax + pad);
-    const double x0 = H.c[d] + H.h[d] * smin + B.org[d], x1 = H.c[d] + H.h[d] * smax + B.org[d];
-    const double wid = 4e-16 * (fabs(B.org[d]) + fabs(H.c[d]) + fabs(H.h[d]));
-    B.tlo[d] = fmin(x0, x1) - wid; B.thi[d] = fmax(x0, x1) + wid;
-  }
+  bnd::box_iso_bounds(nv[3], rho_t, B.gs, B.org, H.c, H.h, B.tlo, B.thi, B.sn, B.sA, B.sB);
   box[a] = B;
 }
 // one warp per active element; lanes stride over its candidate points.  plist entry: bit 63 = goes to the pair buffer, bits 24..62 =
-// active-element index, bits 0..23 = local point index.  cnt[0] = list length, cnt[1] = pairs pruned (statistics).
+// active-element index, bits 0..23 = local point index.  cnt[0] = list length.  seed: per grid point the key of k_pair_scan<0>.
 #define PL_LI_BITS 24
 #ifndef R2S_SCAN_MINB
 #define R2S_SCAN_MINB 4      // pair scan: 64 registers (a few spills), 4 CTAs of 256 threads per SM: project 43.8 -> 42.7 ms against the unconstrained 94-register build
@@ -274,7 +253,7 @@ __global__ void k_box_records(i64 nact, const ActRec *__restrict__ rec, const in
 #endif
 template <int PASS>
 __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, const BoxRec *__restrict__ box, GridDev g, const unsigned char *__restrict__ tile_faces, const double *__restrict__ dist,
-                                                   int prune, u64 *__restrict__ plist, u64 *__restrict__ cnt, u64 *__restrict__ stats) {
+                                                   int prune, u64 *__restrict__ seed, u64 *__restrict__ plist, u64 *__restrict__ cnt, u64 *__restrict__ stats) {
   const i64 a = (blockIdx.x * (i64)blockDim.x + threadIdx.x) >> 5; const int lane = threadIdx.x & 31;
   if (a >= nact) return;
   const int vol = box[a].vol;
@@ -282,22 +261,32 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
   const BoxRec &B = box[a];
   const int nx = B.nx, ny = B.ny, ps0 = B.ps[0], ps1 = B.ps[1], ps2 = B.ps[2];
   const bool ftile = B.ftile != 0;
-  // closed AABB of the element and tight box of its iso-patch, global coordinates.  The point coordinates are taken as amin + cell * i
-  // here (no table look-up; at most an ulp from the tabulated value): which pass a pair belongs to is free to choose, and the bound is
-  // compared with a relative margin of 1e-10.
-  double elo[3], ehi[3], tlo[3], thi[3];
+  // The point coordinates are taken as amin + cell * i here (no table look-up; at most an ulp from the tabulated value): the seed is
+  // free to choose, and the bounds are compared with a relative margin of 1e-10 (lb_box_slab's own margin covers the ulp as well).
+  double tlo[3], thi[3];
 #pragma unroll
-  for (int d = 0; d < 3; d++) {
-    const double c0 = (B.c[d] - B.h[d]) + B.org[d], c1 = (B.c[d] + B.h[d]) + B.org[d];
-    elo[d] = fmin(c0, c1); ehi[d] = fmax(c0, c1); tlo[d] = B.tlo[d]; thi[d] = B.thi[d];
-  }
-  const double sl = 1e-9 * (ehi[0] - elo[0] + ehi[1] - elo[1] + ehi[2] - elo[2]);
-  constexpr int RB = 7;      // rounds handled as one batch: all loads of a batch are issued before the first decision (32 * 7 >= 6^3 points)
-  int npruned = 0;
+  for (int d = 0; d < 3; d++) { tlo[d] = B.tlo[d]; thi[d] = B.thi[d]; }
   // local point index li = lane, lane + 32, ... -> (ci, cj, ck), advanced by 32 per round without divisions (runtime divisors cost ~25
   // instructions each and were 40 % of this kernel's instructions)
   int ci = lane % nx, cj = (lane / nx) % ny, ck = lane / (nx * ny);
   const int r32 = 32 % nx, q32 = 32 / nx, jq = q32 % ny, kq = q32 / ny;
+  if (PASS == 0) {      // seed: no list; the key is read first and the atomic only issued when it would lower it (keys only decrease,
+                        // so a stale read only costs an atomic)
+    for (int li = lane; li < vol; li += 32) {
+      const int pi0 = ps0 + ci, pi1 = ps1 + cj, pi2 = ps2 + ck;
+      { ci += r32; const int c = ci >= nx ? 1 : 0; ci -= c ? nx : 0; cj += jq + c; ck += kq; if (cj >= ny) { cj -= ny; ck++; } }
+      if (ftile && tile_faces[((i64)(pi2 / TILE_Z) * g.nt[1] + pi1 / TILE_Y) * g.nt[0] + pi0 / TILE_X] != 0) continue;
+      const double x0 = fma(g.cell, (double)pi0, g.amin[0]), x1 = fma(g.cell, (double)pi1, g.amin[1]), x2 = fma(g.cell, (double)pi2, g.amin[2]);
+      const double e0 = fmax(fmax(tlo[0] - x0, x0 - thi[0]), 0.0), e1 = fmax(fmax(tlo[1] - x1, x1 - thi[1]), 0.0), e2 = fmax(fmax(tlo[2] - x2, x2 - thi[2]), 0.0);
+      const u64 key = ((u64)__float_as_uint(__double2float_rd(sqrt(fma(e2, e2, fma(e1, e1, e0 * e0))))) << 32) | (u64)a;
+      u64 *sp = &seed[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0];
+      if (key < *sp) atomicMin((unsigned long long *)sp, key);
+    }
+    return;
+  }
+  constexpr int RB = 7;      // rounds handled as one batch: all loads of a batch are issued before the first decision (32 * 7 >= 6^3 points)
+  const bool slab = B.sA != -INFINITY;
+  int npruned = 0;
   for (int base0 = 0; base0 < vol; base0 += 32 * RB) {
     double lb2[RB], cur[RB]; int flags[RB];      // flags: bit 0 valid candidate of this pass, bit 1 to_buf, bit 2 needs the bound test
 #pragma unroll
@@ -308,26 +297,48 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
       { ci += r32; const int c = ci >= nx ? 1 : 0; ci -= c ? nx : 0; cj += jq + c; ck += kq; if (cj >= ny) { cj -= ny; ck++; } }
       if (li < vol) {
         const int pi0 = ps0 + i, pi1 = ps1 + j, pi2 = ps2 + k;
-        const double x0 = fma(g.cell, (double)pi0, g.amin[0]), x1 = fma(g.cell, (double)pi1, g.amin[1]), x2 = fma(g.cell, (double)pi2, g.amin[2]);
+        const i64 v = ((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0;
         const bool to_buf = ftile && tile_faces[((i64)(pi2 / TILE_Z) * g.nt[1] + pi1 / TILE_Y) * g.nt[0] + pi0 / TILE_X] != 0;
-        const bool inner = x0 >= elo[0] - sl && x0 <= ehi[0] + sl && x1 >= elo[1] - sl && x1 <= ehi[1] + sl && x2 >= elo[2] - sl && x2 <= ehi[2] + sl;
-        if (PASS == 0) { if (to_buf || inner || !prune) flags[r] = 1 | (to_buf ? 2 : 0); }
-        else if (!to_buf && !inner) {
+        const bool seeded = !to_buf && prune && (unsigned)seed[v] == (unsigned)a;      // this pair is its point's seed (pass A)
+        if (PASS == 1) { if (to_buf || seeded || !prune) flags[r] = 1 | (to_buf ? 2 : 0); }
+        else if (!to_buf && !seeded) {
+          const double x0 = fma(g.cell, (double)pi0, g.amin[0]), x1 = fma(g.cell, (double)pi1, g.amin[1]), x2 = fma(g.cell, (double)pi2, g.amin[2]);
           const double e0 = fmax(fmax(tlo[0] - x0, x0 - thi[0]), 0.0), e1 = fmax(fmax(tlo[1] - x1, x1 - thi[1]), 0.0), e2 = fmax(fmax(tlo[2] - x2, x2 - thi[2]), 0.0);
           lb2[r] = fma(e2, e2, fma(e1, e1, e0 * e0));
-          cur[r] = dist[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0];
+          cur[r] = dist[v];
           flags[r] = 1 | 4;
         }
       }
+    }
+    // pass B: the tight box first; the two slab bounds only for the pairs it leaves, in a rolled loop (one copy of lb_box_slab; the point
+    // and its dist[] entry, unchanged since the batch read it, are fetched again)
+    unsigned keepb = 0, need = 0;
+#pragma unroll
+    for (int r = 0; r < RB; r++) {
+      bool keep = (flags[r] & 1) != 0;
+      if (PASS == 2 && keep) {
+        if (lb2[r] > cur[r] * cur[r] * (1.0 + 1e-10)) { keep = false; npruned++; }
+        else if (slab) need |= 1u << r;
+      }
+      keepb |= (keep ? 1u : 0u) << r;
+    }
+    while (PASS == 2 && need) {
+      const int r = __ffs(need) - 1; need &= need - 1;
+      const int li = base0 + r * 32 + lane;
+      const int pi0 = ps0 + li % nx, pi1 = ps1 + (li / nx) % ny, pi2 = ps2 + li / (nx * ny);
+      const double c = dist[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0], c2 = c * c * (1.0 + 1e-10);
+      const double P[3] = {fma(g.cell, (double)pi0, g.amin[0]), fma(g.cell, (double)pi1, g.amin[1]), fma(g.cell, (double)pi2, g.amin[2])};
+      const double n[3] = {B.sn[0], B.sn[1], B.sn[2]};
+      bool prn = bnd::lb2_box_gap(P, tlo, thi, n, B.sA, B.sB) > c2;
+      if (!prn) { const double lb = bnd::lb_box_slab(P, tlo, thi, n, B.sA, B.sB); prn = lb * lb > c2; }
+      if (prn) { keepb &= ~(1u << r); npruned++; }
     }
     // ONE list-slot claim per warp and batch: a single global counter serves the whole grid, and same-address atomics retire at about one
     // per clock -- a claim per 32-point round (7 per element) made this kernel atomic-bound (ncu: 3.4 + 7.2 ms)
     unsigned keepm[RB]; int total = 0;
 #pragma unroll
     for (int r = 0; r < RB; r++) {
-      bool keep = (flags[r] & 1) != 0;
-      if (PASS == 1 && keep && lb2[r] > cur[r] * cur[r] * (1.0 + 1e-10)) { keep = false; npruned++; }
-      keepm[r] = __ballot_sync(0xffffffffu, keep);
+      keepm[r] = __ballot_sync(0xffffffffu, (keepb >> r) & 1u);
       total += __popc(keepm[r]);
     }
     if (total) {
@@ -341,7 +352,7 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
       }
     }
   }
-  if (PASS == 1) {      // statistics: spread over the 128 counter slots (summed on the host)
+  if (PASS == 2) {      // statistics: spread over the 128 counter slots (summed on the host)
     for (int o = 16; o > 0; o >>= 1) npruned += __shfl_down_sync(0xffffffffu, npruned, o);
     if (lane == 0 && npruned) atomicAdd(&stats[8 * (1 + (blockIdx.x & 127)) + 4], (u64)npruned);
   }
@@ -856,12 +867,20 @@ int r2s_dev_eval_distances(r2s_ctx *ctx, double rho_t, double delta_factor, bool
         CK(cudaEventRecord(ctx->ev_k[0], st));
         k_box_records<<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->rho_n.as<double>(), ctx->ebox.as<unsigned char>(), rho_t, g, ctx->tile_faces.as<unsigned char>(), box, ctx->counters.as<u64>() + NCTR + 4); LAUNCH_CHECK();
         const int prune = ctx->knobs.proj_prune ? 1 : 0, pgrid = 148 * R2S_PL_MINB * 4;
-        k_pair_scan<0><<<cdiv(nact * 32, 256), 256, 0, st>>>(nact, box, g, ctx->tile_faces.as<unsigned char>(), ctx->dist.as<double>(), prune, pl, pc, ctx->counters.as<u64>()); LAUNCH_CHECK();
+        u64 *seed = nullptr;
+        if (prune) {      // per-point seed keys: all ones = no pair yet
+          CK(ctx->pseed.reserve(sizeof(u64) * (size_t)g.ngp));
+          seed = ctx->pseed.as<u64>();
+          const i64 v0 = (i64)kz0 * g.np[0] * g.np[1], nv = (i64)(kz1 - kz0) * g.np[0] * g.np[1];
+          CK(cudaMemsetAsync(seed + v0, 0xff, sizeof(u64) * (size_t)nv, st));
+          k_pair_scan<0><<<cdiv(nact * 32, 256), 256, 0, st>>>(nact, box, g, ctx->tile_faces.as<unsigned char>(), ctx->dist.as<double>(), prune, seed, pl, pc, ctx->counters.as<u64>()); LAUNCH_CHECK();
+        }
+        k_pair_scan<1><<<cdiv(nact * 32, 256), 256, 0, st>>>(nact, box, g, ctx->tile_faces.as<unsigned char>(), ctx->dist.as<double>(), prune, seed, pl, pc, ctx->counters.as<u64>()); LAUNCH_CHECK();
         CK(cudaEventRecord(ctx->ev_k[1], st));
         k_project_list<<<pgrid, 128, 0, st>>>(pl, pc, box, ctx->IEN32.as<int>(), ctx->rho_n.as<double>(), g, rho_t, ctx->pairbuf.as<double>(), ctx->dist.as<double>(), ctx->counters.as<u64>()); LAUNCH_CHECK();
         CK(cudaEventRecord(ctx->ev_k[2], st));
         if (prune) {
-          k_pair_scan<1><<<cdiv(nact * 32, 256), 256, 0, st>>>(nact, box, g, ctx->tile_faces.as<unsigned char>(), ctx->dist.as<double>(), prune, pl, pc + 2, ctx->counters.as<u64>()); LAUNCH_CHECK();
+          k_pair_scan<2><<<cdiv(nact * 32, 256), 256, 0, st>>>(nact, box, g, ctx->tile_faces.as<unsigned char>(), ctx->dist.as<double>(), prune, seed, pl, pc + 2, ctx->counters.as<u64>()); LAUNCH_CHECK();
           CK(cudaEventRecord(ctx->ev_k[3], st));
           k_project_list<<<pgrid, 128, 0, st>>>(pl, pc + 2, box, ctx->IEN32.as<int>(), ctx->rho_n.as<double>(), g, rho_t, ctx->pairbuf.as<double>(), ctx->dist.as<double>(), ctx->counters.as<u64>()); LAUNCH_CHECK();
         } else CK(cudaEventRecord(ctx->ev_k[3], st));

@@ -7,12 +7,18 @@ element's iso-patch -- is not below the point's final minimum cannot change the 
 the bench workload, how many pairs survive (a) best-first pruning per grid point with the element AABB as the box, (b) the
 same with the tight box of the iso-patch (sub-boxes of the element whose 8 corner densities straddle rho_t: a trilinear
 field takes its extrema over a box at the corners, so the other sub-boxes hold no iso-surface), and the iteration statistics
-a warp of 32 lanes sees.  Uses the host build of the projection solver (tests/host/libiso_host.so)."""
+a warp of 32 lanes sees.  Uses the host build of the projection solver (tests/host/libiso_host.so).
+
+The last block counts the schemes of the device's pair scans with the device's own rules (host build of rho2sdf.jl_b200/csrc/r2s_bound.cuh,
+tests/host/bound_host.cpp): the tight box of k_box_records, the slab that holds the iso-patch, the distance to box /\ slab, and how pass A
+is chosen (pairs inside the element's box, or one pair per point with the smallest bound).  Solver iterations are those of the kernel's
+path (element phase 1, FAST restoration)."""
 import argparse, ctypes as C, os, subprocess, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 from fixtures import Grid, simp_hex8
+import bound_ref
 import oracle
 
 
@@ -66,6 +72,7 @@ def main():
     pc = [g.AABB_min[d] + g.cell_size * np.arange(np_ax[d]) for d in range(3)]
     best = np.full(int(g.ngp), np.inf)
     recs = []           # (voxel ids, dist, lb_aabb, lb_tight, its)
+    dev = []            # device rules: (voxel ids, dist, its, lb tight box, lb slab only, lb box /\ slab, element index)
     for e in crossing:
         Xe = X[IEN[e] - 1]; re = re_all[e]
         lo, hi = Xe.min(0), Xe.max(0)
@@ -85,6 +92,14 @@ def main():
         assert np.all(lbt <= dist * (1 + 1e-9) + 1e-12), (e, float((lbt - dist).max()))
         np.minimum.at(best, vox, dist)
         recs.append((vox, dist, lb, lbt, its))
+        rec = bound_ref.element(Xe, re, rho_t)
+        dd, _, itd = bound_ref.project(Xe, re, rho_t, P)
+        lbx = np.linalg.norm(np.maximum(np.maximum(rec[0:3] - P, P - rec[3:6]), 0), axis=1)
+        t = P @ rec[6:9]
+        lbsl = np.maximum(np.maximum(rec[9] - t, t - rec[10]), 0) if np.isfinite(rec[9]) else np.zeros(len(P))
+        lbs = bound_ref.lb(P, rec)
+        assert np.all(lbs <= dd), e
+        dev.append((vox, dd, itd, lbx, lbsl, lbs, np.full(len(P), len(dev))))
     vox = np.concatenate([r[0] for r in recs]); dist = np.concatenate([r[1] for r in recs]); lb = np.concatenate([r[2] for r in recs])
     lbt = np.concatenate([r[3] for r in recs]); its = np.concatenate([r[4] for r in recs])
     npairs = len(vox); band = int(np.isfinite(best).sum())
@@ -149,6 +164,43 @@ def main():
         need_a.sum(), 100 * need_a.mean(), need_t.sum(), 100 * need_t.mean()))
     print("best-first per grid point with the tight box: %d projections (%.1f%% of the pairs, %.2f per band point; p50 %d p90 %d max %d), %.1f%% of the iterations" % (
         done, 100 * done / npairs, done / band, *np.percentile(per_vox, [50, 90]).astype(int), per_vox.max(), 100 * iters_bf / its.sum()))
+    device_schemes(dev, inA, int(g.ngp))
+
+
+def device_schemes(dev, inner, ngp):
+    """inner: the point lies in the element's box (today's pass A)"""
+    vox, dist, its, lbx, lbsl, lbs, eid = (np.concatenate([r[k] for r in dev]) for k in range(7))
+    final = np.full(ngp, np.inf); np.minimum.at(final, vox, dist)
+    npairs, itall = len(vox), its.sum()
+
+    def two_pass(seedA, bound):
+        cur = np.full(ngp, np.inf); np.minimum.at(cur, vox[seedA], dist[seedA])
+        keepB = ~seedA & ~(bound ** 2 > cur[vox] ** 2 * (1 + 1e-10))
+        assert np.all(dist[~(seedA | keepB)] >= final[vox[~(seedA | keepB)]])
+        solved = seedA | keepB
+        return 100 * solved.mean(), 100 * its[solved].sum() / itall
+
+    f = lbs.astype(np.float32)
+    f = np.where(f.astype(np.float64) > lbs, np.nextafter(f, np.float32(-np.inf)), f)
+    order = np.lexsort((eid, f, vox)); first = np.r_[True, vox[order][1:] != vox[order][:-1]]
+    seed = np.zeros(npairs, bool); seed[order[first]] = True
+    print("device rules (pairs solved, solver iterations; boundary-face tiles not modelled):")
+    for name, A, b in (("pass A = pairs inside the element box, pass B by the tight box", inner, lbx),
+                       ("pass A = inner, bound = max(tight box, slab)", inner, np.maximum(lbx, lbsl)),
+                       ("pass A = inner, bound = distance to box /\\ slab", inner, lbs),
+                       ("pass A = inner + per-point seed, bound = box /\\ slab", inner | seed, lbs),
+                       ("pass A = per-point seed (smallest bound), bound = box /\\ slab  [the kernels]", seed, lbs)):
+        print("  %-80s %5.1f%% %5.1f%%" % ((name,) + two_pass(A, b)))
+    order = np.lexsort((lbs, vox)); vs, ds, ls, it_s = vox[order], dist[order], lbs[order], its[order]
+    starts = np.r_[0, np.nonzero(np.diff(vs))[0] + 1, len(vs)]
+    done = iters = 0
+    for a, b in zip(starts[:-1], starts[1:]):
+        cur = np.inf
+        for q in range(a, b):
+            if ls[q] ** 2 > cur ** 2 * (1 + 1e-10):
+                break
+            cur = min(cur, ds[q]); done += 1; iters += int(it_s[q])
+    print("  %-80s %5.1f%% %5.1f%%" % ("floor: best-first per point with box /\\ slab", 100 * done / npairs, 100 * iters / itall))
 
 
 if __name__ == "__main__":
