@@ -79,6 +79,30 @@ int r2s_find_threshold(r2s_ctx *ctx, const double *rho_n, double target_volume, 
 int r2s_eval_distances(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, double *dist, double *xp);
 /* Sign_Detection (src/SignedDistances/SignDetection.jl:275-283): signs[ngp] in {-1,+1} */
 int r2s_sign_detection(r2s_ctx *ctx, const double *rho_n, double rho_t, double *signs);
+/* evalDistances / Sign_Detection at arbitrary points (csrc/r2s_points.cu): the reference's `points` argument, which it bins with
+ * LinkedList(grid, points) (Grid.jl:47-69).  r2s_set_mesh and r2s_set_grid must have been called: the grid is the frame of the binning.
+ * Points are double, x y z per point (Julia's 3 x n; Python's (n, 3) like generateGridPoints).
+ *   distances: a point's cell per axis is c_d = floor(N_d (x_d - amin_d) / (amax_d - amin_d)) (the reference's cell expression, every
+ *     operation rounded, not clamped).  An element, and each of its boundary-face triangles, considers the point iff c lies in its
+ *     clamped cell range (calculateMiniAABB_grid, Grid.jl:122-154, AABB +- delta_factor * cell_size) on all three axes.  The value is the
+ *     reference's running minimum over the elements in ascending index -- boundary faces before the iso projection
+ *     (process_isocontour_element!), the strict < of WriteValue, xp from the first writer -- and dist = |value|.  A point that no element
+ *     considers gets 1e10 and xp = 0; in particular every point whose cell lies outside [0, N_d] on some axis (this library's rule for
+ *     points outside the grid).  For the grid's own points the rule is the grid path's: their cells are the cells r2s_eval_distances uses.
+ *   signs: SignDetection.jl per point.  HEX8: the candidates are the elements whose closed AABB contains the point, in ascending index;
+ *     TET4: the elements of the padded per-cell lists of create_grid_tetrahedra_mapping_TET4 for the point's cell point_to_grid_index =
+ *     clamp(floor((x - amin) / cell_size) + 1, 1, N + 1).  A point without a candidate gets -1.
+ * The results are a function of the point alone: independent of the order of the points, of chunking, and of a slab set with
+ * r2s_set_slab (element ranges are never clipped); any context works, a slab rank or r2s_multi_context(m, 0) too (the call is local to
+ * it).  Host arrays pass through a bounded device buffer in chunks of 2^22 points.  The call leaves the resident results as it found them
+ * (sdf_dists, fine_sdf, the smoothing weights and th, an isosurface, the nodal densities of r2s_upload_nodal_densities): it uploads rho_n
+ * into buffers of its own.  Rejected with an error: non-finite coordinates, n < 0, n > 0 with a NULL array, no mesh, no grid.
+ * Report (r2s_last_report): the distance call sets n_solid, n_crossing, n_active, n_pairs ((crossing element, point) pairs whose range
+ * holds the point), n_pairs_pruned (those skipped by a lower bound), n_newton_iters, n_not_converged, ms_bin and ms_project (the whole
+ * call); the sign call sets ms_bin and ms_sign (the whole call).  R2S_PROJ_PRUNE=0 turns the bound pruning off (same bits). */
+int r2s_eval_distances_points(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, const double *points, int64_t n, double *dist,
+                              double *xp /* 3 * n or NULL */);
+int r2s_sign_detection_points(r2s_ctx *ctx, const double *rho_n, double rho_t, const double *points, int64_t n, double *signs);
 /* remove_sdf_artifacts! (src/SignedDistances/SdfArtifactRemoval.jl:134-245): sdf[ngp] in/out */
 int r2s_remove_artifacts(r2s_ctx *ctx, double *sdf, double threshold, double min_component_ratio, int64_t *flipped);
 /* RBFs_smoothing (src/SdfSmoothing/RBFs4Smoothing.jl:321-377): fine_sdf[prod(N*smooth+1)], x fastest */

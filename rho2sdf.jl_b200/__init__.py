@@ -97,6 +97,8 @@ def load_library():
     L.r2s_find_threshold.argtypes = [vp, vp, C.c_double, C.c_double, C.c_int, dp]
     L.r2s_eval_distances.argtypes = [vp, vp, C.c_double, C.c_double, vp, vp]
     L.r2s_sign_detection.argtypes = [vp, vp, C.c_double, vp]
+    L.r2s_eval_distances_points.argtypes = [vp, vp, C.c_double, C.c_double, vp, C.c_int64, vp, vp]
+    L.r2s_sign_detection_points.argtypes = [vp, vp, C.c_double, vp, C.c_int64, vp]
     L.r2s_remove_artifacts.argtypes = [vp, vp, C.c_double, C.c_double, ip]
     L.r2s_rbf_smoothing.argtypes = [vp, vp, C.c_int, C.c_int, C.c_double, C.c_double, vp, fp, fp]
     L.r2s_volume_from_sdf.argtypes = [vp, vp, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_float, C.c_int, dp]
@@ -445,17 +447,28 @@ def find_threshold_for_volume(mesh, nodal_values, tolerance=1e-4, max_iterations
 # ---------------------------------------------------------------------------------------------------------------------
 # SignedDistances
 # ---------------------------------------------------------------------------------------------------------------------
-def _check_points(grid, points):
-    if points is not None and np.shape(points)[0] != grid.ngp:
-        raise R2SError("points must hold grid.ngp columns (generateGridPoints(grid))")
+def _points(points):
+    p = np.ascontiguousarray(points, dtype=np.float64)
+    if p.ndim != 2 or p.shape[1] != 3:
+        raise R2SError("points must be an (n, 3) array")
+    return p
 
 
 def evalDistances(mesh, grid, points, rho_n, rho_t, delta_factor=1.1, want_xp=True):
-    """src/SignedDistances/sdfOnDensityField.jl:139-486 -> (dists, xp).  `delta_factor` is the reference's hard-wired 1.1 (:158)."""
-    _check_points(grid, points)
+    """src/SignedDistances/sdfOnDensityField.jl:139-486 -> (dists, xp).  `delta_factor` is the reference's hard-wired 1.1 (:158).
+    points=None: at the grid's points (grid.ngp values).  points = (n, 3) float64: at those points, binned in the grid's frame like the
+    reference's LinkedList(grid, points) -- (n,) and (n, 3); the rule (and what points outside the grid get) is stated in include/r2s.h."""
     mesh._use_grid(grid)
     c = mesh.ctx
     rn = _f64(rho_n)
+    if points is not None:
+        p = _points(points)
+        n = p.shape[0]
+        dist = np.empty(n)
+        xp = np.zeros((n, 3)) if want_xp else None
+        c.check(c.lib.r2s_eval_distances_points(c.h, _ptr(rn), float(rho_t), float(delta_factor), _ptr(p) if n else None, n, _ptr(dist) if n else None,
+                                                _ptr(xp) if (want_xp and n) else None))
+        return dist, xp
     dist = np.empty(grid.ngp)
     xp = np.zeros((grid.ngp, 3)) if want_xp else None
     c.check(c.lib.r2s_eval_distances(c.h, _ptr(rn), float(rho_t), float(delta_factor), _ptr(dist), _ptr(xp) if want_xp else None))
@@ -463,11 +476,17 @@ def evalDistances(mesh, grid, points, rho_n, rho_t, delta_factor=1.1, want_xp=Tr
 
 
 def Sign_Detection(mesh, grid, points, rho_n, rho_t):
-    """src/SignedDistances/SignDetection.jl:275-283 -> signs in {-1, +1}."""
-    _check_points(grid, points)
+    """src/SignedDistances/SignDetection.jl:275-283 -> signs in {-1, +1}.  points=None: at the grid's points; (n, 3) float64: at those
+    points -> (n,)."""
     mesh._use_grid(grid)
     c = mesh.ctx
     rn = _f64(rho_n)
+    if points is not None:
+        p = _points(points)
+        n = p.shape[0]
+        s = np.empty(n)
+        c.check(c.lib.r2s_sign_detection_points(c.h, _ptr(rn), float(rho_t), _ptr(p) if n else None, n, _ptr(s) if n else None))
+        return s
     s = np.empty(grid.ngp)
     c.check(c.lib.r2s_sign_detection(c.h, _ptr(rn), float(rho_t), _ptr(s)))
     return s

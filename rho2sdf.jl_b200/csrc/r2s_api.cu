@@ -42,7 +42,9 @@ void r2s_destroy(r2s_ctx *ctx) {
                    &ctx->counters, &ctx->box_rec, &ctx->plist, &ctx->dist, &ctx->xp, &ctx->sdf, &ctx->signs, &ctx->s_rng, &ctx->s_el, &ctx->s_cnt, &ctx->s_keys, &ctx->s_keys_alt, &ctx->s_tile_ptr,
                    &ctx->cc_label, &ctx->cc_size, &ctx->cc_scal, &ctx->cc_bits, &ctx->cc_bits_all, &ctx->cc_gsz, &ctx->cc_seen, &ctx->f_s, &ctx->f_w, &ctx->f_r, &ctx->f_u, &ctx->f_c, &ctx->f_lsf, &ctx->f_fine, &ctx->f_part,
                    &ctx->f_scal, &ctx->cutlist, &ctx->slablist, &ctx->v_part, &ctx->vlist[0], &ctx->vlist[1], &ctx->vent[0], &ctx->vent[1], &ctx->vrec, &ctx->bis_state, &ctx->lat_xs, &ctx->lat_cell, &ctx->lat_map, &ctx->lat_info, &ctx->lat_pt,
-                   &ctx->surf_rows, &ctx->surf_V, &ctx->surf_T, &ctx->rbf_tab, &ctx->smp_in, &ctx->smp_out};
+                   &ctx->surf_rows, &ctx->surf_V, &ctx->surf_T, &ctx->rbf_tab, &ctx->smp_in, &ctx->smp_out, &ctx->pt_rn, &ctx->pt_cls, &ctx->pt_flag, &ctx->pt_idx,
+                   &ctx->pt_rec, &ctx->pt_hex, &ctx->pt_cnt, &ctx->pt_off, &ctx->pt_tkeys, &ctx->pt_tkeys_alt, &ctx->pt_tile_ptr, &ctx->pt_tri, &ctx->pt_in, &ctx->pt_keys, &ctx->pt_keys_alt,
+                   &ctx->pt_out, &ctx->pt_ctr};
   for (DevBuf *b : all) b->release();
   for (int i = 0; i < 16; i++) cudaEventDestroy(ctx->ev[i]);
   for (int i = 0; i < 5; i++) { cudaEventDestroy(ctx->ev_probe[i]); cudaEventDestroy(ctx->ev_k[i]); }

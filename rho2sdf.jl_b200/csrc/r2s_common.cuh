@@ -118,6 +118,9 @@ struct r2s_ctx {
   // distance / sign work buffers
   DevBuf cls, act_flag, act_idx, act_rec, cnt_a, cnt_b, keys, keys_alt, tile_ptr, tile_faces, face_tiles, fc_list, tri_cnt, tri_rec, pairbuf, pairxp, cubtmp, counters, box_rec, plist, pseed;
   DevBuf dist, xp, sdf, signs;
+  // evalDistances / Sign_Detection at arbitrary points (r2s_points.cu): own nodal densities and scratch, so a points call leaves every
+  // resident result (sdf, fine_sdf, smoothing weights, isosurface, the uploaded rho_n) as it found it
+  DevBuf pt_rn, pt_cls, pt_flag, pt_idx, pt_rec, pt_hex, pt_cnt, pt_off, pt_tkeys, pt_tkeys_alt, pt_tile_ptr, pt_tri, pt_in, pt_keys, pt_keys_alt, pt_out, pt_ctr;
   DevBuf s_rng, s_el, s_cnt, s_keys, s_keys_alt, s_tile_ptr;
   // connected components
   DevBuf cc_label, cc_size, cc_scal, cc_bits, cc_bits_all, cc_gsz, cc_seen;
@@ -220,6 +223,9 @@ int r2s_sample_points_ctx(r2s_ctx *ctx, const double *pts, i64 n, float *val, fl
 int r2s_sample_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float o[3], float h[3]);
 int r2s_sample_lattice_planes(r2s_ctx *ctx, const float o[3], const float h[3], const int64_t dims[3], i64 ka, i64 kb, float *out);
 int r2s_sample_download_weights(r2s_ctx *ctx, float *w, float *th, i64 k0, i64 k1);
+// r2s_points.cu: evalDistances / Sign_Detection at n host points (rho_n on the host)
+int r2s_points_distances(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, const double *pts, i64 n, double *dist, double *xp);
+int r2s_points_signs(r2s_ctx *ctx, const double *rho_n, double rho_t, const double *pts, i64 n, double *signs);
 // in-process groups (r2s_multi.cu drives them): one context per slab, one host thread per context
 LocalGroup *r2s_local_group_create(r2s_ctx **ctxs, int n, std::string *err);
 void r2s_local_group_destroy(LocalGroup *g);

@@ -604,3 +604,6 @@ __device__ inline bool project_tet4(const double Xe[3][4], const double re[4], c
   return best < INFINITY;
 }
 }  // namespace iso
+
+// solver variant the distance kernels use (r2s_dist.cu, r2s_points.cu): FAST restoration, one code path for all tangent-step cases
+#define PMODE 3

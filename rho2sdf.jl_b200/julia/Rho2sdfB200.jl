@@ -7,7 +7,7 @@
 module Rho2sdfB200
 
 using Rho2sdf                      # the reference package: Mesh, Grid, Rho2sdfOptions, HEX8/TET4, grid set-up, exports
-using Rho2sdf.MeshGrid: Mesh, Grid
+using Rho2sdf.MeshGrid: Mesh, Grid, generateGridPoints
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
@@ -80,17 +80,33 @@ function find_threshold_for_volume(mesh::Mesh, nodal_values::Vector{Float64}; to
 end
 
 # ---- src/SignedDistances/sdfOnDensityField.jl:139-486 ---------------------------------------------------------------------
+# points = the grid's own point set: the grid entry point (faster, same result); any other 3 x n points: the points entry point, binned in
+# the grid's frame like the reference's LinkedList(grid, points) (rule in include/r2s.h)
+is_grid_points(grid::Grid, points::Matrix{Float64}) = size(points, 2) == grid.ngp && points == generateGridPoints(grid)
 function evalDistances(mesh::Mesh, grid::Grid, points::Matrix{Float64}, ρₙ::Vector{Float64}, ρₜ::Float64; delta_factor::Float64=1.1)
   c = context(mesh); use_grid(c, grid)
-  dist = Vector{Float64}(undef, grid.ngp); xp = zeros(Float64, 3, grid.ngp)
-  check(c, ccall((:r2s_eval_distances, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}), c.h, ρₙ, ρₜ, delta_factor, dist, xp))
+  if is_grid_points(grid, points)
+    dist = Vector{Float64}(undef, grid.ngp); xp = zeros(Float64, 3, grid.ngp)
+    check(c, ccall((:r2s_eval_distances, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Cdouble, Ptr{Cdouble}, Ptr{Cdouble}), c.h, ρₙ, ρₜ, delta_factor, dist, xp))
+    return dist, xp
+  end
+  size(points, 1) == 3 || error("points must be a 3 x n matrix")
+  n = size(points, 2); dist = Vector{Float64}(undef, n); xp = zeros(Float64, 3, n)
+  check(c, ccall((:r2s_eval_distances_points, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Cdouble, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}),
+                 c.h, ρₙ, ρₜ, delta_factor, points, n, dist, xp))
   return dist, xp
 end
 # ---- src/SignedDistances/SignDetection.jl:275-283 -----------------------------------------------------------------------
 function Sign_Detection(mesh::Mesh, grid::Grid, points::Matrix{Float64}, ρₙ::Vector{Float64}, ρₜ::Float64)
   c = context(mesh); use_grid(c, grid)
-  signs = Vector{Float64}(undef, grid.ngp)
-  check(c, ccall((:r2s_sign_detection, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}), c.h, ρₙ, ρₜ, signs))
+  if is_grid_points(grid, points)
+    signs = Vector{Float64}(undef, grid.ngp)
+    check(c, ccall((:r2s_sign_detection, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}), c.h, ρₙ, ρₜ, signs))
+    return signs
+  end
+  size(points, 1) == 3 || error("points must be a 3 x n matrix")
+  n = size(points, 2); signs = Vector{Float64}(undef, n)
+  check(c, ccall((:r2s_sign_detection_points, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Cdouble, Ptr{Cdouble}, Int64, Ptr{Cdouble}), c.h, ρₙ, ρₜ, points, n, signs))
   return signs
 end
 # ---- src/SignedDistances/SdfArtifactRemoval.jl:134-245 ------------------------------------------------------------------
