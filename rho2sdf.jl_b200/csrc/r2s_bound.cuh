@@ -1,5 +1,6 @@
 // r2s_bound.cuh -- lower bounds of the distance from a grid point to the iso-patch of an axis-aligned box element, shared by the pair
-// scans of the box projection (r2s_dist.cu) and compiled for the host by tests/host/bound_host.cpp.
+// scans of the box projection (r2s_dist.cu) and the points path (r2s_points.cu), with the per-element set-up of the HEX8 projection, and
+// compiled for the host by tests/host/bound_host.cpp.
 //
 // The element maps xi in [-1, 1]^3 to X_d = org_d + c_d + h_d xi_d; rho - rho_t is trilinear in xi.  box_iso_bounds gives two sets that
 // contain every point the solver (r2s_iso.cuh) can return for the element, i.e. every point of the element where |rho - rho_t| is at
@@ -29,6 +30,7 @@
 // (n = 0, A = -inf, B = +inf): lb_box_slab is then the distance to the tight box.
 #pragma once
 #include <math.h>
+#include "r2s_iso.cuh"
 
 #ifndef R2S_HD
 #if defined(__CUDACC__)
@@ -168,6 +170,55 @@ R2S_HD double lb_box_slab(const double P[3], const double tlo[3], const double t
   const double e0 = y[0] - P[0], e1 = y[1] - P[1], e2 = y[2] - P[2];
   const double dist = sqrt(e0 * e0 + e1 * e1 + e2 * e2);
   return fmax(0.0, dist * (1.0 - 1e-14) - dlt);
+}
+
+// The pair bound against box /\ slab: true if the distance from P to it, squared, exceeds the running value c squared with a relative margin
+// of 1e-10 (the scans take P as amin + cell i, an ulp or so from the tabulated point) -- the gap bound first, lb_box_slab only if it fails
+R2S_HD bool box_slab_prunes(const double P[3], const double tlo[3], const double thi[3], const double n[3], double A, double B, double c) {
+  const double c2 = c * c * (1.0 + 1e-10);
+  if (lb2_box_gap(P, tlo, thi, n, A, B) > c2) return true;
+  const double lb = lb_box_slab(P, tlo, thi, n, A, B);
+  return lb * lb > c2;
+}
+
+// The per-element set-up of a crossing HEX8 element's projection (k_box_records, the points path's solver records): node 0 subtracted
+// from the coordinates, the monomial coefficients A of the local x, y, z and of rho, the tolerance scale gs, phase 1 (Newton projection of
+// xi = 0 onto the iso-surface: xi0, ok0) and, for a box element (iso::HexBox), the tight box and slab of its iso-patch; otherwise (general
+// trilinear element, iso::HexTri) an unbounded box and slab.  nv: x, y, z and rho of the 8 nodes; the coordinates become element-local.
+struct __align__(16) HexSetup {
+  double A[4][8];
+  double org[3], xi0[3], gs;
+  double tlo[3], thi[3], sn[3], sA, sB;      // global coordinates
+  int box, ok0;
+};
+__device__ inline void hex8_setup(double nv[4][8], double rho_t, bool box, HexSetup &P) {
+#pragma unroll
+  for (int d = 0; d < 3; d++) {
+    P.org[d] = nv[d][0];
+#pragma unroll
+    for (int k = 0; k < 8; k++) nv[d][k] -= P.org[d];
+  }
+#pragma unroll
+  for (int c = 0; c < 4; c++) iso::monomial8(nv[c], P.A[c]);
+  double gs = fabs(rho_t);
+#pragma unroll
+  for (int k = 0; k < 8; k++) gs = fmax(gs, fabs(nv[3][k]));
+  P.gs = fmax(gs, 1.0);
+  P.box = box ? 1 : 0;
+  iso::ProjState S0;
+  if (box) {
+    iso::HexBox H; iso::make_box(P.A, H);
+    P.ok0 = iso::proj_init_element<iso::HexBox, PMODE>(H, rho_t, P.gs, S0) ? 1 : 0;
+    box_iso_bounds(nv[3], rho_t, P.gs, P.org, H.c, H.h, P.tlo, P.thi, P.sn, P.sA, P.sB);
+  } else {
+    iso::HexTri H; H.A = P.A;
+    P.ok0 = iso::proj_init_element<iso::HexTri, PMODE>(H, rho_t, P.gs, S0) ? 1 : 0;
+#pragma unroll
+    for (int d = 0; d < 3; d++) { P.tlo[d] = -INFINITY; P.thi[d] = INFINITY; P.sn[d] = 0.0; }
+    P.sA = -INFINITY; P.sB = INFINITY;
+  }
+#pragma unroll
+  for (int d = 0; d < 3; d++) P.xi0[d] = S0.xi[d];
 }
 
 }  // namespace bnd

@@ -118,9 +118,10 @@ struct r2s_ctx {
   // distance / sign work buffers
   DevBuf cls, act_flag, act_idx, act_rec, cnt_a, cnt_b, keys, keys_alt, tile_ptr, tile_faces, face_tiles, fc_list, tri_cnt, tri_rec, pairbuf, pairxp, cubtmp, counters, box_rec, plist, pseed;
   DevBuf dist, xp, sdf, signs;
-  // evalDistances / Sign_Detection at arbitrary points (r2s_points.cu): own nodal densities and scratch, so a points call leaves every
-  // resident result (sdf, fine_sdf, smoothing weights, isosurface, the uploaded rho_n) as it found it
-  DevBuf pt_rn, pt_cls, pt_flag, pt_idx, pt_rec, pt_hex, pt_cnt, pt_off, pt_tkeys, pt_tkeys_alt, pt_tile_ptr, pt_tri, pt_in, pt_keys, pt_keys_alt, pt_out, pt_ctr;
+  // evalDistances / Sign_Detection at arbitrary points (r2s_points.cu): own nodal densities and point buffers, so a points call leaves every
+  // resident result (sdf, fine_sdf, smoothing weights, isosurface, the uploaded rho_n) as it found it; it bins in the grid calls' scratch
+  // above, which those rewrite before they read it
+  DevBuf pt_rn, pt_hex, pt_in, pt_keys, pt_keys_alt, pt_out, pt_ctr;
   DevBuf s_rng, s_el, s_cnt, s_keys, s_keys_alt, s_tile_ptr;
   // connected components
   DevBuf cc_label, cc_size, cc_scal, cc_bits, cc_bits_all, cc_gsz, cc_seen;
@@ -179,6 +180,12 @@ int r2s_dev_mesh_volume(r2s_ctx *ctx, double *vd, double *vf);             // r2
 int r2s_dev_nodal_densities(r2s_ctx *ctx);                                 // r2s_mesh.cu (rho_e -> rho_n, device)
 int r2s_dev_isocontour_volume(r2s_ctx *ctx, double thr, double *vol);      // r2s_mesh.cu
 int r2s_dev_eval_distances(r2s_ctx *ctx, double rho_t, double delta_factor, bool want_xp);   // r2s_dist.cu -> ctx->dist (,xp)
+// r2s_dist.cu: the element binning of evalDistances, shared by the grid and the points path.  Classifies with the nodal densities rn (class
+// counters in counters[0], [1]), gives every active element the candidate range of its AABB +- delta and builds act_rec, tri_rec and the
+// per-tile lists (tile_ptr, *sorted).  Grid mode (cells = false): grid-point ranges clipped to the planes [k0, k1), elements outside this
+// slab's z interval left inactive; also the pair offsets and counts, tile_faces and fc_list.  Cell mode: cell ranges over the whole grid.
+struct DistBins { i64 nact, npairs, nitems; u64 *sorted; };
+int r2s_dist_bins(r2s_ctx *ctx, const double *rn, double rho_t, double delta, bool cells, DistBins *b);
 int r2s_dev_sign(r2s_ctx *ctx, double rho_t, bool write_signs, bool write_sdf);              // r2s_sign.cu -> ctx->signs / ctx->sdf
 int r2s_dev_remove_artifacts(r2s_ctx *ctx, double thr, double ratio, i64 *flipped);          // r2s_cc.cu on ctx->sdf
 int r2s_dev_rbf(r2s_ctx *ctx, int is_interp, int smooth, double rbf_cut, double target, bool final_volume, float *th, float *vol);   // r2s_rbf.cu: ctx->sdf -> ctx->f_fine
@@ -186,6 +193,9 @@ int r2s_dev_volume_from_sdf(r2s_ctx *ctx, const float *sdf_dev, i64 nx, i64 ny, 
 int r2s_scan_exclusive_i64(r2s_ctx *ctx, const i64 *in, i64 *out, i64 n);  // r2s_util.cu (cub)
 int r2s_scan_exclusive_i32(r2s_ctx *ctx, const int *in, int *out, i64 n);
 int r2s_sort_keys_u64(r2s_ctx *ctx, u64 *keys, u64 *alt, i64 n, int end_bit, u64 **sorted);
+// per-tile lists from nkeys (tile << 32 | id) keys: sorts them (*sorted = whichever of keys / alt holds the result), then turns the tile
+// counts at tile_ptr[1 .. ntiles] into offsets tile_ptr[0 .. ntiles] (scratch: ctx->s_cnt)
+int r2s_tile_lists(r2s_ctx *ctx, u64 *keys, u64 *alt, i64 nkeys, int *tile_ptr, u64 **sorted);
 int r2s_sort_f64(r2s_ctx *ctx, double *keys, double *alt, i64 n, double **sorted);
 int r2s_unique_f64(r2s_ctx *ctx, const double *sorted, double *out, i64 n, i64 *count);      // distinct values of a sorted array
 // read-backs through the mapped buffer: rb_put enqueues a copy of `bytes` at src_dev and returns its offset (or (size_t)-1), rb_sync
@@ -232,6 +242,26 @@ void r2s_local_group_destroy(LocalGroup *g);
 void r2s_local_group_abort(LocalGroup *g);      // a rank failed: wake everybody waiting at a host barrier
 
 #ifdef __CUDACC__
+// ---- tiles of the binning steps ---------------------------------------------------------------------------------------------------
+// tile of grid point (or cell, or 0-based bin) (c0, c1, c2)
+__device__ __forceinline__ i64 tile_of(const GridDev &g, int c0, int c1, int c2) {
+  return ((i64)(c2 / TILE_Z) * g.nt[1] + c1 / TILE_Y) * g.nt[0] + c0 / TILE_X;
+}
+// the tiles an inclusive, 0-based index range [lo, hi] per axis overlaps: how many, and each of them in ascending order
+__device__ __forceinline__ i64 tile_span(const int lo[3], const int hi[3]) {
+  return (i64)(hi[0] / TILE_X - lo[0] / TILE_X + 1) * (hi[1] / TILE_Y - lo[1] / TILE_Y + 1) * (hi[2] / TILE_Z - lo[2] / TILE_Z + 1);
+}
+template <class F>
+__device__ __forceinline__ void for_tiles(const GridDev &g, const int lo[3], const int hi[3], F f) {
+  for (int tz = lo[2] / TILE_Z; tz <= hi[2] / TILE_Z; tz++)
+    for (int ty = lo[1] / TILE_Y; ty <= hi[1] / TILE_Y; ty++)
+      for (int tx = lo[0] / TILE_X; tx <= hi[0] / TILE_X; tx++) f(((u64)tz * g.nt[1] + ty) * g.nt[0] + tx);
+}
+// the (tile << 32 | id) key of every tile of [lo, hi] from keys[0] on, counted in tile_cnt[tile]
+__device__ __forceinline__ void emit_tile_keys(const GridDev &g, const int lo[3], const int hi[3], i64 id, u64 *__restrict__ keys, int *__restrict__ tile_cnt) {
+  for_tiles(g, lo, hi, [&](u64 t) { *keys++ = (t << 32) | (u64)id; atomicAdd(&tile_cnt[t], 1); });
+}
+
 // ---- warp-private staging of list entries in shared memory ------------------------------------------------------------------------
 // Every device-built list (pairs, cut cells, active cells, cells to evaluate, hard sign points) is appended to through ONE global counter.  Same-address atomics
 // retire at about one per clock, so a claim per 32-lane round makes a kernel atomic-bound (measured: k_vol_rows, k_vl_step, k_pair_scan).

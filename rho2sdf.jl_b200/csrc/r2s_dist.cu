@@ -44,10 +44,12 @@ __global__ void k_classify(i64 nel, int nen, const int *__restrict__ IEN, const 
   __syncthreads();
   if (threadIdx.x == 0) { if (s1) atomicAdd((u64 *)&counts[0], (u64)s1); if (s2) atomicAdd((u64 *)&counts[1], (u64)s2); }
 }
-// compacted active list: record with point ranges, tile count, pair count
-__global__ void k_act_records(i64 nel, int nen, const int *__restrict__ IEN, const double *__restrict__ X, const unsigned char *__restrict__ cls,
+// compacted active list: record with its candidate range, tile and triangle counts; grid mode (CELLS = false): grid-point ranges
+// [cstart[I0], cstart[I1 + 1]) clipped to the planes [kz0, kz1), and the pair and chunk counts; cell mode: the cell ranges [I0, I1 + 1)
+template <bool CELLS>
+__global__ void k_act_records(i64 nel, int nen, int nsn, const int *__restrict__ IEN, const double *__restrict__ X, const unsigned char *__restrict__ cls,
                               const unsigned char *__restrict__ fb, const int *__restrict__ flag, const int *__restrict__ idx, GridDev g, double delta,
-                              int kz0, int kz1, ActRec *__restrict__ rec, i64 *__restrict__ ntile, i64 *__restrict__ npair, i64 *__restrict__ nchunk) {
+                              int kz0, int kz1, ActRec *__restrict__ rec, i64 *__restrict__ ntile, int *__restrict__ ntri, i64 *__restrict__ npair, i64 *__restrict__ nchunk) {
   i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (e >= nel || !flag[e]) return;
   double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
@@ -57,37 +59,33 @@ __global__ void k_act_records(i64 nel, int nen, const int *__restrict__ IEN, con
   for (int d = 0; d < 3; d++) {
     int I0 = 0, I1 = -1;
     ok = ok && ex::cell_range_axis(lo[d], hi[d], delta, g.amin[d], g.amax[d], g.N[d], I0, I1);
-    if (ok) { r.ps[d] = g.cstart[g.cs_off[d] + I0]; r.pe[d] = g.cstart[g.cs_off[d] + I1 + 1]; } else { r.ps[d] = 0; r.pe[d] = 0; }
+    if (!ok) { r.ps[d] = 0; r.pe[d] = 0; }
+    else if (CELLS) { r.ps[d] = I0; r.pe[d] = I1 + 1; }
+    else { r.ps[d] = g.cstart[g.cs_off[d] + I0]; r.pe[d] = g.cstart[g.cs_off[d] + I1 + 1]; }
   }
   // z-slab restriction (multi-GPU): only planes [kz0,kz1)
-  if (r.ps[2] < kz0) r.ps[2] = kz0;
-  if (r.pe[2] > kz1) r.pe[2] = kz1;
+  if (!CELLS) { if (r.ps[2] < kz0) r.ps[2] = kz0; if (r.pe[2] > kz1) r.pe[2] = kz1; }
   i64 vol = 0, nt = 0;
   if (ok && r.pe[0] > r.ps[0] && r.pe[1] > r.ps[1] && r.pe[2] > r.ps[2]) {
     vol = (i64)(r.pe[0] - r.ps[0]) * (r.pe[1] - r.ps[1]) * (r.pe[2] - r.ps[2]);
-    nt = (i64)((r.pe[0] - 1) / TILE_X - r.ps[0] / TILE_X + 1) * ((r.pe[1] - 1) / TILE_Y - r.ps[1] / TILE_Y + 1) * ((r.pe[2] - 1) / TILE_Z - r.ps[2] / TILE_Z + 1);
+    const int last[3] = {r.pe[0] - 1, r.pe[1] - 1, r.pe[2] - 1};
+    nt = tile_span(r.ps, last);
   } else { r.pe[0] = r.ps[0]; r.pe[1] = r.ps[1]; r.pe[2] = r.ps[2]; }
   int a = idx[e];
-  rec[a] = r; ntile[a] = nt;
-  i64 np = (r.cls == 2) ? vol : 0;
-  npair[a] = np; nchunk[a] = (np + 31) / 32;
+  rec[a] = r; ntile[a] = nt; ntri[a] = __popc((unsigned)r.fmask) * nsn;
+  if (!CELLS) { i64 np = (r.cls == 2) ? vol : 0; npair[a] = np; nchunk[a] = (np + 31) / 32; }
 }
+// keys of the tiles each record covers; grid mode (poff) also the pair offsets and the tiles that hold boundary-face elements
 __global__ void k_emit_keys(i64 nact, ActRec *__restrict__ rec, const i64 *__restrict__ toff, const i64 *__restrict__ poff, GridDev g,
                             u64 *__restrict__ keys, int *__restrict__ tile_cnt, unsigned char *__restrict__ tile_faces) {
   i64 a = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (a >= nact) return;
   ActRec r = rec[a];
-  rec[a].pair_off = poff[a];
+  if (poff) rec[a].pair_off = poff[a];
   if (r.pe[0] <= r.ps[0]) return;
-  i64 o = toff[a];
-  for (int tz = r.ps[2] / TILE_Z; tz <= (r.pe[2] - 1) / TILE_Z; tz++)
-    for (int ty = r.ps[1] / TILE_Y; ty <= (r.pe[1] - 1) / TILE_Y; ty++)
-      for (int tx = r.ps[0] / TILE_X; tx <= (r.pe[0] - 1) / TILE_X; tx++) {
-        u64 t = ((u64)tz * g.nt[1] + ty) * g.nt[0] + tx;
-        keys[o++] = (t << 32) | (u64)a;
-        atomicAdd(&tile_cnt[t], 1);
-        if (r.fmask) tile_faces[t] = 1;       // this tile needs the boundary-face path of the assemble kernel
-      }
+  const int last[3] = {r.pe[0] - 1, r.pe[1] - 1, r.pe[2] - 1};
+  emit_tile_keys(g, r.ps, last, a, keys + toff[a], tile_cnt);
+  if (poff && r.fmask) for_tiles(g, r.ps, last, [&](u64 t) { tile_faces[t] = 1; });      // this tile needs the boundary-face path of the assemble kernel
 }
 
 // ------------------------------------------------------------------------------------------------ project (hot, FP64)
@@ -165,7 +163,7 @@ __global__ void __launch_bounds__(128, WANT_XP ? (BOX ? 4 : 2) : 4) k_project_he
     const double dd = sqrt(fma(d2, d2, fma(d1, d1, d0 * d0)));
     bool direct = false;
     if constexpr (!WANT_XP) {
-      direct = tile_faces[((i64)(pi2 / TILE_Z) * g.nt[1] + pi1 / TILE_Y) * g.nt[0] + pi0 / TILE_X] == 0;
+      direct = tile_faces[tile_of(g, pi0, pi1, pi2)] == 0;
       if (direct) atomicMin((u64 *)&dist[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0], (u64)__double_as_longlong(dd));
     }
     if (!direct) pairbuf[r.pair_off + li] = dd;
@@ -212,34 +210,20 @@ __global__ void k_box_records(i64 nact, const ActRec *__restrict__ rec, const in
   double nv[4][8];
 #pragma unroll
   for (int k = 0; k < 8; k++) { const i64 n = IEN[8 * (i64)r.el + k]; nv[0][k] = X[3 * n]; nv[1][k] = X[3 * n + 1]; nv[2][k] = X[3 * n + 2]; nv[3][k] = rn[n]; }
-  double A[4][8];
-#pragma unroll
-  for (int d = 0; d < 3; d++) {
-    B.org[d] = nv[d][0];
-#pragma unroll
-    for (int k = 0; k < 8; k++) nv[d][k] -= B.org[d];
-    iso::monomial8(nv[d], A[d]);
-  }
-  iso::monomial8(nv[3], A[3]);
-  iso::HexBox H; iso::make_box(A, H);
+  bnd::HexSetup P; bnd::hex8_setup(nv, rho_t, true, P);
+  iso::HexBox H; iso::make_box(P.A, H);
 #pragma unroll
   for (int k = 0; k < 8; k++) B.R[k] = H.R[k];
-  double gs = fabs(rho_t);
+  B.gs = P.gs; B.ok0 = P.ok0; B.sA = P.sA; B.sB = P.sB;
 #pragma unroll
-  for (int k = 0; k < 8; k++) gs = fmax(gs, fabs(nv[3][k]));
-  B.gs = fmax(gs, 1.0);
-  iso::ProjState S0; B.ok0 = iso::proj_init_element<iso::HexBox, PMODE>(H, rho_t, B.gs, S0) ? 1 : 0;
-#pragma unroll
-  for (int d = 0; d < 3; d++) { B.c[d] = H.c[d]; B.h[d] = H.h[d]; B.xi0[d] = S0.xi[d]; B.ps[d] = r.ps[d]; }
+  for (int d = 0; d < 3; d++) { B.c[d] = H.c[d]; B.h[d] = H.h[d]; B.org[d] = P.org[d]; B.xi0[d] = P.xi0[d]; B.tlo[d] = P.tlo[d]; B.thi[d] = P.thi[d]; B.sn[d] = P.sn[d]; B.ps[d] = r.ps[d]; }
   B.nx = r.pe[0] - r.ps[0]; B.ny = r.pe[1] - r.ps[1]; B.vol = B.nx * B.ny * (r.pe[2] - r.ps[2]);
   if ((i64)B.nx * B.ny * (r.pe[2] - r.ps[2]) >= (1ll << 24)) { B.vol = 0; atomicAdd(too_big, 1ull); }      // a pair-list entry holds 24 bits of local point index (PL_LI_BITS)
   B.ftile = 0; B.pad_ = 0;
-  if (B.vol > 0)
-    for (int tz = r.ps[2] / TILE_Z; tz <= (r.pe[2] - 1) / TILE_Z; tz++)
-      for (int ty = r.ps[1] / TILE_Y; ty <= (r.pe[1] - 1) / TILE_Y; ty++)
-        for (int tx = r.ps[0] / TILE_X; tx <= (r.pe[0] - 1) / TILE_X; tx++)
-          if (tile_faces[((i64)tz * g.nt[1] + ty) * g.nt[0] + tx]) B.ftile = 1;
-  bnd::box_iso_bounds(nv[3], rho_t, B.gs, B.org, H.c, H.h, B.tlo, B.thi, B.sn, B.sA, B.sB);
+  if (B.vol > 0) {
+    const int last[3] = {r.pe[0] - 1, r.pe[1] - 1, r.pe[2] - 1};
+    for_tiles(g, r.ps, last, [&](u64 t) { if (tile_faces[t]) B.ftile = 1; });
+  }
   box[a] = B;
 }
 // one warp per active element; lanes stride over its candidate points.  plist entry: bit 63 = goes to the pair buffer, bits 24..62 =
@@ -275,7 +259,7 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
     for (int li = lane; li < vol; li += 32) {
       const int pi0 = ps0 + ci, pi1 = ps1 + cj, pi2 = ps2 + ck;
       { ci += r32; const int c = ci >= nx ? 1 : 0; ci -= c ? nx : 0; cj += jq + c; ck += kq; if (cj >= ny) { cj -= ny; ck++; } }
-      if (ftile && tile_faces[((i64)(pi2 / TILE_Z) * g.nt[1] + pi1 / TILE_Y) * g.nt[0] + pi0 / TILE_X] != 0) continue;
+      if (ftile && tile_faces[tile_of(g, pi0, pi1, pi2)] != 0) continue;
       const double x0 = fma(g.cell, (double)pi0, g.amin[0]), x1 = fma(g.cell, (double)pi1, g.amin[1]), x2 = fma(g.cell, (double)pi2, g.amin[2]);
       const double e0 = fmax(fmax(tlo[0] - x0, x0 - thi[0]), 0.0), e1 = fmax(fmax(tlo[1] - x1, x1 - thi[1]), 0.0), e2 = fmax(fmax(tlo[2] - x2, x2 - thi[2]), 0.0);
       const u64 key = ((u64)__float_as_uint(__double2float_rd(sqrt(fma(e2, e2, fma(e1, e1, e0 * e0))))) << 32) | (u64)a;
@@ -298,7 +282,7 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
       if (li < vol) {
         const int pi0 = ps0 + i, pi1 = ps1 + j, pi2 = ps2 + k;
         const i64 v = ((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0;
-        const bool to_buf = ftile && tile_faces[((i64)(pi2 / TILE_Z) * g.nt[1] + pi1 / TILE_Y) * g.nt[0] + pi0 / TILE_X] != 0;
+        const bool to_buf = ftile && tile_faces[tile_of(g, pi0, pi1, pi2)] != 0;
         const bool seeded = !to_buf && prune && (unsigned)seed[v] == (unsigned)a;      // this pair is its point's seed (pass A)
         if (PASS == 1) { if (to_buf || seeded || !prune) flags[r] = 1 | (to_buf ? 2 : 0); }
         else if (!to_buf && !seeded) {
@@ -326,12 +310,10 @@ __global__ void __launch_bounds__(256, R2S_SCAN_MINB) k_pair_scan(i64 nact, cons
       const int r = __ffs(need) - 1; need &= need - 1;
       const int li = base0 + r * 32 + lane;
       const int pi0 = ps0 + li % nx, pi1 = ps1 + (li / nx) % ny, pi2 = ps2 + li / (nx * ny);
-      const double c = dist[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0], c2 = c * c * (1.0 + 1e-10);
+      const double c = dist[((i64)pi2 * g.np[1] + pi1) * g.np[0] + pi0];
       const double P[3] = {fma(g.cell, (double)pi0, g.amin[0]), fma(g.cell, (double)pi1, g.amin[1]), fma(g.cell, (double)pi2, g.amin[2])};
       const double n[3] = {B.sn[0], B.sn[1], B.sn[2]};
-      bool prn = bnd::lb2_box_gap(P, tlo, thi, n, B.sA, B.sB) > c2;
-      if (!prn) { const double lb = bnd::lb_box_slab(P, tlo, thi, n, B.sA, B.sB); prn = lb * lb > c2; }
-      if (prn) { keepb &= ~(1u << r); npruned++; }
+      if (bnd::box_slab_prunes(P, tlo, thi, n, B.sA, B.sB, c)) { keepb &= ~(1u << r); npruned++; }
     }
     // ONE list-slot claim per warp and batch: a single global counter serves the whole grid, and same-address atomics retire at about one
     // per clock -- a claim per 32-point round (7 per element) made this kernel atomic-bound (ncu: 3.4 + 7.2 ms)
@@ -434,12 +416,8 @@ __global__ void __launch_bounds__(128) k_project_tet4(i64 nitems, i64 nact, cons
   }
 }
 
-__global__ void k_tri_count(i64 nact, const ActRec *__restrict__ rec, int nsn, int *__restrict__ cnt) {
-  i64 a = blockIdx.x * (i64)blockDim.x + threadIdx.x;
-  if (a >= nact) return;
-  cnt[a] = __popc((unsigned)rec[a].fmask) * nsn;
-}
-template <int NEN>
+// boundary-face triangle table (face_triangles<NEN, CELLS>); grid mode also lists the crossing elements with boundary faces
+template <int NEN, bool CELLS>
 __global__ void k_tri_records(i64 nact, ActRec *__restrict__ rec, const int *__restrict__ toff, const int *__restrict__ IEN, const double *__restrict__ X, GridDev g,
                               double delta, TriRec *__restrict__ tri, int *__restrict__ fc_list, u64 *__restrict__ fc_count) {
   i64 a = blockIdx.x * (i64)blockDim.x + threadIdx.x;
@@ -447,10 +425,10 @@ __global__ void k_tri_records(i64 nact, ActRec *__restrict__ rec, const int *__r
   ActRec r = rec[a];
   rec[a].tri_off = toff[a];
   if (!r.fmask) return;
-  if (r.cls == 2) fc_list[atomicAdd(fc_count, 1ull)] = (int)a;      // crossing element with boundary faces: work list of k_faces_crossing (a few 10^4 entries)
+  if (!CELLS && r.cls == 2) fc_list[atomicAdd(fc_count, 1ull)] = (int)a;      // crossing element with boundary faces: work list of k_faces_crossing (a few 10^4 entries)
   double Xe[3][NEN];
   for (int q = 0; q < NEN; q++) { i64 n = IEN[NEN * (i64)r.el + q]; for (int d = 0; d < 3; d++) Xe[d][q] = X[3 * n + d]; }
-  face_triangles<NEN, false>(Xe, r.fmask, g, delta, tri + toff[a]);
+  face_triangles<NEN, CELLS>(Xe, r.fmask, g, delta, tri + toff[a]);
 }
 // Boundary faces of CROSSING elements (process_boundary_faces!(..., false), :584).  For a crossing element every candidate of
 // process_triangle_projection! is accepted or rejected by the rho-test alone (IsProjectedOnFullSegment, :78-119) -- never by
@@ -584,7 +562,8 @@ __global__ void __launch_bounds__(TILE_VOX) k_assemble(GridDev g, int kz0, int k
           if (pi[0] < T.ps[0] || pi[0] >= T.pe[0] || pi[1] < T.ps[1] || pi[1] >= T.pe[1] || pi[2] < T.ps[2] || pi[2] >= T.pe[2]) continue;
           if (r.cls == 1) {
             // solid element: no candidate of this triangle can be below the distance to its bounding box; if that is not
-            // below the running value the triangle changes nothing (exact; the margin covers the rounding of the candidates)
+            // below the running value the triangle changes nothing (exact; the margin covers the rounding of the candidates).  This is
+            // box_not_below written out: calling it here lets the compiler schedule this loop differently
             double lb2 = 0.0;
 #pragma unroll
             for (int d = 0; d < 3; d++) {
@@ -613,12 +592,7 @@ __global__ void __launch_bounds__(TILE_VOX) k_assemble(GridDev g, int kz0, int k
           if (ntri && r.cls == 1) {
             // solid element: if even the box around all its boundary triangles is not closer than the running value, none of them can
             // change it (same bound and margin as per triangle below) -- skip the record without touching its triangles
-            const TriRec &T0 = tri[r.tri_off];
-            double lb2 = 0.0;
-#pragma unroll
-            for (int d = 0; d < 3; d++) { const double e = fmax(fmax(T0.rlo[d] - x[d], x[d] - T0.rhi[d]), 0.0); lb2 = fma(e, e, lb2); }
-            const double cv = fabs(s.c) * (1.0 + 1e-12);
-            if (lb2 * (1.0 - 1e-12) > cv * cv) ntri = 0;
+            if (box_not_below(tri[r.tri_off].rlo, tri[r.tri_off].rhi, x, s.c)) ntri = 0;
           }
         }
       }
@@ -648,6 +622,80 @@ __global__ void __launch_bounds__(TILE_VOX) k_assemble(GridDev g, int kz0, int k
 }
 
 // ------------------------------------------------------------------------------------------------ host driver
+constexpr int NCTR = 8 * 129;      // counters: slot 0 element classes; slots 1..128 projection statistics; 8 more words: pair-list counters
+int r2s_dist_bins(r2s_ctx *ctx, const double *rn, double rho_t, double delta, bool cells, DistBins *b) {
+  const GridDev &g = ctx->g; cudaStream_t st = ctx->stream;
+  const i64 nel = ctx->nel; const int nen = ctx->nen;
+  const int kz0 = (int)ctx->k0, kz1 = (int)ctx->k1;
+  CK(ctx->cls.reserve((size_t)nel));
+  CK(ctx->act_flag.reserve(sizeof(int) * (size_t)(nel + 1)));
+  CK(ctx->act_idx.reserve(sizeof(int) * (size_t)(nel + 1)));
+  CK(ctx->counters.reserve(sizeof(u64) * (NCTR + 8)));
+  CK(cudaMemsetAsync(ctx->counters.p, 0, sizeof(u64) * (NCTR + 8), st));
+  CK(cudaMemsetAsync(ctx->act_flag.as<int>() + nel, 0, sizeof(int), st));
+  // z-interval of this rank's planes with a margin of (delta + 2 cells): only elements that can reach them are classified
+  double zlo = -1e300, zhi = 1e300;
+  if (!cells && (kz0 > 0 || kz1 < g.np[2])) { const double m = delta + 2.0 * g.cell; zlo = ctx->h_pc[2][(size_t)kz0] - m; zhi = ctx->h_pc[2][(size_t)kz1 - 1] + m; }
+  k_classify<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->IEN32.as<int>(), rn, ctx->fbnd.as<unsigned char>(), ctx->ezr.as<double2>(), zlo, zhi, rho_t,
+                                             ctx->cls.as<unsigned char>(), ctx->act_flag.as<int>(), ctx->counters.as<i64>()); LAUNCH_CHECK();
+  if (r2s_scan_exclusive_i32(ctx, ctx->act_flag.as<int>(), ctx->act_idx.as<int>(), nel + 1)) return 1;
+  int nact_i = 0;
+  if (r2s_readback(ctx, &nact_i, ctx->act_idx.as<int>() + nel, sizeof(int))) return 1;
+  const i64 nact = nact_i;
+  CK(ctx->tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
+  CK(cudaMemsetAsync(ctx->tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
+  if (!cells) {
+    CK(ctx->tile_faces.reserve((size_t)g.ntiles + 16));
+    CK(cudaMemsetAsync(ctx->tile_faces.p, 0, (size_t)g.ntiles, st));
+  }
+  b->nact = nact; b->npairs = 0; b->nitems = 0;
+  i64 nkeys = 0;
+  if (nact > 0) {
+    CK(ctx->act_rec.reserve(sizeof(ActRec) * (size_t)nact));
+    CK(ctx->cnt_a.reserve(sizeof(i64) * 3 * (size_t)(nact + 1)));
+    CK(ctx->cnt_b.reserve(sizeof(i64) * 3 * (size_t)(nact + 1)));
+    CK(ctx->tri_cnt.reserve(sizeof(int) * 2 * (size_t)(nact + 1)));
+    i64 *ntile = ctx->cnt_a.as<i64>(), *npair = ntile + (nact + 1), *nchunk = npair + (nact + 1);
+    i64 *toff = ctx->cnt_b.as<i64>(), *poff = toff + (nact + 1), *choff = poff + (nact + 1);
+    int *tcnt = ctx->tri_cnt.as<int>(), *toff32 = tcnt + (nact + 1);
+    CK(cudaMemsetAsync(ctx->cnt_a.p, 0, sizeof(i64) * 3 * (size_t)(nact + 1), st));
+    CK(cudaMemsetAsync(tcnt + nact, 0, sizeof(int), st));
+#define RECS(C) k_act_records<C><<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->nsn, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->cls.as<unsigned char>(), ctx->fbnd.as<unsigned char>(), \
+      ctx->act_flag.as<int>(), ctx->act_idx.as<int>(), g, delta, kz0, kz1, ctx->act_rec.as<ActRec>(), ntile, tcnt, npair, nchunk)
+    if (cells) RECS(true); else RECS(false);
+#undef RECS
+    LAUNCH_CHECK();
+    if (r2s_scan_exclusive_i64(ctx, ntile, toff, nact + 1)) return 1;
+    if (r2s_scan_exclusive_i32(ctx, tcnt, toff32, nact + 1)) return 1;
+    if (!cells) {
+      if (r2s_scan_exclusive_i64(ctx, npair, poff, nact + 1)) return 1;
+      if (r2s_scan_exclusive_i64(ctx, nchunk, choff, nact + 1)) return 1;
+    }
+    const size_t o0 = r2s_rb_put(ctx, toff + nact, sizeof(i64)), o1 = r2s_rb_put(ctx, toff32 + nact, sizeof(int));
+    const size_t o2 = cells ? 0 : r2s_rb_put(ctx, poff + nact, sizeof(i64)), o3 = cells ? 0 : r2s_rb_put(ctx, choff + nact, sizeof(i64));
+    if (o0 == (size_t)-1 || o1 == (size_t)-1 || o2 == (size_t)-1 || o3 == (size_t)-1 || r2s_rb_sync(ctx)) return 1;
+    nkeys = *(const i64 *)r2s_rb_at(ctx, o0);
+    const int ntri = *(const int *)r2s_rb_at(ctx, o1);
+    if (!cells) { b->npairs = *(const i64 *)r2s_rb_at(ctx, o2); b->nitems = *(const i64 *)r2s_rb_at(ctx, o3); }
+    if (nkeys >= (1ll << 31) || b->npairs >= (1ll << 40)) FAIL("distance binning: problem too large for one slab (key/pair count overflow)");
+    CK(ctx->keys.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
+    CK(ctx->keys_alt.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
+    k_emit_keys<<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), toff, cells ? nullptr : poff, g, ctx->keys.as<u64>(), ctx->tile_ptr.as<int>() + 1,
+                                                 ctx->tile_faces.as<unsigned char>()); LAUNCH_CHECK();
+    // boundary-face triangle table
+    CK(ctx->tri_rec.reserve(sizeof(TriRec) * (size_t)(ntri + 1)));
+    if (!cells) CK(ctx->fc_list.reserve(sizeof(int) * (size_t)(nact + 16)));
+    u64 *fc_count = ctx->counters.as<u64>() + NCTR + 5;
+#define TRIS(NEN, C) k_tri_records<NEN, C><<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), toff32, ctx->IEN32.as<int>(), ctx->X.as<double>(), g, delta, \
+      ctx->tri_rec.as<TriRec>(), ctx->fc_list.as<int>(), fc_count)
+    if (nen == 8) { if (cells) TRIS(8, true); else TRIS(8, false); }
+    else { if (cells) TRIS(4, true); else TRIS(4, false); }
+#undef TRIS
+    LAUNCH_CHECK();
+  }
+  return r2s_tile_lists(ctx, ctx->keys.as<u64>(), ctx->keys_alt.as<u64>(), nkeys, ctx->tile_ptr.as<int>(), &b->sorted);
+}
+
 int r2s_dev_eval_distances(r2s_ctx *ctx, double rho_t, double delta_factor, bool want_xp) {
   if (!ctx->has_grid) FAIL("r2s_set_grid has not been called");
   if (ctx->nel == 0) FAIL("r2s_set_mesh has not been called");
@@ -656,80 +704,15 @@ int r2s_dev_eval_distances(r2s_ctx *ctx, double rho_t, double delta_factor, bool
   double delta = delta_factor * g.cell;
   int kz0 = (int)ctx->k0, kz1 = (int)ctx->k1;
   CK(cudaEventRecord(ctx->ev[0], st));
-  CK(ctx->cls.reserve((size_t)nel));
-  CK(ctx->act_flag.reserve(sizeof(int) * (size_t)(nel + 1)));
-  CK(ctx->act_idx.reserve(sizeof(int) * (size_t)(nel + 1)));
-  constexpr int NCTR = 8 * 129;      // slot 0: element classes; slots 1..128: projection statistics; 8 more words: pair-list counters
-  CK(ctx->counters.reserve(sizeof(u64) * (NCTR + 8)));
-  CK(cudaMemsetAsync(ctx->counters.p, 0, sizeof(u64) * (NCTR + 8), st));
-  CK(cudaMemsetAsync(ctx->act_flag.as<int>() + nel, 0, sizeof(int), st));
-  // z-interval of this rank's planes with a margin of (delta + 2 cells): only elements that can reach them are classified
-  double zlo = -1e300, zhi = 1e300;
-  if (kz0 > 0 || kz1 < g.np[2]) { const double m = delta + 2.0 * g.cell; zlo = ctx->h_pc[2][(size_t)kz0] - m; zhi = ctx->h_pc[2][(size_t)kz1 - 1] + m; }
-  k_classify<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->IEN32.as<int>(), ctx->rho_n.as<double>(), ctx->fbnd.as<unsigned char>(), ctx->ezr.as<double2>(), zlo, zhi, rho_t,
-                                             ctx->cls.as<unsigned char>(), ctx->act_flag.as<int>(), ctx->counters.as<i64>()); LAUNCH_CHECK();
-  if (r2s_scan_exclusive_i32(ctx, ctx->act_flag.as<int>(), ctx->act_idx.as<int>(), nel + 1)) return 1;
-  int nact_i = 0;
-  if (r2s_readback(ctx, &nact_i, ctx->act_idx.as<int>() + nel, sizeof(int))) return 1;
-  i64 nact = nact_i;
+  DistBins bins;
+  if (r2s_dist_bins(ctx, ctx->rho_n.as<double>(), rho_t, delta, false, &bins)) return 1;
+  const i64 nact = bins.nact, npairs = bins.npairs, nitems = bins.nitems;
+  const u64 *sorted = bins.sorted;
   CK(ctx->dist.reserve(sizeof(double) * (size_t)g.ngp));
   if (want_xp) CK(ctx->xp.reserve(sizeof(double) * 3 * (size_t)g.ngp));
-  CK(ctx->tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-  CK(cudaMemsetAsync(ctx->tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
-  CK(ctx->tile_faces.reserve((size_t)g.ntiles + 16));
-  CK(cudaMemsetAsync(ctx->tile_faces.p, 0, (size_t)g.ntiles, st));
-  i64 npairs = 0, nkeys = 0, nitems = 0; int ntri = 0;
-  u64 *sorted = nullptr;
   if (nact > 0) {
-    CK(ctx->act_rec.reserve(sizeof(ActRec) * (size_t)nact));
-    CK(ctx->cnt_a.reserve(sizeof(i64) * 3 * (size_t)(nact + 1)));
-    CK(ctx->cnt_b.reserve(sizeof(i64) * 3 * (size_t)(nact + 1)));
-    i64 *ntile = ctx->cnt_a.as<i64>(), *npair = ntile + (nact + 1), *nchunk = npair + (nact + 1);
-    i64 *toff = ctx->cnt_b.as<i64>(), *poff = toff + (nact + 1), *choff = poff + (nact + 1);
-    CK(cudaMemsetAsync(ctx->cnt_a.p, 0, sizeof(i64) * 3 * (size_t)(nact + 1), st));
-    k_act_records<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->cls.as<unsigned char>(), ctx->fbnd.as<unsigned char>(),
-                                                  ctx->act_flag.as<int>(), ctx->act_idx.as<int>(), g, delta, kz0, kz1, ctx->act_rec.as<ActRec>(), ntile, npair, nchunk);
-    LAUNCH_CHECK();
-    if (r2s_scan_exclusive_i64(ctx, ntile, toff, nact + 1)) return 1;
-    if (r2s_scan_exclusive_i64(ctx, npair, poff, nact + 1)) return 1;
-    if (r2s_scan_exclusive_i64(ctx, nchunk, choff, nact + 1)) return 1;
-    {
-      const size_t o0 = r2s_rb_put(ctx, toff + nact, sizeof(i64)), o1 = r2s_rb_put(ctx, poff + nact, sizeof(i64)), o2 = r2s_rb_put(ctx, choff + nact, sizeof(i64));
-      if (o0 == (size_t)-1 || o1 == (size_t)-1 || o2 == (size_t)-1) return 1;
-      // the triangle count of the boundary-face table is read back with the same synchronisation
-      CK(ctx->tri_cnt.reserve(sizeof(int) * 2 * (size_t)(nact + 1)));
-      int *tcnt = ctx->tri_cnt.as<int>(), *toff32 = tcnt + (nact + 1);
-      CK(cudaMemsetAsync(tcnt + nact, 0, sizeof(int), st));
-      k_tri_count<<<cdiv(nact, 256), 256, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), ctx->nsn, tcnt); LAUNCH_CHECK();
-      if (r2s_scan_exclusive_i32(ctx, tcnt, toff32, nact + 1)) return 1;
-      const size_t o3 = r2s_rb_put(ctx, toff32 + nact, sizeof(int));
-      if (o3 == (size_t)-1) return 1;
-      if (r2s_rb_sync(ctx)) return 1;
-      nkeys = *(const i64 *)r2s_rb_at(ctx, o0); npairs = *(const i64 *)r2s_rb_at(ctx, o1); nitems = *(const i64 *)r2s_rb_at(ctx, o2); ntri = *(const int *)r2s_rb_at(ctx, o3);
-    }
-    if (nkeys >= (1ll << 31) || npairs >= (1ll << 40)) FAIL("distance binning: problem too large for one slab (key/pair count overflow)");
-    CK(ctx->keys.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
-    CK(ctx->keys_alt.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
     CK(ctx->pairbuf.reserve(sizeof(double) * (size_t)(npairs + 1)));
     if (want_xp) CK(ctx->pairxp.reserve(sizeof(double) * 3 * (size_t)(npairs + 1)));
-    k_emit_keys<<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), toff, poff, g, ctx->keys.as<u64>(), ctx->tile_ptr.as<int>() + 1, ctx->tile_faces.as<unsigned char>()); LAUNCH_CHECK();
-    int tbits = 1; while ((1ll << tbits) < g.ntiles) tbits++;
-    if (nkeys > 0) { if (r2s_sort_keys_u64(ctx, ctx->keys.as<u64>(), ctx->keys_alt.as<u64>(), nkeys, 32 + tbits, &sorted)) return 1; }
-    // boundary-face triangle table
-    int *toff32 = ctx->tri_cnt.as<int>() + (nact + 1);
-    CK(ctx->tri_rec.reserve(sizeof(TriRec) * (size_t)(ntri + 1)));
-    CK(ctx->fc_list.reserve(sizeof(int) * (size_t)(nact + 16)));
-    u64 *fc_count = ctx->counters.as<u64>() + NCTR + 5;
-    if (nen == 8) k_tri_records<8><<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), toff32, ctx->IEN32.as<int>(), ctx->X.as<double>(), g, delta, ctx->tri_rec.as<TriRec>(), ctx->fc_list.as<int>(), fc_count);
-    else k_tri_records<4><<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), toff32, ctx->IEN32.as<int>(), ctx->X.as<double>(), g, delta, ctx->tri_rec.as<TriRec>(), ctx->fc_list.as<int>(), fc_count);
-    LAUNCH_CHECK();
-  }
-  // tile_ptr[t+1] currently holds the count of tile t (tile_ptr[0] = 0): inclusive scan in place == exclusive offsets
-  {
-    DevBuf &tmp = ctx->s_cnt;   // reuse as scratch
-    CK(tmp.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-    if (r2s_scan_exclusive_i32(ctx, ctx->tile_ptr.as<int>() + 1, tmp.as<int>(), g.ntiles + 1)) return 1;
-    CK(cudaMemcpyAsync(ctx->tile_ptr.as<int>(), tmp.as<int>(), sizeof(int) * (size_t)(g.ntiles + 1), cudaMemcpyDeviceToDevice, st));
   }
   CK(cudaEventRecord(ctx->ev[1], st));
   // Without xp, dist[] starts at BIG and receives the minima of the face-free tiles by atomicMin; k_assemble then replays only the tiles

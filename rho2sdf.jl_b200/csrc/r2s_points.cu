@@ -1,10 +1,11 @@
 // r2s_points.cu -- evalDistances and Sign_Detection at arbitrary points (the reference's `points` argument, binned by LinkedList(grid,
 // points), Grid.jl:47-69) on the GPU.  The rule is written out in include/r2s.h.
 //
-// Distances, once per call: the active elements (solid with boundary faces, crossing) get the CELL range of their AABB +- delta
-// (calculateMiniAABB_grid, Grid.jl:122-154) over the whole grid -- no slab clipping -- and are binned into tiles of cells, (tile, element)
-// keys radix-sorted into per-tile lists in ascending element order; the boundary-face triangles get cell ranges too (face_triangles<.., true>),
-// and every crossing HEX8 element a solver record (phase 1 of the projection done once).  Per chunk of points: each point's cell, its
+// Distances, once per call: the binning of the grid path (r2s_dist_bins) in cell mode -- the active elements (solid with boundary faces,
+// crossing) get the CELL range of their AABB +- delta (calculateMiniAABB_grid, Grid.jl:122-154) over the whole grid, no slab clipping, and
+// are binned into tiles of cells, (tile, element) keys radix-sorted into per-tile lists in ascending element order; the boundary-face
+// triangles get cell ranges too (face_triangles<.., true>) -- and every crossing HEX8 element a solver record (bnd::hex8_setup: phase 1 of
+// the projection done once).  Per chunk of points: each point's cell, its
 // tile, the point ids sorted by tile; one thread per point walks its tile's list in element order and replays the running minimum
 // (r2s_replay.cuh) with the per-pair solvers of the grid path's closest-point (xp) kernels.  A triangle or an iso pair is skipped when a
 // lower bound of everything it could write is not below the running |value| (triangle box; box /\ slab of r2s_bound.cuh for box elements):
@@ -29,13 +30,6 @@
 #define PT_CHUNK (1ll << 22)      // points per chunk: the bounded device buffer (as r2s_sample_sdf)
 #define PT_IDX_BITS 22            // sort key = tile << PT_IDX_BITS | point index in the chunk
 
-// crossing HEX8 element: the solver constants of k_project_hex8 (element-local coordinates, node 0 subtracted) and phase 1
-struct __align__(16) PtHex {
-  double A[4][8];            // monomial coefficients of x, y, z (local) and rho
-  double org[3], xi0[3], gs;
-  double tlo[3], thi[3], sn[3], sA, sB;      // box elements: tight box and slab of the iso-patch, global coordinates (r2s_bound.cuh)
-  int box, ok0;
-};
 // element of the sign binning: closed AABB, inclusive bin range per axis (1-based bins), hot = some nodal density >= rho_t (:36)
 struct SPRec { double lo[3], hi[3]; int b0[3], b1[3]; int hot, pad; };
 
@@ -49,105 +43,19 @@ __device__ __forceinline__ bool pt_cell(const GridDev &g, const double x[3], int
   }
   return ok;
 }
-// point_to_grid_index (SignDetection.jl:256-268): clamp(floor((x - amin) / cell) + 1, 1, N + 1), clamped before the conversion
-__device__ __forceinline__ int pt_bin(double x, double amin, double cell, int n1) {
-  const double f = floor(ex::dvd(ex::sub(x, amin), cell)) + 1.0;
-  return f < 1.0 ? 1 : (f > (double)n1 ? n1 : (int)f);
-}
-__device__ __forceinline__ i64 tile_of(const GridDev &g, int c0, int c1, int c2) {
-  return ((i64)(c2 / TILE_Z) * g.nt[1] + c1 / TILE_Y) * g.nt[0] + c0 / TILE_X;
-}
-
 // ------------------------------------------------------------------------------------------------ distances: once per call
-__global__ void k_pt_classify(i64 nel, int nen, const int *__restrict__ IEN, const double *__restrict__ rn, const unsigned char *__restrict__ fb, double rho_t,
-                              unsigned char *__restrict__ cls, int *__restrict__ flag, u64 *__restrict__ ctr) {
-  const i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
-  int c = 0;
-  if (e < nel) {
-    double mn = 1e300, mx = -1e300;
-    for (int a = 0; a < nen; a++) { const double r = rn[IEN[nen * e + a]]; mn = fmin(mn, r); mx = fmax(mx, r); }
-    c = mn >= rho_t ? 1 : (mx > rho_t ? 2 : 0);      // :199-201, :312
-    cls[e] = (unsigned char)c;
-    flag[e] = (c == 2 || (c == 1 && fb[e] != 0)) ? 1 : 0;
-  }
-  const unsigned m1 = __ballot_sync(0xffffffffu, c == 1), m2 = __ballot_sync(0xffffffffu, c == 2);      // class counters (report): one atomic per warp
-  if ((threadIdx.x & 31) == 0) { if (m1) atomicAdd(&ctr[0], (u64)__popc(m1)); if (m2) atomicAdd(&ctr[1], (u64)__popc(m2)); }
-}
-// active record with CELL ranges [ps, pe) (ActRec's fields hold cells here, not grid points), its tile and triangle counts
-__global__ void k_pt_records(i64 nel, int nen, int nsn, const int *__restrict__ IEN, const double *__restrict__ X, const unsigned char *__restrict__ cls,
-                             const unsigned char *__restrict__ fb, const int *__restrict__ flag, const int *__restrict__ idx, GridDev g, double delta,
-                             ActRec *__restrict__ rec, i64 *__restrict__ ntile, int *__restrict__ ntri) {
-  const i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
-  if (e >= nel || !flag[e]) return;
-  double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-  for (int a = 0; a < nen; a++) { const i64 n = IEN[nen * e + a]; for (int d = 0; d < 3; d++) { const double c = X[3 * n + d]; lo[d] = fmin(lo[d], c); hi[d] = fmax(hi[d], c); } }
-  ActRec r; r.el = (int)e; r.cls = cls[e]; r.fmask = fb[e]; r.tri_off = 0; r.pair_off = 0;
-  bool ok = true;
-  for (int d = 0; d < 3; d++) {
-    int I0 = 0, I1 = -1;
-    ok = ok && ex::cell_range_axis(lo[d], hi[d], delta, g.amin[d], g.amax[d], g.N[d], I0, I1);
-    r.ps[d] = ok ? I0 : 0; r.pe[d] = ok ? I1 + 1 : 0;
-  }
-  const int a = idx[e];
-  if (!ok) { for (int d = 0; d < 3; d++) r.pe[d] = r.ps[d]; }
-  rec[a] = r;
-  ntile[a] = ok ? (i64)((r.pe[0] - 1) / TILE_X - r.ps[0] / TILE_X + 1) * ((r.pe[1] - 1) / TILE_Y - r.ps[1] / TILE_Y + 1) * ((r.pe[2] - 1) / TILE_Z - r.ps[2] / TILE_Z + 1) : 0;
-  ntri[a] = __popc((unsigned)r.fmask) * nsn;
-}
-template <int NEN>
-__global__ void k_pt_emit(i64 nact, ActRec *__restrict__ rec, const i64 *__restrict__ toff, const int *__restrict__ troff, const int *__restrict__ IEN,
-                          const double *__restrict__ X, const double *__restrict__ rn, const unsigned char *__restrict__ ebox, int proj_box, GridDev g, double delta,
-                          double rho_t, u64 *__restrict__ keys, int *__restrict__ tile_cnt, TriRec *__restrict__ tri, PtHex *__restrict__ hex) {
+// solver record of every crossing HEX8 element (k_project_hex8's set-up, element-local coordinates)
+__global__ void k_pt_hex(i64 nact, const ActRec *__restrict__ rec, const int *__restrict__ IEN, const double *__restrict__ X, const double *__restrict__ rn,
+                         const unsigned char *__restrict__ ebox, int proj_box, double rho_t, bnd::HexSetup *__restrict__ hex) {
   const i64 a = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (a >= nact) return;
-  ActRec r = rec[a];
-  rec[a].tri_off = troff[a];
-  if (r.pe[0] > r.ps[0]) {
-    i64 o = toff[a];
-    for (int tz = r.ps[2] / TILE_Z; tz <= (r.pe[2] - 1) / TILE_Z; tz++)
-      for (int ty = r.ps[1] / TILE_Y; ty <= (r.pe[1] - 1) / TILE_Y; ty++)
-        for (int tx = r.ps[0] / TILE_X; tx <= (r.pe[0] - 1) / TILE_X; tx++) {
-          const u64 t = ((u64)tz * g.nt[1] + ty) * g.nt[0] + tx;
-          keys[o++] = (t << 32) | (u64)a;
-          atomicAdd(&tile_cnt[t], 1);
-        }
-  }
-  double Xe[3][NEN];
-  for (int q = 0; q < NEN; q++) { const i64 n = IEN[NEN * (i64)r.el + q]; for (int d = 0; d < 3; d++) Xe[d][q] = X[3 * n + d]; }
-  if (r.fmask) face_triangles<NEN, true>(Xe, r.fmask, g, delta, tri + troff[a]);
-  if (NEN == 8 && r.cls == 2) {      // the arithmetic of k_project_hex8 / k_box_records
-    PtHex P; double nv[4][8];
+  const ActRec r = rec[a];
+  if (r.cls != 2) return;
+  double nv[4][8];
 #pragma unroll
-    for (int k = 0; k < 8; k++) { nv[0][k] = Xe[0][k]; nv[1][k] = Xe[1][k]; nv[2][k] = Xe[2][k]; nv[3][k] = rn[IEN[8 * (i64)r.el + k]]; }
-#pragma unroll
-    for (int d = 0; d < 3; d++) {
-      P.org[d] = nv[d][0];
-#pragma unroll
-      for (int k = 0; k < 8; k++) nv[d][k] -= P.org[d];
-    }
-#pragma unroll
-    for (int c = 0; c < 4; c++) iso::monomial8(nv[c], P.A[c]);
-    double gs = fabs(rho_t);
-#pragma unroll
-    for (int k = 0; k < 8; k++) gs = fmax(gs, fabs(nv[3][k]));
-    P.gs = fmax(gs, 1.0);
-    P.box = (proj_box && ebox[r.el]) ? 1 : 0;
-    iso::ProjState S0;
-    if (P.box) {
-      iso::HexBox H; iso::make_box(P.A, H);
-      P.ok0 = iso::proj_init_element<iso::HexBox, PMODE>(H, rho_t, P.gs, S0) ? 1 : 0;
-      bnd::box_iso_bounds(nv[3], rho_t, P.gs, P.org, H.c, H.h, P.tlo, P.thi, P.sn, P.sA, P.sB);
-    } else {
-      iso::HexTri H; H.A = P.A;
-      P.ok0 = iso::proj_init_element<iso::HexTri, PMODE>(H, rho_t, P.gs, S0) ? 1 : 0;
-#pragma unroll
-      for (int d = 0; d < 3; d++) { P.tlo[d] = -INFINITY; P.thi[d] = INFINITY; P.sn[d] = 0.0; }
-      P.sA = -INFINITY; P.sB = INFINITY;
-    }
-#pragma unroll
-    for (int d = 0; d < 3; d++) P.xi0[d] = S0.xi[d];
-    hex[a] = P;
-  }
+  for (int k = 0; k < 8; k++) { const i64 n = IEN[8 * (i64)r.el + k]; nv[0][k] = X[3 * n]; nv[1][k] = X[3 * n + 1]; nv[2][k] = X[3 * n + 2]; nv[3][k] = rn[n]; }
+  bnd::HexSetup P; bnd::hex8_setup(nv, rho_t, proj_box && ebox[r.el], P);
+  hex[a] = P;
 }
 
 // ------------------------------------------------------------------------------------------------ per chunk
@@ -165,7 +73,7 @@ __global__ void k_pt_keys(i64 m, const double *__restrict__ pts, GridDev g, int 
 
 // the iso distance of one (crossing HEX8 element, point) pair: k_project_hex8<true, BOX>'s arithmetic
 template <bool BOX>
-__device__ __forceinline__ double pt_project_hex8(const PtHex &P, const int *__restrict__ IEN, const double *__restrict__ rn, int el, double rho_t, const double xg[3],
+__device__ __forceinline__ double pt_project_hex8(const bnd::HexSetup &P, const int *__restrict__ IEN, const double *__restrict__ rn, int el, double rho_t, const double xg[3],
                                                   double xp[3], int &nit, bool &ok) {
   double A[4][8], re[8];
 #pragma unroll
@@ -188,19 +96,10 @@ __device__ __forceinline__ double pt_project_hex8(const PtHex &P, const int *__r
   for (int d = 0; d < 3; d++) xp[d] = p[d] + P.org[d];
   return sqrt(fma(d2, d2, fma(d1, d1, d0 * d0)));
 }
-// lower bound of |point - y| over every y a triangle (or an element's triangles) can write, against the running value (k_assemble's margins)
-__device__ __forceinline__ bool box_not_below(const double lo[3], const double hi[3], const double x[3], double c) {
-  double lb2 = 0.0;
-#pragma unroll
-  for (int d = 0; d < 3; d++) { const double e = fmax(fmax(lo[d] - x[d], x[d] - hi[d]), 0.0); lb2 = fma(e, e, lb2); }
-  const double cv = fabs(c) * (1.0 + 1e-12);
-  return lb2 * (1.0 - 1e-12) > cv * cv;
-}
-
 // stats: [0] pairs (crossing element whose range holds the point), [1] pairs pruned, [2] Newton iterations, [3] not converged
 template <bool WANT_XP, int NEN>
 __global__ void __launch_bounds__(128) k_pt_dist(i64 m, const u64 *__restrict__ skeys, const double *__restrict__ pts, GridDev g, const int *__restrict__ tile_ptr,
-                                                 const u64 *__restrict__ tkeys, const ActRec *__restrict__ rec, const TriRec *__restrict__ tri, const PtHex *__restrict__ hex,
+                                                 const u64 *__restrict__ tkeys, const ActRec *__restrict__ rec, const TriRec *__restrict__ tri, const bnd::HexSetup *__restrict__ hex,
                                                  const int *__restrict__ IEN, const double *__restrict__ X, const double *__restrict__ rn, double rho_t, int prune,
                                                  double *__restrict__ dist, double *__restrict__ xpo, u64 *__restrict__ stats) {
   constexpr int NSN = NEN == 8 ? 4 : 3;
@@ -239,17 +138,16 @@ __global__ void __launch_bounds__(128) k_pt_dist(i64 m, const u64 *__restrict__ 
         npair++;
         double dt, p[3];
         if (NEN == 8) {
-          const PtHex &P = hex[a];
+          const bnd::HexSetup &P = hex[a];
           if (prune && P.box) {      // tight box, then box /\ slab (k_pair_scan<2>'s tests and margin)
-            const double cur = fabs(st.c), c2 = cur * cur * (1.0 + 1e-10);
+            const double cur = fabs(st.c);
             double lb2 = 0.0;
 #pragma unroll
             for (int d = 0; d < 3; d++) { const double e = fmax(fmax(P.tlo[d] - x[d], x[d] - P.thi[d]), 0.0); lb2 = fma(e, e, lb2); }
-            bool prn = lb2 > c2;
+            bool prn = lb2 > cur * cur * (1.0 + 1e-10);
             if (!prn && P.sA != -INFINITY) {
               const double n3[3] = {P.sn[0], P.sn[1], P.sn[2]};
-              prn = bnd::lb2_box_gap(x, P.tlo, P.thi, n3, P.sA, P.sB) > c2;
-              if (!prn) { const double lb = bnd::lb_box_slab(x, P.tlo, P.thi, n3, P.sA, P.sB); prn = lb * lb > c2; }
+              prn = bnd::box_slab_prunes(x, P.tlo, P.thi, n3, P.sA, P.sB, cur);
             }
             if (prn) { npruned++; continue; }
           }
@@ -288,16 +186,15 @@ __global__ void k_pt_sign_records(i64 nel, int nen, const int *__restrict__ IEN,
                                   SPRec *__restrict__ rng, SignEl *__restrict__ sel, i64 *__restrict__ ntile) {
   const i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (e >= nel) return;
-  SPRec R; double rmax = -1e300;
-  for (int d = 0; d < 3; d++) { R.lo[d] = 1e300; R.hi[d] = -1e300; }
-  for (int a = 0; a < nen; a++) { const i64 n = IEN[nen * e + a]; rmax = fmax(rmax, rn[n]); for (int d = 0; d < 3; d++) { const double c = X[3 * n + d]; R.lo[d] = fmin(R.lo[d], c); R.hi[d] = fmax(R.hi[d], c); } }
-  R.hot = (nen == 4 || !(rmax < rho_t)) ? 1 : 0; R.pad = 0;
+  SignElem E; sign_element(e, nen, IEN, X, rn, rho_t, g, E);
+  SPRec R; R.hot = E.hot; R.pad = 0;
   bool ok = true;
   for (int d = 0; d < 3; d++) {
     const int n1 = g.np[d];
+    R.lo[d] = E.lo[d]; R.hi[d] = E.hi[d];
     if (nen == 8) { R.b0[d] = pt_bin(R.lo[d], g.amin[d], g.cell, n1); R.b1[d] = pt_bin(R.hi[d], g.amin[d], g.cell, n1); }
     else {      // create_grid_tetrahedra_mapping_TET4 (:195-196), as k_sign_ranges, clamped before the conversion
-      const double mi = floor(ex::dvd(ex::sub(R.lo[d], g.amin[d]), g.cell)) - 1.0, ma = ceil(ex::dvd(ex::sub(R.hi[d], g.amin[d]), g.cell)) + 1.0;
+      const double mi = E.fl[d] - 1.0, ma = E.cu[d] + 1.0;
       R.b0[d] = mi < 1.0 ? 1 : (mi > (double)n1 ? n1 + 1 : (int)mi);
       R.b1[d] = ma > (double)n1 ? n1 : (ma < 1.0 ? 0 : (int)ma);
     }
@@ -305,27 +202,17 @@ __global__ void k_pt_sign_records(i64 nel, int nen, const int *__restrict__ IEN,
   }
   if (!ok) { R.b0[0] = 1; R.b1[0] = 0; }
   rng[e] = R;
-  if (nen == 8) {
-    double A[3][8];
-    for (int d = 0; d < 3; d++) { double v[8]; for (int a = 0; a < 8; a++) v[a] = X[3 * (i64)IEN[8 * e + a] + d]; ex::mono8(v, A[d]); }
-    SignEl S; ex::affine_inverse_prepare(A, S);
-    sel[e] = S;
-  }
-  ntile[e] = ok ? (i64)((R.b1[0] - 1) / TILE_X - (R.b0[0] - 1) / TILE_X + 1) * ((R.b1[1] - 1) / TILE_Y - (R.b0[1] - 1) / TILE_Y + 1) * ((R.b1[2] - 1) / TILE_Z - (R.b0[2] - 1) / TILE_Z + 1) : 0;
+  if (nen == 8) sel[e] = sign_affine(e, IEN, X);
+  const int lo[3] = {R.b0[0] - 1, R.b0[1] - 1, R.b0[2] - 1}, hi[3] = {R.b1[0] - 1, R.b1[1] - 1, R.b1[2] - 1};      // 0-based bins
+  ntile[e] = ok ? tile_span(lo, hi) : 0;
 }
 __global__ void k_pt_sign_emit(i64 nel, const SPRec *__restrict__ rng, const i64 *__restrict__ toff, GridDev g, u64 *__restrict__ keys, int *__restrict__ tile_cnt) {
   const i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (e >= nel) return;
   const SPRec R = rng[e];
   if (R.b0[0] > R.b1[0]) return;
-  i64 o = toff[e];
-  for (int tz = (R.b0[2] - 1) / TILE_Z; tz <= (R.b1[2] - 1) / TILE_Z; tz++)
-    for (int ty = (R.b0[1] - 1) / TILE_Y; ty <= (R.b1[1] - 1) / TILE_Y; ty++)
-      for (int tx = (R.b0[0] - 1) / TILE_X; tx <= (R.b1[0] - 1) / TILE_X; tx++) {
-        const u64 t = ((u64)tz * g.nt[1] + ty) * g.nt[0] + tx;
-        keys[o++] = (t << 32) | (u64)e;
-        atomicAdd(&tile_cnt[t], 1);
-      }
+  const int lo[3] = {R.b0[0] - 1, R.b0[1] - 1, R.b0[2] - 1}, hi[3] = {R.b1[0] - 1, R.b1[1] - 1, R.b1[2] - 1};
+  emit_tile_keys(g, lo, hi, e, keys + toff[e], tile_cnt);
 }
 template <int NEN>
 __global__ void __launch_bounds__(128) k_pt_sign(i64 m, const u64 *__restrict__ skeys, const double *__restrict__ pts, GridDev g, const int *__restrict__ tile_ptr,
@@ -378,17 +265,6 @@ static int pt_check(r2s_ctx *ctx, const double *rho_n, const double *pts, i64 n,
   CK(cudaMemcpyAsync(ctx->pt_rn.p, rho_n, sizeof(double) * (size_t)ctx->nnp, cudaMemcpyHostToDevice, ctx->stream));
   return 0;
 }
-// per-tile lists from (tile << 32 | id) keys: sort, then the counts tile_cnt (at tile_ptr + 1) scanned into offsets
-static int pt_tile_lists(r2s_ctx *ctx, i64 nkeys, u64 **sorted) {
-  const GridDev &g = ctx->g; cudaStream_t st = ctx->stream;
-  int tbits = 1; while ((1ll << tbits) < g.ntiles) tbits++;
-  *sorted = ctx->pt_tkeys.as<u64>();
-  if (nkeys > 0 && r2s_sort_keys_u64(ctx, ctx->pt_tkeys.as<u64>(), ctx->pt_tkeys_alt.as<u64>(), nkeys, 32 + tbits, sorted)) return 1;
-  CK(ctx->pt_off.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-  if (r2s_scan_exclusive_i32(ctx, ctx->pt_tile_ptr.as<int>() + 1, ctx->pt_off.as<int>(), g.ntiles + 1)) return 1;
-  CK(cudaMemcpyAsync(ctx->pt_tile_ptr.as<int>(), ctx->pt_off.as<int>(), sizeof(int) * (size_t)(g.ntiles + 1), cudaMemcpyDeviceToDevice, st));
-  return 0;
-}
 // the chunk loop both calls share: upload, key, sort, run(m, sorted keys, device points), download, check the coordinates
 template <class RUN>
 static int pt_chunks(r2s_ctx *ctx, const double *pts, i64 n, int kind, RUN run) {
@@ -398,8 +274,8 @@ static int pt_chunks(r2s_ctx *ctx, const double *pts, i64 n, int kind, RUN run) 
   CK(ctx->pt_in.reserve(sizeof(double) * 3 * (size_t)ch));
   CK(ctx->pt_keys.reserve(sizeof(u64) * (size_t)ch));
   CK(ctx->pt_keys_alt.reserve(sizeof(u64) * (size_t)ch));
-  CK(ctx->pt_ctr.reserve(sizeof(u64) * 8 * 129 + sizeof(int)));
-  int *err = (int *)(ctx->pt_ctr.as<u64>() + 8 * 129);
+  CK(ctx->pt_ctr.reserve(sizeof(int)));
+  int *err = ctx->pt_ctr.as<int>();
   for (i64 s0 = 0; s0 < n; s0 += ch) {
     const i64 m = std::min(ch, n - s0);
     CK(cudaMemsetAsync(err, 0, sizeof(int), st));
@@ -418,60 +294,27 @@ static int pt_chunks(r2s_ctx *ctx, const double *pts, i64 n, int kind, RUN run) 
 int r2s_points_distances(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, const double *pts, i64 n, double *dist, double *xp) {
   if (pt_check(ctx, rho_n, pts, n, dist)) return 1;
   const GridDev &g = ctx->g; cudaStream_t st = ctx->stream;
-  const i64 nel = ctx->nel; const int nen = ctx->nen;
+  const int nen = ctx->nen;
   const double delta = delta_factor * g.cell;
   const bool want_xp = xp != nullptr;
   CK(cudaEventRecord(ctx->ev[0], st));
-  CK(ctx->pt_ctr.reserve(sizeof(u64) * 8 * 129 + sizeof(int)));
-  u64 *ctr = ctx->pt_ctr.as<u64>();
-  CK(cudaMemsetAsync(ctr, 0, sizeof(u64) * 8 * 129, st));
-  CK(ctx->pt_cls.reserve((size_t)nel));
-  CK(ctx->pt_flag.reserve(sizeof(int) * (size_t)(nel + 1)));
-  CK(ctx->pt_idx.reserve(sizeof(int) * (size_t)(nel + 1)));
-  CK(cudaMemsetAsync(ctx->pt_flag.as<int>() + nel, 0, sizeof(int), st));
-  k_pt_classify<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->IEN32.as<int>(), ctx->pt_rn.as<double>(), ctx->fbnd.as<unsigned char>(), rho_t, ctx->pt_cls.as<unsigned char>(),
-                                                ctx->pt_flag.as<int>(), ctr); LAUNCH_CHECK();
-  if (r2s_scan_exclusive_i32(ctx, ctx->pt_flag.as<int>(), ctx->pt_idx.as<int>(), nel + 1)) return 1;
-  int nact_i = 0;
-  if (r2s_readback(ctx, &nact_i, ctx->pt_idx.as<int>() + nel, sizeof(int))) return 1;
-  const i64 nact = nact_i;
-  CK(ctx->pt_tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-  CK(cudaMemsetAsync(ctx->pt_tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
-  i64 nkeys = 0; int ntri = 0;
-  u64 *tsorted = ctx->pt_tkeys.as<u64>();
-  if (nact > 0) {
-    CK(ctx->pt_rec.reserve(sizeof(ActRec) * (size_t)nact));
-    CK(ctx->pt_cnt.reserve((sizeof(i64) + sizeof(int)) * 2 * (size_t)(nact + 1)));
-    i64 *ntile = ctx->pt_cnt.as<i64>(), *toff = ntile + (nact + 1);
-    int *ntr = (int *)(toff + (nact + 1)), *troff = ntr + (nact + 1);
-    CK(cudaMemsetAsync(ntile + nact, 0, sizeof(i64), st));
-    CK(cudaMemsetAsync(ntr + nact, 0, sizeof(int), st));
-    k_pt_records<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->nsn, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_cls.as<unsigned char>(), ctx->fbnd.as<unsigned char>(),
-                                                 ctx->pt_flag.as<int>(), ctx->pt_idx.as<int>(), g, delta, ctx->pt_rec.as<ActRec>(), ntile, ntr); LAUNCH_CHECK();
-    if (r2s_scan_exclusive_i64(ctx, ntile, toff, nact + 1)) return 1;
-    if (r2s_scan_exclusive_i32(ctx, ntr, troff, nact + 1)) return 1;
-    const size_t o0 = r2s_rb_put(ctx, toff + nact, sizeof(i64)), o1 = r2s_rb_put(ctx, troff + nact, sizeof(int));
-    if (o0 == (size_t)-1 || o1 == (size_t)-1 || r2s_rb_sync(ctx)) return 1;
-    nkeys = *(const i64 *)r2s_rb_at(ctx, o0); ntri = *(const int *)r2s_rb_at(ctx, o1);
-    if (nkeys >= (1ll << 31)) FAIL("points: too many (tile, element) pairs");
-    CK(ctx->pt_tkeys.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
-    CK(ctx->pt_tkeys_alt.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
-    CK(ctx->pt_tri.reserve(sizeof(TriRec) * (size_t)(ntri + 1)));
-    if (nen == 8) CK(ctx->pt_hex.reserve(sizeof(PtHex) * (size_t)nact));
-#define EMIT(NEN) k_pt_emit<NEN><<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->pt_rec.as<ActRec>(), toff, troff, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), \
-      ctx->ebox.as<unsigned char>(), ctx->knobs.proj_box, g, delta, rho_t, ctx->pt_tkeys.as<u64>(), ctx->pt_tile_ptr.as<int>() + 1, ctx->pt_tri.as<TriRec>(), ctx->pt_hex.as<PtHex>())
-    if (nen == 8) EMIT(8); else EMIT(4);
-#undef EMIT
-    LAUNCH_CHECK();
+  DistBins bins;
+  if (r2s_dist_bins(ctx, ctx->pt_rn.as<double>(), rho_t, delta, true, &bins)) return 1;
+  const i64 nact = bins.nact;
+  const u64 *tsorted = bins.sorted;
+  u64 *ctr = ctx->counters.as<u64>();      // word 0, 1: the element classes (r2s_dist_bins); slots 1..128: k_pt_dist's statistics
+  if (nen == 8 && nact > 0) {
+    CK(ctx->pt_hex.reserve(sizeof(bnd::HexSetup) * (size_t)nact));
+    k_pt_hex<<<cdiv(nact, 128), 128, 0, st>>>(nact, ctx->act_rec.as<ActRec>(), ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), ctx->ebox.as<unsigned char>(),
+                                              ctx->knobs.proj_box, rho_t, ctx->pt_hex.as<bnd::HexSetup>()); LAUNCH_CHECK();
   }
-  if (pt_tile_lists(ctx, nkeys, &tsorted)) return 1;
   CK(cudaEventRecord(ctx->ev[1], st));
   CK(ctx->pt_out.reserve(sizeof(double) * 4 * (size_t)std::min<i64>(PT_CHUNK, std::max<i64>(n, 1))));
   double *dd = ctx->pt_out.as<double>(), *dx = dd + std::min<i64>(PT_CHUNK, std::max<i64>(n, 1));
   const int prune = ctx->knobs.proj_prune ? 1 : 0;
   auto run = [&](i64 s0, i64 m, const u64 *sk) -> int {
-#define DIST(XP, NEN) k_pt_dist<XP, NEN><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->pt_tile_ptr.as<int>(), tsorted, ctx->pt_rec.as<ActRec>(), \
-      ctx->pt_tri.as<TriRec>(), ctx->pt_hex.as<PtHex>(), ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, prune, dd, dx, ctr)
+#define DIST(XP, NEN) k_pt_dist<XP, NEN><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->tile_ptr.as<int>(), tsorted, ctx->act_rec.as<ActRec>(), \
+      ctx->tri_rec.as<TriRec>(), ctx->pt_hex.as<bnd::HexSetup>(), ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, prune, dd, dx, ctr)
     if (nen == 8) { if (want_xp) DIST(true, 8); else DIST(false, 8); }
     else { if (want_xp) DIST(true, 4); else DIST(false, 4); }
 #undef DIST
@@ -499,31 +342,32 @@ int r2s_points_signs(r2s_ctx *ctx, const double *rho_n, double rho_t, const doub
   const GridDev &g = ctx->g; cudaStream_t st = ctx->stream;
   const i64 nel = ctx->nel; const int nen = ctx->nen;
   CK(cudaEventRecord(ctx->ev[0], st));
-  // sign records in pt_hex (SPRec per element), the affine inverse-map data in pt_rec, tile counts / offsets in pt_cnt
+  // sign records in pt_hex (SPRec per element), the affine inverse-map data in s_el, tile counts / offsets in cnt_a / cnt_b
   CK(ctx->pt_hex.reserve(sizeof(SPRec) * (size_t)nel));
-  if (nen == 8) CK(ctx->pt_rec.reserve(sizeof(SignEl) * (size_t)nel));
-  CK(ctx->pt_cnt.reserve(sizeof(i64) * 2 * (size_t)(nel + 1)));
-  CK(ctx->pt_tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-  CK(cudaMemsetAsync(ctx->pt_tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
-  i64 *ntile = ctx->pt_cnt.as<i64>(), *toff = ntile + (nel + 1);
+  if (nen == 8) CK(ctx->s_el.reserve(sizeof(SignEl) * (size_t)nel));
+  CK(ctx->cnt_a.reserve(sizeof(i64) * (size_t)(nel + 1)));
+  CK(ctx->cnt_b.reserve(sizeof(i64) * (size_t)(nel + 1)));
+  CK(ctx->s_tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
+  CK(cudaMemsetAsync(ctx->s_tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
+  i64 *ntile = ctx->cnt_a.as<i64>(), *toff = ctx->cnt_b.as<i64>();
   CK(cudaMemsetAsync(ntile + nel, 0, sizeof(i64), st));
-  SPRec *rng = ctx->pt_hex.as<SPRec>(); SignEl *sel = ctx->pt_rec.as<SignEl>();
+  SPRec *rng = ctx->pt_hex.as<SPRec>(); SignEl *sel = ctx->s_el.as<SignEl>();
   k_pt_sign_records<<<cdiv(nel, 256), 256, 0, st>>>(nel, nen, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, g, rng, sel, ntile); LAUNCH_CHECK();
   if (r2s_scan_exclusive_i64(ctx, ntile, toff, nel + 1)) return 1;
   i64 nkeys = 0;
   if (r2s_readback(ctx, &nkeys, toff + nel, sizeof(i64))) return 1;
   if (nkeys >= (1ll << 31)) FAIL("points: too many (tile, element) pairs");
-  CK(ctx->pt_tkeys.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
-  CK(ctx->pt_tkeys_alt.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
-  if (nkeys > 0) { k_pt_sign_emit<<<cdiv(nel, 128), 128, 0, st>>>(nel, rng, toff, g, ctx->pt_tkeys.as<u64>(), ctx->pt_tile_ptr.as<int>() + 1); LAUNCH_CHECK(); }
+  CK(ctx->s_keys.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
+  CK(ctx->s_keys_alt.reserve(sizeof(u64) * (size_t)(nkeys + 1)));
+  if (nkeys > 0) { k_pt_sign_emit<<<cdiv(nel, 128), 128, 0, st>>>(nel, rng, toff, g, ctx->s_keys.as<u64>(), ctx->s_tile_ptr.as<int>() + 1); LAUNCH_CHECK(); }
   u64 *tsorted = nullptr;
-  if (pt_tile_lists(ctx, nkeys, &tsorted)) return 1;
+  if (r2s_tile_lists(ctx, ctx->s_keys.as<u64>(), ctx->s_keys_alt.as<u64>(), nkeys, ctx->s_tile_ptr.as<int>(), &tsorted)) return 1;
   CK(cudaEventRecord(ctx->ev[1], st));
   CK(ctx->pt_out.reserve(sizeof(double) * (size_t)std::min<i64>(PT_CHUNK, std::max<i64>(n, 1))));
   double *ds = ctx->pt_out.as<double>();
   auto run = [&](i64 s0, i64 m, const u64 *sk) -> int {
-    if (nen == 8) k_pt_sign<8><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->pt_tile_ptr.as<int>(), tsorted, rng, sel, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, ds);
-    else k_pt_sign<4><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->pt_tile_ptr.as<int>(), tsorted, rng, sel, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, ds);
+    if (nen == 8) k_pt_sign<8><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->s_tile_ptr.as<int>(), tsorted, rng, sel, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, ds);
+    else k_pt_sign<4><<<cdiv(m, 128), 128, 0, st>>>(m, sk, ctx->pt_in.as<double>(), g, ctx->s_tile_ptr.as<int>(), tsorted, rng, sel, ctx->IEN32.as<int>(), ctx->X.as<double>(), ctx->pt_rn.as<double>(), rho_t, ds);
     LAUNCH_CHECK();
     CK(cudaMemcpyAsync(signs + s0, ds, sizeof(double) * (size_t)m, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));

@@ -10,6 +10,15 @@ template <bool WANT_XP>
 __device__ __forceinline__ void write_value(VoxState &s, double dt, const double xp[3]) {   // WriteValue :44-57
   if (fabs(dt) < fabs(s.c)) { s.c = dt; if (WANT_XP) { s.xp[0] = xp[0]; s.xp[1] = xp[1]; s.xp[2] = xp[2]; } }
 }
+// Lower bound of |x - y| over the box [lo, hi] not below the running value c: nothing a triangle (or an element's triangles) in that box
+// writes can pass WriteValue's strict `<`.  The margins cover the rounding of the candidate distances.
+__device__ __forceinline__ bool box_not_below(const double lo[3], const double hi[3], const double x[3], double c) {
+  double lb2 = 0.0;
+#pragma unroll
+  for (int d = 0; d < 3; d++) { const double e = fmax(fmax(lo[d] - x[d], x[d] - hi[d]), 0.0); lb2 = fma(e, e, lb2); }
+  const double cv = fabs(c) * (1.0 + 1e-12);
+  return lb2 * (1.0 - 1e-12) > cv * cv;
+}
 // IsProjectedOnFullSegment (:78-119)
 template <bool WANT_XP, int NEN>
 __device__ inline bool projected_on_full_segment(const double Xe[3][NEN], const double re[NEN], double rho_t, const double xp[3], const double x[3], VoxState &s,

@@ -11,13 +11,9 @@
 #include "r2s_exact.cuh"
 #include "r2s_signrule.cuh"
 
-struct SRange { int a[3], b[3]; int hot, pad; };   // inclusive grid-point index range of the candidate points of one element; pad = density class (below);
+struct SRange { int a[3], b[3]; int hot, pad; };   // inclusive grid-point index range of the candidate points of one element; pad = density class (sign_element);
                                                    // hot = some nodal density >= rho_t (HEX8 skip rule, SignDetection.jl:36)
 
-__device__ __forceinline__ int tet_cell_index(double x, double amin, double cell, int n1) {   // point_to_grid_index :256-268 (1-based, clamped)
-  int idx = (int)floor(ex::dvd(ex::sub(x, amin), cell)) + 1;
-  return max(1, min(n1, idx));
-}
 __global__ void k_sign_ranges(i64 nel, int nen, const int *__restrict__ IEN, const double *__restrict__ X, const double *__restrict__ rn, double rho_t,
                               GridDev g, int kz0, int kz1, const double2 *__restrict__ ezr, double zlo, double zhi, SRange *__restrict__ rng, i64 *__restrict__ ntile,
                               SignEl *__restrict__ sel) {
@@ -25,66 +21,40 @@ __global__ void k_sign_ranges(i64 nel, int nen, const int *__restrict__ IEN, con
   if (e >= nel) return;
   { const double2 z = ezr[e];      // z-slab: elements that cannot reach this rank's planes get an empty range without touching their nodes
     if (z.y < zlo || z.x > zhi) { SRange r; r.a[0] = 1; r.b[0] = 0; r.a[1] = r.a[2] = 1; r.b[1] = r.b[2] = 0; r.hot = 0; r.pad = 0; rng[e] = r; ntile[e] = 0; return; } }
-
-  double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300}, rmax = -1e300, rmin = 1e300;
-  for (int a = 0; a < nen; a++) { i64 n = IEN[nen * e + a]; rmax = fmax(rmax, rn[n]); rmin = fmin(rmin, rn[n]); for (int d = 0; d < 3; d++) { double c = X[3 * n + d]; lo[d] = fmin(lo[d], c); hi[d] = fmax(hi[d], c); } }
+  SignElem E; sign_element(e, nen, IEN, X, rn, rho_t, g, E);
   SRange r; bool ok = true;
-  // Density class of a HEX8 element for the opt-in shortcut of k_sign<8, true>: for max|xi| < 1.01 every shape function is above
-  // -0.01 * 2.01^2 / 8 and they sum to one, so the interpolated density stays within [rmin - 0.05 range, rmax + 0.05 range].
-  // 1: it is >= rho_t for every admissible xi (the test "rho >= rho_t" is known to hold), 2: it is < rho_t, 0: undecided.
-  r.pad = 0;
-  if (nen == 8) {
-    const double range = rmax - rmin, tolc = 1e-9 * fmax(1.0, fabs(rho_t));
-    if (rmin - 0.05 * range >= rho_t + tolc) r.pad = 1; else if (rmax + 0.05 * range < rho_t - tolc) r.pad = 2;
-  }
-  r.hot = (nen == 4 || !(rmax < rho_t)) ? 1 : 0;
+  r.pad = E.dcls; r.hot = E.hot;
   for (int d = 0; d < 3; d++) {
     const double *pc = g.pc + g.pc_off[d]; int n1 = g.np[d], a, b;
     if (nen == 8) {
-      // closed AABB test lo <= x <= hi (sdfOnDensityField.jl:60-69): first point >= lo, last point <= hi (pc is monotone)
+      // the grid points in the closed AABB: first point >= lo, last point <= hi (pc is monotone)
       int l = 0, h = n1;
-      while (l < h) { int m = (l + h) >> 1; if (pc[m] < lo[d]) l = m + 1; else h = m; }
+      while (l < h) { int m = (l + h) >> 1; if (pc[m] < E.lo[d]) l = m + 1; else h = m; }
       a = l; l = 0; h = n1;
-      while (l < h) { int m = (l + h) >> 1; if (pc[m] <= hi[d]) l = m + 1; else h = m; }
+      while (l < h) { int m = (l + h) >> 1; if (pc[m] <= E.hi[d]) l = m + 1; else h = m; }
       b = l - 1;
     } else {
       // create_grid_tetrahedra_mapping_TET4 (:195-196): cells max(1, floor((lo-min)/cell)-1) .. min(dims, ceil((hi-min)/cell)+1)
-      int mi = (int)floor(ex::dvd(ex::sub(lo[d], g.amin[d]), g.cell)) - 1; if (mi < 1) mi = 1;
-      int ma = (int)ceil(ex::dvd(ex::sub(hi[d], g.amin[d]), g.cell)) + 1; if (ma > n1) ma = n1;
+      int mi = (int)E.fl[d] - 1; if (mi < 1) mi = 1;
+      int ma = (int)E.cu[d] + 1; if (ma > n1) ma = n1;
       a = n1; b = -1;
       int p0 = max(0, mi - 4), p1 = min(n1 - 1, ma + 3);
-      for (int p = p0; p <= p1; p++) { int idx = tet_cell_index(pc[p], g.amin[d], g.cell, n1); if (idx >= mi && idx <= ma) { if (p < a) a = p; if (p > b) b = p; } }
+      for (int p = p0; p <= p1; p++) { int idx = pt_bin(pc[p], g.amin[d], g.cell, n1); if (idx >= mi && idx <= ma) { if (p < a) a = p; if (p > b) b = p; } }
     }
     if (d == 2) { if (a < kz0) a = kz0; if (b > kz1 - 1) b = kz1 - 1; }
     r.a[d] = a; r.b[d] = b; ok = ok && (a <= b);
   }
   if (!ok) { r.a[0] = 1; r.b[0] = 0; }
   rng[e] = r;
-  if (nen == 8 && ok) {      // only elements with candidate points in this slab
-    double A[3][8];
-    for (int d = 0; d < 3; d++) {
-      double v[8];
-      for (int a = 0; a < 8; a++) v[a] = X[3 * (i64)IEN[8 * e + a] + d];
-      ex::mono8(v, A[d]);
-    }
-    SignEl S; ex::affine_inverse_prepare(A, S);
-    sel[e] = S;
-  }
-  ntile[e] = ok ? (i64)(r.b[0] / TILE_X - r.a[0] / TILE_X + 1) * (r.b[1] / TILE_Y - r.a[1] / TILE_Y + 1) * (r.b[2] / TILE_Z - r.a[2] / TILE_Z + 1) : 0;
+  if (nen == 8 && ok) sel[e] = sign_affine(e, IEN, X);      // only elements with candidate points in this slab
+  ntile[e] = ok ? tile_span(r.a, r.b) : 0;
 }
 __global__ void k_sign_emit(i64 nel, const SRange *__restrict__ rng, const i64 *__restrict__ toff, GridDev g, u64 *__restrict__ keys, int *__restrict__ tile_cnt) {
   i64 e = blockIdx.x * (i64)blockDim.x + threadIdx.x;
   if (e >= nel) return;
   SRange r = rng[e];
   if (r.a[0] > r.b[0]) return;
-  i64 o = toff[e];
-  for (int tz = r.a[2] / TILE_Z; tz <= r.b[2] / TILE_Z; tz++)
-    for (int ty = r.a[1] / TILE_Y; ty <= r.b[1] / TILE_Y; ty++)
-      for (int tx = r.a[0] / TILE_X; tx <= r.b[0] / TILE_X; tx++) {
-        u64 t = ((u64)tz * g.nt[1] + ty) * g.nt[0] + tx;
-        keys[o++] = (t << 32) | (u64)e;
-        atomicAdd(&tile_cnt[t], 1);
-      }
+  emit_tile_keys(g, r.a, r.b, e, keys + toff[e], tile_cnt);
 }
 
 // One CTA per tile, one thread per grid point.  Each WARP walks the tile's element list 32 entries at a time, keeps the
@@ -92,7 +62,7 @@ __global__ void k_sign_emit(i64 nel, const SRange *__restrict__ rng, const i64 *
 // preserved), then every lane advances through that culled list on its own: all lanes run the expensive inverse map at
 // the same time, each on its own next candidate, instead of serialising over elements.
 #define CULL_CAP 96
-// CLS: candidates whose element is of density class 1 / 2 (k_sign_ranges) skip the gather of the eight
+// CLS: candidates whose element is of density class 1 / 2 (sign_element) skip the gather of the eight
 // nodal densities and the shape functions -- the outcome of "rho >= rho_t" is known; the state updates (max_local, break) are the same.
 template <int NEN, bool CLS>
 __global__ void __launch_bounds__(TILE_VOX, 2) k_sign(GridDev g, int kz0, int kz1, const int *__restrict__ tile_ptr, const u64 *__restrict__ keys,
@@ -205,7 +175,7 @@ __global__ void k_lat_info(i64 nel, const int *__restrict__ IEN, const double *_
   double rmax = -1e300, rmin = 1e300;
 #pragma unroll
   for (int a = 0; a < 8; a++) { const double r = rn[IEN[8 * e + a]]; rmax = fmax(rmax, r); rmin = fmin(rmin, r); }
-  unsigned cls = 0;      // same density classes as k_sign_ranges
+  unsigned cls = 0;      // same density classes as sign_element
   const double range = rmax - rmin, tolc = 1e-9 * fmax(1.0, fabs(rho_t));
   if (rmin - 0.05 * range >= rho_t + tolc) cls = 1; else if (rmax + 0.05 * range < rho_t - tolc) cls = 2;
   const unsigned hot = !(rmax < rho_t) ? 1u : 0u;
@@ -387,7 +357,6 @@ int r2s_dev_sign(r2s_ctx *ctx, double rho_t, bool write_signs, bool write_sdf) {
   CK(ctx->cnt_a.reserve(sizeof(i64) * (size_t)(nel + 1)));
   CK(ctx->cnt_b.reserve(sizeof(i64) * (size_t)(nel + 1)));
   CK(ctx->s_tile_ptr.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
-  CK(ctx->s_cnt.reserve(sizeof(int) * (size_t)(g.ntiles + 2)));
   CK(cudaMemsetAsync(ctx->s_tile_ptr.p, 0, sizeof(int) * (size_t)(g.ntiles + 2), st));
   CK(cudaMemsetAsync(ctx->cnt_a.as<i64>() + nel, 0, sizeof(i64), st));
   i64 *ntile = ctx->cnt_a.as<i64>(), *toff = ctx->cnt_b.as<i64>();
@@ -398,16 +367,13 @@ int r2s_dev_sign(r2s_ctx *ctx, double rho_t, bool write_signs, bool write_sdf) {
   i64 nkeys = 0;
   if (r2s_readback(ctx, &nkeys, toff + nel, sizeof(i64))) return 1;
   if (nkeys >= (1ll << 31)) FAIL("sign binning: too many (tile, element) pairs for one slab");
-  u64 *sorted = nullptr;
   if (nkeys > 0) {
     CK(ctx->s_keys.reserve(sizeof(u64) * (size_t)nkeys));
     CK(ctx->s_keys_alt.reserve(sizeof(u64) * (size_t)nkeys));
     k_sign_emit<<<cdiv(nel, 128), 128, 0, st>>>(nel, ctx->s_rng.as<SRange>(), toff, g, ctx->s_keys.as<u64>(), ctx->s_tile_ptr.as<int>() + 1); LAUNCH_CHECK();
-    int tbits = 1; while ((1ll << tbits) < g.ntiles) tbits++;
-    if (r2s_sort_keys_u64(ctx, ctx->s_keys.as<u64>(), ctx->s_keys_alt.as<u64>(), nkeys, 32 + tbits, &sorted)) return 1;
   }
-  if (r2s_scan_exclusive_i32(ctx, ctx->s_tile_ptr.as<int>() + 1, ctx->s_cnt.as<int>(), g.ntiles + 1)) return 1;
-  CK(cudaMemcpyAsync(ctx->s_tile_ptr.as<int>(), ctx->s_cnt.as<int>(), sizeof(int) * (size_t)(g.ntiles + 1), cudaMemcpyDeviceToDevice, st));
+  u64 *sorted = nullptr;
+  if (r2s_tile_lists(ctx, ctx->s_keys.as<u64>(), ctx->s_keys_alt.as<u64>(), nkeys, ctx->s_tile_ptr.as<int>(), &sorted)) return 1;
   double *signs = nullptr, *sdf = nullptr;
   if (write_signs) { CK(ctx->signs.reserve(sizeof(double) * (size_t)g.ngp)); signs = ctx->signs.as<double>(); }
   if (write_sdf) { CK(ctx->sdf.reserve(sizeof(double) * (size_t)g.ngp)); sdf = ctx->sdf.as<double>(); ctx->have_sdf = true; }

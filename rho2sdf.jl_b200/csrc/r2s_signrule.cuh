@@ -6,6 +6,44 @@
 
 typedef ex::AffineInv SignEl;      // per-element affine inverse-map data (r2s_exact.cuh)
 
+// point_to_grid_index (SignDetection.jl:256-268): clamp(floor((x - amin) / cell) + 1, 1, N + 1), clamped before the conversion
+__device__ __forceinline__ int pt_bin(double x, double amin, double cell, int n1) {
+  const double f = floor(ex::dvd(ex::sub(x, amin), cell)) + 1.0;
+  return f < 1.0 ? 1 : (f > (double)n1 ? n1 : (int)f);
+}
+// The element prologue of both sign binnings (k_sign_ranges on the grid, k_pt_sign_records for points): closed AABB lo <= x <= hi
+// (sdfOnDensityField.jl:60-69); hot = some nodal density >= rho_t (the skip rule, :36; every TET4 element); the density class of a HEX8
+// element for k_sign<8, true> (see k_sign_ranges); for TET4 per axis fl = floor((lo - amin) / cell) and cu = ceil((hi - amin) / cell), the
+// cell range of create_grid_tetrahedra_mapping_TET4 (:195-196) before its -1 / +1 and its clamps.
+struct SignElem { double lo[3], hi[3], fl[3], cu[3]; int hot, dcls; };
+__device__ __forceinline__ void sign_element(i64 e, int nen, const int *__restrict__ IEN, const double *__restrict__ X, const double *__restrict__ rn, double rho_t,
+                                             const GridDev &g, SignElem &E) {
+  double rmax = -1e300, rmin = 1e300;
+  for (int d = 0; d < 3; d++) { E.lo[d] = 1e300; E.hi[d] = -1e300; }
+  for (int a = 0; a < nen; a++) {
+    const i64 n = IEN[nen * e + a]; rmax = fmax(rmax, rn[n]); rmin = fmin(rmin, rn[n]);
+    for (int d = 0; d < 3; d++) { const double c = X[3 * n + d]; E.lo[d] = fmin(E.lo[d], c); E.hi[d] = fmax(E.hi[d], c); }
+  }
+  // HEX8 density class: for max|xi| < 1.01 every shape function is above -0.01 * 2.01^2 / 8 and they sum to one, so the interpolated density
+  // stays within [rmin - 0.05 range, rmax + 0.05 range].  1: it is >= rho_t for every admissible xi (the test "rho >= rho_t" is known to
+  // hold), 2: it is < rho_t, 0: undecided.
+  E.dcls = 0;
+  if (nen == 8) {
+    const double range = rmax - rmin, tolc = 1e-9 * fmax(1.0, fabs(rho_t));
+    if (rmin - 0.05 * range >= rho_t + tolc) E.dcls = 1; else if (rmax + 0.05 * range < rho_t - tolc) E.dcls = 2;
+  }
+  E.hot = (nen == 4 || !(rmax < rho_t)) ? 1 : 0;
+  if (nen == 4)
+    for (int d = 0; d < 3; d++) { E.fl[d] = floor(ex::dvd(ex::sub(E.lo[d], g.amin[d]), g.cell)); E.cu[d] = ceil(ex::dvd(ex::sub(E.hi[d], g.amin[d]), g.cell)); }
+}
+// the affine inverse-map data of HEX8 element e
+__device__ __forceinline__ SignEl sign_affine(i64 e, const int *__restrict__ IEN, const double *__restrict__ X) {
+  double A[3][8];
+  for (int d = 0; d < 3; d++) { double v[8]; for (int a = 0; a < 8; a++) v[a] = X[3 * (i64)IEN[8 * e + a] + d]; ex::mono8(v, A[d]); }
+  SignEl S; ex::affine_inverse_prepare(A, S);
+  return S;
+}
+
 // HEX8 candidate e in the loop over the point's candidates: sign and max_local carry the loop state; returns true at the loop's break
 // (:51-59).  dcls = density class of the element (k_sign_ranges: 1 rho >= rho_t, 2 rho < rho_t wherever max|xi| < 1.01) or 0 = evaluate.
 __device__ __forceinline__ bool sign_hex8_candidate(const SignEl &S, int e, const int *__restrict__ IEN, const double *__restrict__ X, const double *__restrict__ rn,

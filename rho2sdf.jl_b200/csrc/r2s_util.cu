@@ -30,6 +30,16 @@ int r2s_sort_keys_u64(r2s_ctx *ctx, u64 *keys, u64 *alt, i64 n, int end_bit, u64
   *sorted = db.Current();
   return 0;
 }
+int r2s_tile_lists(r2s_ctx *ctx, u64 *keys, u64 *alt, i64 nkeys, int *tile_ptr, u64 **sorted) {
+  const i64 ntiles = ctx->g.ntiles;
+  int tbits = 1; while ((1ll << tbits) < ntiles) tbits++;
+  *sorted = keys;
+  if (nkeys > 0 && r2s_sort_keys_u64(ctx, keys, alt, nkeys, 32 + tbits, sorted)) return 1;
+  CK(ctx->s_cnt.reserve(sizeof(int) * (size_t)(ntiles + 2)));
+  if (r2s_scan_exclusive_i32(ctx, tile_ptr + 1, ctx->s_cnt.as<int>(), ntiles + 1)) return 1;
+  CK(cudaMemcpyAsync(tile_ptr, ctx->s_cnt.as<int>(), sizeof(int) * (size_t)(ntiles + 1), cudaMemcpyDeviceToDevice, ctx->stream));
+  return 0;
+}
 
 // sorts n doubles ascending (used by the edge-length median of the grid set-up)
 int r2s_sort_f64(r2s_ctx *ctx, double *keys, double *alt, i64 n, double **sorted) {

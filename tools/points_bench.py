@@ -70,7 +70,7 @@ def main():
         rep = c.report()
         out.update(dist_s=t, dist_ns_per_point=t / n * 1e9, pairs_per_point=(rep.n_pairs - rep.n_pairs_pruned) / n, pairs_in_range_per_point=rep.n_pairs / n,
                    pruned_share=rep.n_pairs_pruned / max(rep.n_pairs, 1), not_converged=rep.n_not_converged)
-        out["dist_kernel_ms"] = kernel_ms(lambda: r2s.evalDistances(mesh, grid, P, rn, rt, delta_factor=delta, want_xp=False), ["k_pt_dist", "k_pt_emit", "k_pt_keys"])
+        out["dist_kernel_ms"] = kernel_ms(lambda: r2s.evalDistances(mesh, grid, P, rn, rt, delta_factor=delta, want_xp=False), ["k_pt_dist", "k_pt_hex", "k_pt_keys"])
         t = timed(lambda: r2s.Sign_Detection(mesh, grid, P, rn, rt))
         out.update(sign_s=t, sign_ns_per_point=t / n * 1e9)
         out["sign_kernel_ms"] = kernel_ms(lambda: r2s.Sign_Detection(mesh, grid, P, rn, rt), ["k_pt_sign", "k_pt_keys"])
