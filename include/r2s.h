@@ -254,6 +254,46 @@ int r2s_multi_sample_sdf(r2s_multi *m, const double *points, int64_t n, float *v
 int r2s_multi_sample_sdf_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float *values);
 int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th);
 
+/* ---- zero surface of the continuous field on any lattice (csrc/r2s_surf.cu, r2s_snap.cuh) ---------------------------------------- */
+/* The surface {f = iso} of the continuous smoothed field f above (the field r2s_sample_sdf evaluates) on the lattice origin + i * spacing,
+ * i < dims, streamed through the device: the lattice values are never held whole and never leave the device.
+ *   lattice values: a lattice point's value is bit for bit what r2s_sample_sdf_lattice returns for it; its coordinates are
+ *     float(origin_d) + float(i_d) * float(spacing_d) in Float32 (rule 7 above)
+ *   topology and triangles: exactly those of r2s_isosurface_from_sdf applied to that lattice field with the same origin, spacing and iso
+ *     -- the same corner rule (inside iff value >= iso), face rule and case table (r2s_mc.cuh), vertex numbering (the edge's lower point,
+ *     then axis x < y < z), triangle order and orientation.  The triangle array is identical, so the mesh is closed and consistently
+ *     oriented wherever that one is, and the vertex count is equal.
+ *   vertex placement: a crossing edge runs from lattice point a to lattice point b along axis d (a the lower point).  The vertex's two
+ *     other coordinates are the lattice's Float32 coordinates; its axis-d coordinate is a Float32 x in [x_a, x_b] found by a deterministic
+ *     bracketing search over Float32 values, with f evaluated by the sampler's per-point arithmetic (rules 1-6; s(x) = f(x) >= iso):
+ *       bracket (lo, hi) = (x_a, x_b), keeping s(lo) = s(a), s(hi) = s(b); it starts from the lattice values (no re-evaluation).
+ *       step: the Illinois regula-falsi point lo + (hi - lo) * glo / (glo - ghi) in double (every operation rounded, glo / ghi the residuals
+ *         f - iso of the two ends, the one kept twice in a row halved), rounded to float; if it is not strictly inside (lo, hi) the step
+ *         takes the midpoint of lo and hi in the order-preserving integer image of the floats instead.  One evaluation per step.
+ *       stop: lo and hi are adjacent floats, or R2S_SNAP_MAX_EVALS = 48 evaluations have been made.
+ *       result: whichever of lo and hi has the smaller |f - iso| (in double), ties to lo.
+ *     csrc/r2s_snap.cuh states every operation; a host build replays it bit for bit.  The vertex stays on its own edge, so connectivity
+ *     and closedness are those of the triangle array.  These coordinates are in the sampler's Float32 lattice frame, which differs in the
+ *     last bit from the double frame origin + spacing * (p + t) of r2s_isosurface / r2s_isosurface_from_sdf: a vertex that the search
+ *     leaves at a lattice point can differ from that frame by one rounding.
+ *   memory: planes stream through a device buffer of a bounded number of planes (R2S_SURF_PLANES per chunk, read by r2s_create; default
+ *     as many as fit 1 GiB of values) plus the two planes above a chunk that marching cubes reads; every plane is sampled twice (a count
+ *     sweep, then an emit sweep after a host scan of the chunk totals).  Device memory: O((chunk planes + 2) * nx * ny + per-row scratch
+ *     of a chunk + the output mesh).  The mesh does not depend on the chunk size.
+ *   determinism: the mesh is a function of (weights, th, lattice, iso) alone: the same for any chunk size, on one context and on any slab
+ *     layout of r2s_multi (given the same weights).  Several slabs: each extracts the lattice planes r2s_multi_sample_sdf_lattice assigns
+ *     it; it evaluates the two lattice planes above its last plane itself, and every evaluation (lattice points and the search) reads the
+ *     weights of the slab that owns the point's floor plane, through peer memory -- the rule of r2s_multi_sample_sdf, so every value is the
+ *     one that slab computes.  Global bases come from a host scan of the slab totals in plane order.
+ * Rejected with an error: no smoothed field on the device, a non-finite origin, spacing or lattice coordinate, dims < 2 on an axis, 2^31
+ * or more cells or vertices, a non-finite iso; the single-context call fails on a slab rank of the NCCL communicator (use r2s_multi).
+ * sdf_dists, fine_sdf, the weights and th are untouched; the mesh replaces this context's (handle's) surface: download / export it with
+ * r2s_download_isosurface / r2s_export_isosurface (r2s_multi_download_isosurface / r2s_multi_export_isosurface). */
+int r2s_isosurface_lattice(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
+                           int64_t *n_vertices, int64_t *n_triangles);
+int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
+                                 int64_t *n_vertices, int64_t *n_triangles);
+
 /* ---- measurement helper (bench.py): FMA-pipe peak of the device in TFLOP/s, fp64 != 0 -> double, else float -------- */
 int r2s_measure_fma_peak(r2s_ctx *ctx, int fp64, double *tflops);
 

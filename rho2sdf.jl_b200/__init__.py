@@ -9,7 +9,7 @@ image, so this module carries the same names, argument meaning and error behavio
     find_threshold_for_volume, calculate_isocontour_volume                  (src/MeshGrid/*)
     evalDistances, Sign_Detection, remove_sdf_artifacts                     (src/SignedDistances/*)
     RBFs_smoothing, calculate_volume_from_sdf                               (src/SdfSmoothing/*)
-    isosurface, isosurface_from_sdf, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}; the reference leaves it to
+    isosurface, isosurface_from_sdf, isosurface_lattice, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}, or of the continuous field on any lattice; the reference leaves it to
                                                                              src/Visualizations / ParaView)
     sample_sdf, sample_sdf_lattice, rbf_weights                             (the smoothed SDF as a continuous function:
                                                                              rbf_interpolation_kdtree, RBFs4Smoothing.jl:219-248)
@@ -29,7 +29,7 @@ __all__ = ["HEX8", "TET4", "Rho2sdfOptions", "Mesh", "Grid", "getMesh_AABB", "ge
            "DenseInNodes", "find_threshold_for_volume", "calculate_isocontour_volume", "evalDistances", "Sign_Detection",
            "remove_sdf_artifacts", "RBFs_smoothing", "calculate_volume_from_sdf", "rho2sdf", "rho2sdf_hex8", "rho2sdf_tet4",
            "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti",
-           "isosurface", "isosurface_from_sdf", "export_isosurface", "read_stl", "read_ply",
+           "isosurface", "isosurface_from_sdf", "isosurface_lattice", "export_isosurface", "read_stl", "read_ply",
            "sample_sdf", "sample_sdf_lattice", "rbf_weights", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -144,6 +144,8 @@ def load_library():
     L.r2s_multi_isosurface.argtypes = [vp, C.c_float, ip, ip]
     L.r2s_multi_download_isosurface.argtypes = [vp, vp, vp]
     L.r2s_multi_export_isosurface.argtypes = [vp, C.c_char_p, C.c_int]
+    L.r2s_isosurface_lattice.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip]
+    L.r2s_multi_isosurface_lattice.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip]
     for pre in ("r2s_", "r2s_multi_"):
         getattr(L, pre + "sample_sdf").argtypes = [vp, vp, C.c_int64, vp, vp]
         getattr(L, pre + "sample_sdf_lattice").argtypes = [vp, vp, vp, vp, vp]
@@ -652,8 +654,20 @@ def _download_surface(obj, download, nv, nt):
     return V, T
 
 
-def _extract(mesh, iso):
+def _lattice_args(origin, spacing, shape):
+    o = _f64(np.broadcast_to(np.asarray(origin, dtype=np.float64), (3,)))
+    h = _f64(np.broadcast_to(np.asarray(spacing, dtype=np.float64), (3,)))
+    dims = np.ascontiguousarray(np.broadcast_to(np.asarray(shape, dtype=np.int64), (3,)))
+    return o, h, dims
+
+
+def _extract(mesh, iso, lattice=None):
     nv, nt = C.c_int64(), C.c_int64()
+    if lattice is not None:
+        o, h, dims = _lattice_args(*lattice)
+        obj, pre = _sampler(mesh)
+        obj.check(getattr(obj.lib, pre + "isosurface_lattice")(obj.h, _ptr(o), _ptr(h), _ptr(dims), float(iso), C.byref(nv), C.byref(nt)))
+        return obj, getattr(obj.lib, pre + "download_isosurface"), nv.value, nt.value
     if mesh.multi is not None:
         m = mesh.multi
         m.check(m.lib.r2s_multi_isosurface(m.h, float(iso), C.byref(nv), C.byref(nt)))
@@ -686,10 +700,21 @@ def isosurface_from_sdf(fine_sdf, origin, spacing, iso=0.0, ctx=None):
     return _download_surface(c, c.lib.r2s_download_isosurface, nv.value, nt.value)
 
 
-def export_isosurface(mesh, path, iso=0.0):
-    """Extract {fine_sdf = iso} on the device(s) of `mesh` and write it to `path`: binary STL (.stl) or binary little-endian PLY (.ply)."""
+def isosurface_lattice(mesh, origin, spacing, shape, iso=0.0):
+    """Triangle mesh of {f = iso} for the continuous field f of the last pipeline / smoothing call on the device(s) of `mesh` (what
+    sample_sdf evaluates), extracted on the lattice origin + i * spacing, i < shape (the arguments of sample_sdf_lattice) without holding
+    the lattice field anywhere.  The triangles are those of isosurface_from_sdf(sample_sdf_lattice(mesh, origin, spacing, shape), origin,
+    spacing, iso); each vertex lies on its lattice edge at the Float32 coordinate that a bracketing search on f finds closest to the zero
+    set (include/r2s.h states the rule).  Returns (V (nv, 3) float32, T (nt, 3) int32, 0-based)."""
+    obj, dl, nv, nt = _extract(mesh, iso, (origin, spacing, shape))
+    return _download_surface(obj, dl, nv, nt)
+
+
+def export_isosurface(mesh, path, iso=0.0, lattice=None):
+    """Extract {fine_sdf = iso} on the device(s) of `mesh` and write it to `path`: binary STL (.stl) or binary little-endian PLY (.ply).
+    lattice=(origin, spacing, shape): extract the continuous field's surface on that lattice instead, as isosurface_lattice does."""
     fmt = _surface_format(path)
-    obj, _, _, _ = _extract(mesh, iso)
+    obj, _, _, _ = _extract(mesh, iso, lattice)
     if mesh.multi is not None:
         obj.check(obj.lib.r2s_multi_export_isosurface(obj.h, str(path).encode(), fmt))
     else:

@@ -68,6 +68,18 @@ struct Knobs {
   int proj_prune = 1;     // R2S_PROJ_PRUNE=0: the box projection evaluates every (element, point) pair (no lower-bound pruning)
   int debug_sync = 0;     // R2S_DEBUG_SYNC=1: synchronise after every kernel launch, so that a device fault is reported at the launch that caused it
   int vol_cache = 1;      // R2S_VOL_CACHE=0: LS_Threshold re-evaluates every cut cell at every bisection (no cached quadratures)
+  int surf_planes = 0;    // R2S_SURF_PLANES=n: lattice planes per chunk of r2s_isosurface_lattice (0: as many as fit SURF_LAT_BUDGET bytes)
+};
+
+// weights of the slab that owns the coarse planes below k1 (r2s_isosurface_lattice: every evaluation reads the weights of the slab that
+// owns the point's floor plane, as r2s_multi_sample_sdf routes it; one entry with k1 = INT64_MAX on a single context)
+struct SurfSlabW { i64 k1; const float *w; long long px; };
+// the lattice surface of one context between its two sweeps: lattice frame (Float32), its lattice planes [ka, kb), planes per chunk,
+// the chunk counts of the first sweep
+struct SurfLattice {
+  float o[3], h[3]; int64_t dims[3]; float iso; i64 ka, kb, planes;
+  std::vector<SurfSlabW> slabs;
+  std::vector<i64> cnv, cnt;
 };
 
 struct LocalGroup;      // in-process slab group (r2s_multi_*): r2s_comm.cu
@@ -145,6 +157,9 @@ struct r2s_ctx {
   const float *surf_f = nullptr; i64 surf_nx = 0, surf_ny = 0, surf_nz = 0, surf_z0 = 0, surf_z1 = 0; float surf_iso = 0.0f;
   double surf_origin[3] = {0, 0, 0}, surf_spacing[3] = {0, 0, 0};
   i64 surf_nv = 0, surf_nt = 0, surf_vglob = 0, surf_nv_all = 0, surf_nt_all = 0;
+  // r2s_isosurface_lattice: the chunk of sampled lattice planes, the device copy of surf_lat.slabs
+  DevBuf surf_buf, surf_wtab;
+  SurfLattice surf_lat;
 };
 
 #define CK(call)                                                                                   \
@@ -225,6 +240,10 @@ int r2s_surf_count_slab(r2s_ctx *ctx, float iso, i64 *nv, i64 *nt);       // pas
 int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);                  // pass 2 with this slab's first global vertex id
 int r2s_surf_download_slab(r2s_ctx *ctx, float *V, int32_t *T, i64 tglob, bool staging);   // this slab's part into the whole arrays
 int r2s_surf_write_file(const char *path, int format, const float *V, i64 nv, const int *T, i64 nt, std::string *err);
+// the surface of the continuous field on a lattice (r2s_isosurface_lattice): checks, then two sweeps over ctx->surf_lat's planes
+int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3]);
+int r2s_surf_lattice_count(r2s_ctx *ctx, i64 *nv, i64 *nt);                // sweep 1: chunk counts, this context's totals
+int r2s_surf_lattice_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);          // sweep 2: emit + snap with this context's first global vertex id
 // r2s_sample.cu: the sampler of the continuous field, for r2s_rbf.cu (record) and r2s_multi.cu (one slab's share, no rank check)
 struct SampleGrid;
 int r2s_sample_record(r2s_ctx *ctx, const float *w, int px, float th, double rbf_cut);
@@ -232,6 +251,7 @@ int r2s_sample_grid(r2s_ctx *ctx, SampleGrid *G, bool dev);
 int r2s_sample_points_ctx(r2s_ctx *ctx, const double *pts, i64 n, float *val, float *grad);
 int r2s_sample_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float o[3], float h[3]);
 int r2s_sample_lattice_planes(r2s_ctx *ctx, const float o[3], const float h[3], const int64_t dims[3], i64 ka, i64 kb, float *out);
+int r2s_sample_lattice_dev(r2s_ctx *ctx, const SampleGrid &G, const float o[3], const float h[3], const int64_t dims[3], i64 ka, i64 kb, float *out_dev);
 int r2s_sample_download_weights(r2s_ctx *ctx, float *w, float *th, i64 k0, i64 k1);
 // r2s_points.cu: evalDistances / Sign_Detection at n host points (rho_n on the host)
 int r2s_points_distances(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, const double *pts, i64 n, double *dist, double *xp);

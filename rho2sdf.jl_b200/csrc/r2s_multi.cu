@@ -297,6 +297,72 @@ int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th) {
   return run_all(m, [&](int r) { return r2s_sample_download_weights(m->ctx[(size_t)r], weights, r == 0 ? th : nullptr, m->cut[(size_t)r], m->cut[(size_t)r + 1]); });
 }
 
+// Zero surface of the continuous field on a lattice (r2s_surf.cu): every slab extracts the lattice planes r2s_multi_sample_sdf_lattice
+// gives it (a contiguous run, since the plane z is monotone in k), reading the two planes above its run -- and every snapping evaluation
+// -- with the weights of the slab owning the point's floor plane, through peer memory (plain pointers on a shared device).  The weights
+// are settled when the call starts and nothing writes them during it, so no exchange is ordered.  The host scans the slab counts in plane
+// order, as r2s_multi_isosurface does in slab order.
+int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                                 int64_t *n_triangles) {
+  if (!m) return 1;
+  if (!m->has_grid) { m->err = "r2s_multi_set_grid has not been called"; return 1; }
+  m->have_surface = false;
+  if (m->n == 1) {
+    int64_t a = 0, b = 0;
+    if (r2s_isosurface_lattice(m->ctx[0], origin, spacing, dims, iso, &a, &b)) { m->err = m->ctx[0]->err; return 1; }
+    m->surf_vb.assign({0, a}); m->surf_tb.assign({0, b});
+    m->have_surface = true;
+    if (n_vertices) *n_vertices = a;
+    if (n_triangles) *n_triangles = b;
+    return 0;
+  }
+  for (int r = 0; r < m->n; r++) m->ctx[(size_t)r]->have_surface = false;
+  float o[3], h[3];
+  SampleGrid G;
+  if (multi_sample_ready(m, &G)) return 1;
+  if (r2s_surf_lattice_check(m->ctx[0], origin, spacing, dims, iso, o, h)) { m->err = m->ctx[0]->err; return 1; }
+  std::vector<i64> ka((size_t)m->n, 0), kb((size_t)m->n, 0);
+  std::vector<bool> seen((size_t)m->n, false);
+  int prev = -1;
+  for (i64 k = 0; k < dims[2]; k++) {
+    const int r = owner_of(m, G, smp_add(o[2], smp_mul((float)k, h[2])));
+    if (r != prev) {
+      if (seen[(size_t)r]) { m->err = "isosurface: a slab owns two runs of lattice planes"; return 1; }      // z is monotone in k: unreachable
+      seen[(size_t)r] = true; ka[(size_t)r] = k;
+    }
+    kb[(size_t)r] = k + 1; prev = r;
+  }
+  std::vector<SurfSlabW> slabs((size_t)m->n);
+  for (int q = 0; q < m->n; q++)
+    slabs[(size_t)q] = SurfSlabW{q + 1 < m->n ? m->cut[(size_t)q + 1] : (i64)INT64_MAX, m->ctx[(size_t)q]->rbf_w, (long long)m->ctx[(size_t)q]->rbf_px};
+  for (int r = 0; r < m->n; r++) {
+    SurfLattice &L = m->ctx[(size_t)r]->surf_lat;
+    for (int d = 0; d < 3; d++) { L.o[d] = o[d]; L.h[d] = h[d]; L.dims[d] = dims[d]; }
+    L.iso = iso; L.ka = ka[(size_t)r]; L.kb = kb[(size_t)r]; L.slabs = slabs;
+  }
+  std::vector<i64> nv((size_t)m->n, 0), nt((size_t)m->n, 0);
+  if (run_all(m, [&](int r) { return r2s_surf_lattice_count(m->ctx[(size_t)r], &nv[(size_t)r], &nt[(size_t)r]); })) return 1;
+  // global bases in plane order (slab order unless the lattice runs downwards in z)
+  std::vector<int> order((size_t)m->n);
+  for (int r = 0; r < m->n; r++) order[(size_t)r] = r;
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return ka[(size_t)a] < ka[(size_t)b]; });
+  m->surf_vb.assign((size_t)m->n + 1, 0); m->surf_tb.assign((size_t)m->n + 1, 0);
+  i64 v = 0, t = 0;
+  for (int r : order) { m->surf_vb[(size_t)r] = v; m->surf_tb[(size_t)r] = t; v += nv[(size_t)r]; t += nt[(size_t)r]; }
+  m->surf_vb[(size_t)m->n] = v; m->surf_tb[(size_t)m->n] = t;
+  if (run_all(m, [&](int r) {
+        r2s_ctx *c = m->ctx[(size_t)r];
+        if (r2s_surf_lattice_emit(c, m->surf_vb[(size_t)r], v)) return 1;
+        c->surf_part = true;
+        return 0;
+      }))
+    return 1;
+  m->have_surface = true;
+  if (n_vertices) *n_vertices = v;
+  if (n_triangles) *n_triangles = t;
+  return 0;
+}
+
 int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format) {
   if (!m) return 1;
   if (!path) { m->err = "r2s_multi_export_isosurface: path is required"; return 1; }

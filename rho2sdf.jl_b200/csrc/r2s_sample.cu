@@ -159,6 +159,23 @@ int r2s_sample_lattice_planes(r2s_ctx *ctx, const float o[3], const float h[3], 
   return 0;
 }
 
+// the whole lattice planes [ka, kb) into the device array out_dev (x fastest, plane ka first), with the weights G carries (the streamed
+// lattice surface passes another slab's weights for the planes that slab owns); the same kernel, so the same bits as the calls above
+int r2s_sample_lattice_dev(r2s_ctx *ctx, const SampleGrid &G, const float o[3], const float h[3], const int64_t dims[3], i64 ka, i64 kb, float *out_dev) {
+  CK(cudaSetDevice(ctx->device));
+  LatBox B;
+  for (int d = 0; d < 3; d++) { B.o[d] = o[d]; B.h[d] = h[d]; }
+  B.i0 = 0; B.j0 = 0; B.bx = (int)dims[0]; B.by = (int)dims[1];
+  B.tx = cdiv(B.bx, SL_X); B.ty = cdiv(B.by, SL_Y);
+  const i64 per = (i64)B.tx * B.ty, mz = SL_Z * std::max<i64>(1, ((1ll << 31) - 1) / per / 2);      // planes per launch: grid.x < 2^31
+  for (i64 k = ka; k < kb; k += mz) {
+    B.k0 = (int)k; B.bz = (int)std::min(mz, kb - k);
+    k_sample_lattice<<<(unsigned)(per * cdiv(B.bz, SL_Z)), SL_X * SL_Y * SL_Z, 0, ctx->stream>>>(G, B, out_dev + (k - ka) * dims[0] * dims[1]);
+    LAUNCH_CHECK();
+  }
+  return 0;
+}
+
 // this context's weight planes [k0, k1) into the whole-grid array w (unpitched, x fastest)
 int r2s_sample_download_weights(r2s_ctx *ctx, float *w, float *th, i64 k0, i64 k1) {
   SampleGrid G;

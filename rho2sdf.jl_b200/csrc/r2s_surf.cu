@@ -26,6 +26,8 @@
 #include <vector>
 #include "r2s_common.cuh"
 #include "r2s_mc.cuh"
+#include "r2s_sample.cuh"
+#include "r2s_snap.cuh"
 
 __constant__ uint8_t c_mc[256][16];      // per case: triangle count, then 3 cube edges per triangle (mc_build_case)
 __constant__ uint8_t c_mc_edge[12];      // per cube edge: start corner | axis << 4
@@ -97,6 +99,9 @@ __device__ __forceinline__ unsigned warp_scan_u32(unsigned x, int lane) {
   return x;
 }
 
+// REC = false: vertex coordinates by mc_vertex.  REC = true (r2s_isosurface_lattice): each vertex slot of V receives its edge instead, as
+// three uint32 (i, j, (k - z0) << 2 | axis), which k_surf_snap reads and overwrites with the snapped vertex
+template <bool REC>
 __global__ void __launch_bounds__(32 * SURF_WARPS) k_surf_emit(SurfArgs a) {
   const int lane = threadIdx.x & 31, j = blockIdx.x * SURF_WARPS + (threadIdx.x >> 5), k = a.z0 + blockIdx.y;
   if (j >= a.ny) return;
@@ -143,7 +148,17 @@ __global__ void __launch_bounds__(32 * SURF_WARPS) k_surf_emit(SurfArgs a) {
     const unsigned inc = warp_scan_u32(cnt, lane), exc = inc - cnt, tot = __shfl_sync(0xffffffffu, inc, 31);
     const unsigned m4x = __shfl_down_sync(0xffffffffu, m4, 1);      // masks of point i + 1 (lane 29 reads lane 30: complete)
     // vertices of this row
-    if (own && (m4 & 7)) {
+    if (REC && own && (m4 & 7)) {
+      i64 id = base[0] + (exc & 255);
+#pragma unroll
+      for (int ax = 0; ax < 3; ax++) {
+        if (!(m4 >> ax & 1)) continue;
+        uint32_t *rec = (uint32_t *)(a.V + 3 * id);
+        rec[0] = (uint32_t)i; rec[1] = (uint32_t)j; rec[2] = (uint32_t)(k - a.z0) << 2 | (uint32_t)ax;
+        id++;
+      }
+    }
+    if (!REC && own && (m4 & 7)) {
       i64 id = base[0] + (exc & 255);
       const i64 p = ((i64)k * a.ny + j) * a.nx + i;
       const float va = a.f[p];
@@ -178,6 +193,41 @@ __global__ void __launch_bounds__(32 * SURF_WARPS) k_surf_emit(SurfArgs a) {
     for (int R = 0; R < 4; R++) base[R] += (tot >> (8 * R)) & 255;
     tb += ttot;
   }
+}
+
+// one thread per vertex of a lattice chunk: the edge record k_surf_emit<true> left in V -> the vertex on the continuous field's zero set
+// (r2s_snap.cuh).  f: the chunk's lattice values (globally indexed planes, as SurfArgs::f); every evaluation reads the weights of the slab
+// owning the point's floor plane (tab, nslab entries; nslab = 1: G's own weights)
+struct SnapArgs {
+  const float *f;
+  int nx, ny, z0, nslab;
+  float o[3], h[3], iso;
+  i64 n;
+  const SurfSlabW *tab;
+  float *V;
+};
+__global__ void __launch_bounds__(128) k_surf_snap(SampleGrid G, SnapArgs s) {
+  const i64 t = blockIdx.x * (i64)blockDim.x + threadIdx.x;
+  if (t >= s.n) return;
+  const uint32_t *rec = (const uint32_t *)(s.V + 3 * t);
+  const int i = (int)rec[0], j = (int)rec[1], k = s.z0 + (int)(rec[2] >> 2), ax = (int)(rec[2] & 3);
+  const float px = smp_add(s.o[0], smp_mul((float)i, s.h[0])), py = smp_add(s.o[1], smp_mul((float)j, s.h[1])), pz = smp_add(s.o[2], smp_mul((float)k, s.h[2]));
+  const i64 p = ((i64)k * s.ny + j) * s.nx + i;
+  const float va = s.f[p], vb = s.f[p + (ax == 0 ? 1 : ax == 1 ? (i64)s.nx : (i64)s.nx * s.ny)];
+  const int q = ax == 0 ? i : ax == 1 ? j : k;
+  const float xa = ax == 0 ? px : ax == 1 ? py : pz, xb = smp_add(s.o[ax], smp_mul((float)(q + 1), s.h[ax]));
+  const float x = snap_search([&](float v) {
+    const float qx = ax == 0 ? v : px, qy = ax == 1 ? v : py, qz = ax == 2 ? v : pz;
+    SampleGrid g = G;
+    if (s.nslab > 1) {
+      const int c = smp_floor(G.C[2], G.n[2], G.c0[2], G.inv[2], qz);
+      int r = 0;
+      while (r + 1 < s.nslab && c >= s.tab[r].k1) r++;
+      g.w = s.tab[r].w; g.px = s.tab[r].px;
+    }
+    return sample_point<false>(g, qx, qy, qz, nullptr);
+  }, xa, xb, va, vb, s.iso, nullptr);
+  s.V[3 * t] = ax == 0 ? x : px; s.V[3 * t + 1] = ax == 1 ? x : py; s.V[3 * t + 2] = ax == 2 ? x : pz;
 }
 
 __global__ void k_surf_totals(const i64 *vcnt, const i64 *tcnt, const i64 *vbase, const i64 *tbase, i64 nrows, i64 nown, const unsigned *bad, i64 *out) {
@@ -215,19 +265,12 @@ static SurfArgs surf_args(r2s_ctx *ctx, const float *f, i64 nx, i64 ny, i64 nz, 
   return a;
 }
 
-// pass 1 + scans: this context's vertex / triangle counts (owned planes [z0, z1) of an nx x ny x nz field)
-int r2s_surf_count(r2s_ctx *ctx, const float *f, i64 nx, i64 ny, i64 nz, i64 z0, i64 z1, const double origin[3], const double spacing[3], float iso,
-                   i64 *nv, i64 *nt) {
-  ctx->have_surface = false;
-  if (!isfinite(iso)) FAIL("isosurface: iso must be finite");
-  if (nx < 2 || ny < 2 || nz < 2) FAIL("isosurface: the field needs at least 2 points per axis");
-  if ((nx - 1) * (ny - 1) * (nz - 1) >= (1ll << 31)) FAIL("isosurface: 2^31 or more cells");
-  for (int d = 0; d < 3; d++) if (!isfinite(origin[d]) || !isfinite(spacing[d])) FAIL("isosurface: origin and spacing must be finite");
-  CK(cudaSetDevice(ctx->device));
-  if (upload_table(ctx)) return 1;
+// pass 1 + scans on the owned planes [z0, z1) of an nx x ny x nz field: per-row counts and bases in ctx->surf_rows, the owned totals
+static int count_rows(r2s_ctx *ctx, const float *f, i64 nx, i64 ny, i64 nz, i64 z0, i64 z1, float iso, i64 *nv, i64 *nt) {
   const i64 zc = std::min(z1 + 1, nz), nrows = (zc - z0) * ny;
   CK(ctx->surf_rows.reserve(sizeof(i64) * (size_t)(4 * nrows + 4)));
-  SurfArgs a = surf_args(ctx, f, nx, ny, nz, z0, z1, origin, spacing, iso);
+  const double zero[3] = {0, 0, 0};
+  SurfArgs a = surf_args(ctx, f, nx, ny, nz, z0, z1, zero, zero, iso);
   CK(cudaMemsetAsync(a.bad, 0, sizeof(unsigned), ctx->stream));
   k_surf_count<<<dim3(cdiv(ny, SURF_WARPS), (unsigned)(zc - z0)), 32 * SURF_WARPS, 0, ctx->stream>>>(a);
   LAUNCH_CHECK();
@@ -239,6 +282,22 @@ int r2s_surf_count(r2s_ctx *ctx, const float *f, i64 nx, i64 ny, i64 nz, i64 z0,
   i64 h[3];
   if (r2s_readback(ctx, h, tot, sizeof(h))) return 1;
   if (h[2]) FAIL("isosurface: the field holds a non-finite value");
+  *nv = h[0]; *nt = h[1];
+  return 0;
+}
+
+// pass 1 + scans: this context's vertex / triangle counts (owned planes [z0, z1) of an nx x ny x nz field)
+int r2s_surf_count(r2s_ctx *ctx, const float *f, i64 nx, i64 ny, i64 nz, i64 z0, i64 z1, const double origin[3], const double spacing[3], float iso,
+                   i64 *nv, i64 *nt) {
+  ctx->have_surface = false;
+  if (!isfinite(iso)) FAIL("isosurface: iso must be finite");
+  if (nx < 2 || ny < 2 || nz < 2) FAIL("isosurface: the field needs at least 2 points per axis");
+  if ((nx - 1) * (ny - 1) * (nz - 1) >= (1ll << 31)) FAIL("isosurface: 2^31 or more cells");
+  for (int d = 0; d < 3; d++) if (!isfinite(origin[d]) || !isfinite(spacing[d])) FAIL("isosurface: origin and spacing must be finite");
+  CK(cudaSetDevice(ctx->device));
+  if (upload_table(ctx)) return 1;
+  i64 h[2];
+  if (count_rows(ctx, f, nx, ny, nz, z0, z1, iso, &h[0], &h[1])) return 1;
   ctx->surf_f = f; ctx->surf_nx = nx; ctx->surf_ny = ny; ctx->surf_nz = nz; ctx->surf_z0 = z0; ctx->surf_z1 = z1; ctx->surf_iso = iso;
   for (int d = 0; d < 3; d++) { ctx->surf_origin[d] = origin[d]; ctx->surf_spacing[d] = spacing[d]; }
   ctx->surf_nv = h[0]; ctx->surf_nt = h[1];
@@ -256,11 +315,121 @@ int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total) {
   SurfArgs a = surf_args(ctx, ctx->surf_f, ctx->surf_nx, ctx->surf_ny, ctx->surf_nz, ctx->surf_z0, ctx->surf_z1, ctx->surf_origin, ctx->surf_spacing, ctx->surf_iso);
   a.vglob = vglob; a.V = ctx->surf_V.as<float>(); a.T = ctx->surf_T.as<int>();
   if (ctx->surf_z1 > ctx->surf_z0 && (nv > 0 || nt > 0)) {
-    k_surf_emit<<<dim3(cdiv(a.ny, SURF_WARPS), (unsigned)(ctx->surf_z1 - ctx->surf_z0)), 32 * SURF_WARPS, 0, ctx->stream>>>(a);
+    k_surf_emit<false><<<dim3(cdiv(a.ny, SURF_WARPS), (unsigned)(ctx->surf_z1 - ctx->surf_z0)), 32 * SURF_WARPS, 0, ctx->stream>>>(a);
     LAUNCH_CHECK();
   }
   CK(cudaStreamSynchronize(ctx->stream));
   ctx->surf_vglob = vglob; ctx->have_surface = true;
+  return 0;
+}
+
+// ---- the surface of the continuous field on a lattice (r2s_isosurface_lattice) -------------------------------------------------------
+// Lattice planes stream through ctx->surf_buf, `planes` owned planes per chunk plus the two planes above them that the count and emit
+// kernels read; the field is never held whole.  Sweep 1 samples and counts every chunk (chunk totals); after the host scan of the totals
+// (over the slabs too) sweep 2 samples again, counts again for the row bases, emits with the chunk's global bases and snaps the chunk's
+// vertices.  The kernels of a chunk see its buffer through the plane-indexed SurfArgs::f, shifted by the chunk's first plane.  The two
+// planes above a chunk are the next chunk's first two: they move to the front of the buffer instead of being sampled again.
+#define SURF_LAT_BUDGET (1ll << 30)      // bytes of lattice values per chunk when R2S_SURF_PLANES is not set
+
+int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3]) {
+  if (!isfinite(iso)) FAIL("isosurface: iso must be finite");
+  if (r2s_sample_lattice_check(ctx, origin, spacing, dims, o, h)) return 1;
+  if (dims[0] < 2 || dims[1] < 2 || dims[2] < 2) FAIL("isosurface: the field needs at least 2 points per axis");
+  if ((dims[0] - 1) * (dims[1] - 1) * (dims[2] - 1) >= (1ll << 31)) FAIL("isosurface: 2^31 or more cells");
+  SampleGrid G;
+  return r2s_sample_grid(ctx, &G, false);
+}
+
+static int lattice_sweep(r2s_ctx *ctx, bool emit, i64 vglob) {
+  SurfLattice &L = ctx->surf_lat;
+  CK(cudaSetDevice(ctx->device));
+  SampleGrid G, Gh;
+  if (r2s_sample_grid(ctx, &G, true) || r2s_sample_grid(ctx, &Gh, false)) return 1;
+  const i64 nx = L.dims[0], ny = L.dims[1], nz = L.dims[2], pl = nx * ny, P = L.planes;
+  CK(ctx->surf_buf.reserve(sizeof(float) * (size_t)((P + 2) * pl)));
+  float *buf = ctx->surf_buf.as<float>();
+  const int nslab = (int)L.slabs.size();
+  CK(ctx->surf_wtab.reserve(sizeof(SurfSlabW) * (size_t)nslab));
+  CK(cudaMemcpyAsync(ctx->surf_wtab.p, L.slabs.data(), sizeof(SurfSlabW) * (size_t)nslab, cudaMemcpyHostToDevice, ctx->stream));
+  // the slab whose weights serve lattice plane k: the owner of the plane's floor plane (all planes of [ka, kb) are this context's)
+  auto slab_of = [&](i64 k) {
+    const int c = smp_floor(Gh.C[2], Gh.n[2], Gh.c0[2], Gh.inv[2], smp_add(L.o[2], smp_mul((float)k, L.h[2])));
+    int r = 0;
+    while (r + 1 < nslab && c >= L.slabs[(size_t)r].k1) r++;
+    return r;
+  };
+  if (!emit) { L.cnv.clear(); L.cnt.clear(); }
+  i64 have = L.ka, vb = 0, tb = 0;
+  for (i64 c0 = L.ka, ci = 0; c0 < L.kb; c0 += P, ci++) {
+    const i64 c1 = std::min(c0 + P, L.kb), need = std::min(c1 + 2, nz);
+    // planes [c0, have) are the previous chunk's top planes, at buffer positions P + (k - c0): one plane per copy (no overlap for P = 1)
+    for (i64 k = c0; k < have; k++)
+      CK(cudaMemcpyAsync(buf + (k - c0) * pl, buf + (P + k - c0) * pl, sizeof(float) * (size_t)pl, cudaMemcpyDeviceToDevice, ctx->stream));
+    for (i64 k = std::max(have, c0); k < need;) {      // runs of planes read with the same slab's weights
+      const int r = slab_of(k);
+      i64 e = k + 1;
+      while (e < need && slab_of(e) == r) e++;
+      SampleGrid Gr = G;
+      Gr.w = L.slabs[(size_t)r].w; Gr.px = L.slabs[(size_t)r].px;
+      if (r2s_sample_lattice_dev(ctx, Gr, L.o, L.h, L.dims, k, e, buf + (k - c0) * pl)) return 1;
+      k = e;
+    }
+    have = need;
+    const float *f = buf - c0 * pl;      // plane k of the chunk at f + k * pl (only planes [c0, need) are read)
+    i64 cv, ct;
+    if (count_rows(ctx, f, nx, ny, nz, c0, c1, L.iso, &cv, &ct)) return 1;
+    if (!emit) { L.cnv.push_back(cv); L.cnt.push_back(ct); }
+    else {
+      if (cv != L.cnv[(size_t)ci] || ct != L.cnt[(size_t)ci]) FAIL("isosurface: the lattice counts changed between the two sweeps");
+      const double zero[3] = {0, 0, 0};
+      SurfArgs a = surf_args(ctx, f, nx, ny, nz, c0, c1, zero, zero, L.iso);
+      a.vglob = vglob + vb; a.V = ctx->surf_V.as<float>() + 3 * vb; a.T = ctx->surf_T.as<int>() + 3 * tb;
+      if (cv > 0 || ct > 0) {
+        k_surf_emit<true><<<dim3(cdiv(ny, SURF_WARPS), (unsigned)(c1 - c0)), 32 * SURF_WARPS, 0, ctx->stream>>>(a);
+        LAUNCH_CHECK();
+      }
+      if (cv > 0) {
+        SnapArgs s;
+        s.f = f; s.nx = (int)nx; s.ny = (int)ny; s.z0 = (int)c0; s.nslab = nslab; s.iso = L.iso; s.n = cv; s.tab = ctx->surf_wtab.as<SurfSlabW>(); s.V = a.V;
+        for (int d = 0; d < 3; d++) { s.o[d] = L.o[d]; s.h[d] = L.h[d]; }
+        k_surf_snap<<<cdiv(cv, 128), 128, 0, ctx->stream>>>(G, s);
+        LAUNCH_CHECK();
+      }
+    }
+    vb += cv; tb += ct;
+  }
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (!emit) { ctx->surf_nv = vb; ctx->surf_nt = tb; }
+  return 0;
+}
+
+// sweep 1 over ctx->surf_lat (set by the caller): this context's vertex and triangle counts
+int r2s_surf_lattice_count(r2s_ctx *ctx, i64 *nv, i64 *nt) {
+  ctx->have_surface = false;
+  SurfLattice &L = ctx->surf_lat;
+  const i64 pl = L.dims[0] * L.dims[1];
+  L.planes = ctx->knobs.surf_planes > 0 ? (i64)ctx->knobs.surf_planes : std::max<i64>(1, SURF_LAT_BUDGET / (i64)sizeof(float) / pl - 2);
+  L.planes = std::max<i64>(1, std::min(L.planes, L.kb - L.ka));
+  CK(cudaSetDevice(ctx->device));
+  if (upload_table(ctx)) return 1;
+  ctx->surf_nv = ctx->surf_nt = 0;
+  if (L.kb > L.ka && lattice_sweep(ctx, false, 0)) { ctx->surf_buf.release(); return 1; }
+  *nv = ctx->surf_nv; *nt = ctx->surf_nt;
+  return 0;
+}
+
+// sweep 2: the mesh part of this context, its vertices from global id vglob on (nv_total vertices in the whole mesh)
+int r2s_surf_lattice_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total) {
+  CK(cudaSetDevice(ctx->device));
+  if (nv_total >= (1ll << 31)) { ctx->surf_buf.release(); FAIL("isosurface: 2^31 or more vertices (vertex ids are int32)"); }
+  const i64 nv = ctx->surf_nv, nt = ctx->surf_nt;
+  CK(ctx->surf_V.reserve(sizeof(float) * 3 * (size_t)std::max<i64>(nv, 1)));
+  CK(ctx->surf_T.reserve(sizeof(int) * 3 * (size_t)std::max<i64>(nt, 1)));
+  const SurfLattice &L = ctx->surf_lat;
+  const int rc = L.kb > L.ka && (nv > 0 || nt > 0) ? lattice_sweep(ctx, true, vglob) : 0;
+  ctx->surf_buf.release();
+  if (rc) return 1;
+  ctx->surf_f = nullptr; ctx->surf_vglob = vglob; ctx->have_surface = true;
   return 0;
 }
 
@@ -406,6 +575,26 @@ int r2s_isosurface_from_sdf(r2s_ctx *ctx, const float *sdf, int64_t nx, int64_t 
   tmp.release();
   ctx->surf_f = nullptr;
   if (rc) { ctx->have_surface = false; return 1; }
+  ctx->surf_nv_all = nv; ctx->surf_nt_all = nt; ctx->surf_part = false;
+  if (n_vertices) *n_vertices = nv;
+  if (n_triangles) *n_triangles = nt;
+  return 0;
+}
+
+int r2s_isosurface_lattice(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                           int64_t *n_triangles) {
+  if (!ctx) return 1;
+  ctx->have_surface = false;
+  if (ctx->nranks > 1)
+    FAIL(ctx->lg ? "r2s_isosurface_lattice: this context is one slab of an r2s_multi group; use r2s_multi_isosurface_lattice"
+                 : "r2s_isosurface_lattice: not available on a slab rank of the NCCL communicator (one process per GPU); extract on one context or with r2s_multi");
+  SurfLattice &L = ctx->surf_lat;
+  if (r2s_surf_lattice_check(ctx, origin, spacing, dims, iso, L.o, L.h)) return 1;
+  for (int d = 0; d < 3; d++) L.dims[d] = dims[d];
+  L.iso = iso; L.ka = 0; L.kb = dims[2];
+  L.slabs.assign(1, SurfSlabW{INT64_MAX, ctx->rbf_w, (long long)ctx->rbf_px});
+  i64 nv, nt;
+  if (r2s_surf_lattice_count(ctx, &nv, &nt) || r2s_surf_lattice_emit(ctx, 0, nv)) return 1;
   ctx->surf_nv_all = nv; ctx->surf_nt_all = nt; ctx->surf_part = false;
   if (n_vertices) *n_vertices = nv;
   if (n_triangles) *n_triangles = nt;

@@ -11,7 +11,7 @@ using Rho2sdf.MeshGrid: Mesh, Grid, generateGridPoints
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
-       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, sample_sdf, sample_sdf_lattice, rbf_weights
+       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, isosurface_lattice, sample_sdf, sample_sdf_lattice, rbf_weights
 
 const LIB = get(ENV, "R2S_LIBRARY", joinpath(@__DIR__, "..", "libr2s.so"))
 
@@ -232,6 +232,23 @@ function sample_sdf_lattice(mesh::Mesh, origin::AbstractVector{<:Real}, spacing:
   check(c, ccall((:r2s_sample_sdf_lattice, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Ptr{Cfloat}),
                  c.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], out))
   return out
+end
+"""surface {f = iso} of the continuous field on the lattice origin + (i - 1) .* spacing, i = 1 .. dims, streamed through the device (the
+triangles of isosurface(sample_sdf_lattice(...)), each vertex on its lattice edge where a bracketing search puts it closest to the zero set:
+include/r2s.h); a MultiContext extracts on all its slabs"""
+function isosurface_lattice(mesh::Mesh, origin::AbstractVector{<:Real}, spacing::AbstractVector{<:Real}, dims::NTuple{3,Int}; iso::Float32=0f0)
+  c = context(mesh); nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+  check(c, ccall((:r2s_isosurface_lattice, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Cfloat, Ref{Int64}, Ref{Int64}),
+                 c.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], iso, nv, nt))
+  return download_surface(c, nv[], nt[])
+end
+function isosurface_lattice(m::MultiContext, origin::AbstractVector{<:Real}, spacing::AbstractVector{<:Real}, dims::NTuple{3,Int}; iso::Float32=0f0)
+  nv = Ref{Int64}(0); nt = Ref{Int64}(0)
+  mcheck(m, ccall((:r2s_multi_isosurface_lattice, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Cfloat, Ref{Int64}, Ref{Int64}),
+                  m.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], iso, nv, nt))
+  V = Matrix{Float32}(undef, 3, nv[]); T = Matrix{Int32}(undef, 3, nt[])
+  mcheck(m, ccall((:r2s_multi_download_isosurface, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Int32}), m.h, V, T))
+  return V, T .+ Int32(1)
 end
 "(weights on the coarse grid of `grid`, th): the definition of the continuous field"
 function rbf_weights(mesh::Mesh, grid)

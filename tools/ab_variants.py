@@ -12,7 +12,7 @@ sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np
 
 DEFAULT = "default:;no_prune:R2S_PROJ_PRUNE=0;general_proj:R2S_PROJ_BOX=0;sign_lists:R2S_SIGN_LATTICE=0"
-KNOBS = ("R2S_PROJ_BOX", "R2S_PROJ_PRUNE", "R2S_SIGN_LATTICE", "R2S_P2P")
+KNOBS = ("R2S_PROJ_BOX", "R2S_PROJ_PRUNE", "R2S_SIGN_LATTICE", "R2S_P2P", "R2S_SURF_PLANES")      # cleared before every variant (R2S_SURF_PLANES: no effect on the pipeline)
 
 
 def main():
