@@ -294,6 +294,28 @@ int r2s_isosurface_lattice(r2s_ctx *ctx, const double origin[3], const double sp
 int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
                                  int64_t *n_vertices, int64_t *n_triangles);
 
+/* The same surface on lattices of any cell count, sampling only the lattice blocks that can hold it (csrc/r2s_band.cuh, r2s_surf.cu).
+ *   same mesh: lattice values, vertex numbering, triangle order, orientation and the vertex search are those of r2s_isosurface_lattice,
+ *     word for word: on every lattice that call accepts, the two meshes are bit for bit equal.
+ *   limits: up to 2^31 - 1 points per axis and any cell count below 2^63; fewer than 2^31 vertices (triangles hold int32 ids).
+ *   skipping: the lattice is cut into blocks of 8 x 8 x 8 cells (the closed box of their 9^3 points).  A block is skipped -- never
+ *     sampled -- when every coarse weight that a tap of any of its points can reach has one sign and that sign puts every Float32 value
+ *     of the box on one side of iso: weights >= 0 and th >= iso, or weights >= 0 and a rigorous lower bound of the sum reaching iso - th
+ *     (mirror: weights <= 0, values < iso).  The bounds cover every Float32 rounding of the sampler (r2s_band.cuh states them), so a
+ *     skipped cell has no crossing; every crossing edge lies in a sampled block, and every value marching cubes or the vertex search reads
+ *     there is the sampler's.  A NaN weight, or a block whose points read two slabs' weights, is always sampled.  The mesh depends on
+ *     neither the block size nor the chunk size.
+ *   memory: planes stream through the chunk buffer of r2s_isosurface_lattice (R2S_SURF_PLANES); per chunk one byte and one int64 per block.
+ *   n_sampled (NULL or): the lattice points evaluated by one of the two sweeps -- each point at most once; the share of the lattice skipped
+ *     is 1 - n_sampled / (dims[0] dims[1] dims[2]).
+ * Rejected with an error: no smoothed field, a non-finite origin, spacing, lattice coordinate or iso, dims < 2 or >= 2^31 on an axis, 2^31
+ * or more vertices; the single-context call fails on a slab rank of the NCCL communicator (use r2s_multi).  The weights, th and fine_sdf
+ * are untouched; the mesh replaces the context's (handle's) surface, for the download and export calls above. */
+int r2s_isosurface_band(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
+                        int64_t *n_vertices, int64_t *n_triangles, int64_t *n_sampled);
+int r2s_multi_isosurface_band(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
+                              int64_t *n_vertices, int64_t *n_triangles, int64_t *n_sampled);
+
 /* ---- measurement helper (bench.py): FMA-pipe peak of the device in TFLOP/s, fp64 != 0 -> double, else float -------- */
 int r2s_measure_fma_peak(r2s_ctx *ctx, int fp64, double *tflops);
 

@@ -9,7 +9,7 @@ image, so this module carries the same names, argument meaning and error behavio
     find_threshold_for_volume, calculate_isocontour_volume                  (src/MeshGrid/*)
     evalDistances, Sign_Detection, remove_sdf_artifacts                     (src/SignedDistances/*)
     RBFs_smoothing, calculate_volume_from_sdf                               (src/SdfSmoothing/*)
-    isosurface, isosurface_from_sdf, isosurface_lattice, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}, or of the continuous field on any lattice; the reference leaves it to
+    isosurface, isosurface_from_sdf, isosurface_lattice, isosurface_band, export_isosurface, read_stl, read_ply  (the surface {fine_sdf = iso}, or of the continuous field on any lattice; the reference leaves it to
                                                                              src/Visualizations / ParaView)
     sample_sdf, sample_sdf_lattice, rbf_weights                             (the smoothed SDF as a continuous function:
                                                                              rbf_interpolation_kdtree, RBFs4Smoothing.jl:219-248)
@@ -29,7 +29,7 @@ __all__ = ["HEX8", "TET4", "Rho2sdfOptions", "Mesh", "Grid", "getMesh_AABB", "ge
            "DenseInNodes", "find_threshold_for_volume", "calculate_isocontour_volume", "evalDistances", "Sign_Detection",
            "remove_sdf_artifacts", "RBFs_smoothing", "calculate_volume_from_sdf", "rho2sdf", "rho2sdf_hex8", "rho2sdf_tet4",
            "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti",
-           "isosurface", "isosurface_from_sdf", "isosurface_lattice", "export_isosurface", "read_stl", "read_ply",
+           "isosurface", "isosurface_from_sdf", "isosurface_lattice", "isosurface_band", "export_isosurface", "read_stl", "read_ply",
            "sample_sdf", "sample_sdf_lattice", "rbf_weights", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -146,6 +146,8 @@ def load_library():
     L.r2s_multi_export_isosurface.argtypes = [vp, C.c_char_p, C.c_int]
     L.r2s_isosurface_lattice.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip]
     L.r2s_multi_isosurface_lattice.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip]
+    L.r2s_isosurface_band.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip, ip]
+    L.r2s_multi_isosurface_band.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip, ip]
     for pre in ("r2s_", "r2s_multi_"):
         getattr(L, pre + "sample_sdf").argtypes = [vp, vp, C.c_int64, vp, vp]
         getattr(L, pre + "sample_sdf_lattice").argtypes = [vp, vp, vp, vp, vp]
@@ -661,20 +663,26 @@ def _lattice_args(origin, spacing, shape):
     return o, h, dims
 
 
-def _extract(mesh, iso, lattice=None):
+def _extract(mesh, iso, lattice=None, band=None):
     nv, nt = C.c_int64(), C.c_int64()
+    if band is not None:
+        o, h, dims = _lattice_args(*band)
+        obj, pre = _sampler(mesh)
+        ns = C.c_int64()
+        obj.check(getattr(obj.lib, pre + "isosurface_band")(obj.h, _ptr(o), _ptr(h), _ptr(dims), float(iso), C.byref(nv), C.byref(nt), C.byref(ns)))
+        return obj, getattr(obj.lib, pre + "download_isosurface"), nv.value, nt.value, ns.value
     if lattice is not None:
         o, h, dims = _lattice_args(*lattice)
         obj, pre = _sampler(mesh)
         obj.check(getattr(obj.lib, pre + "isosurface_lattice")(obj.h, _ptr(o), _ptr(h), _ptr(dims), float(iso), C.byref(nv), C.byref(nt)))
-        return obj, getattr(obj.lib, pre + "download_isosurface"), nv.value, nt.value
+        return obj, getattr(obj.lib, pre + "download_isosurface"), nv.value, nt.value, None
     if mesh.multi is not None:
         m = mesh.multi
         m.check(m.lib.r2s_multi_isosurface(m.h, float(iso), C.byref(nv), C.byref(nt)))
-        return m, m.lib.r2s_multi_download_isosurface, nv.value, nt.value
+        return m, m.lib.r2s_multi_download_isosurface, nv.value, nt.value, None
     c = mesh.ctx
     c.check(c.lib.r2s_isosurface(c.h, float(iso), C.byref(nv), C.byref(nt)))
-    return c, c.lib.r2s_download_isosurface, nv.value, nt.value
+    return c, c.lib.r2s_download_isosurface, nv.value, nt.value, None
 
 
 def isosurface(mesh, iso=0.0):
@@ -682,7 +690,7 @@ def isosurface(mesh, iso=0.0):
     or all slabs of a multi-GPU mesh).  Returns (V (nv, 3) float32, T (nt, 3) int32, 0-based): one vertex per grid edge that crosses
     iso (a point is inside iff value >= iso), triangles counter-clockwise seen from outside, in the frame of export_device_result_to_vti
     (origin AABB_min, spacing cell_size / smooth).  The mesh is closed wherever the field is below iso on the grid's border."""
-    obj, dl, nv, nt = _extract(mesh, iso)
+    obj, dl, nv, nt, _ = _extract(mesh, iso)
     return _download_surface(obj, dl, nv, nt)
 
 
@@ -706,15 +714,27 @@ def isosurface_lattice(mesh, origin, spacing, shape, iso=0.0):
     the lattice field anywhere.  The triangles are those of isosurface_from_sdf(sample_sdf_lattice(mesh, origin, spacing, shape), origin,
     spacing, iso); each vertex lies on its lattice edge at the Float32 coordinate that a bracketing search on f finds closest to the zero
     set (include/r2s.h states the rule).  Returns (V (nv, 3) float32, T (nt, 3) int32, 0-based)."""
-    obj, dl, nv, nt = _extract(mesh, iso, (origin, spacing, shape))
+    obj, dl, nv, nt, _ = _extract(mesh, iso, (origin, spacing, shape))
     return _download_surface(obj, dl, nv, nt)
 
 
-def export_isosurface(mesh, path, iso=0.0, lattice=None):
+def isosurface_band(mesh, origin, spacing, shape, iso=0.0, stats=False):
+    """The mesh of isosurface_lattice, bit for bit, sampling only the lattice blocks that can hold the surface: a block whose reachable
+    coarse weights share one sign that provably keeps every value of the block on one side of iso is never evaluated.  Any cell count
+    (fewer than 2^31 vertices).  Returns (V, T); with stats=True (V, T, n_sampled), n_sampled the lattice points evaluated per sweep."""
+    obj, dl, nv, nt, ns = _extract(mesh, iso, band=(origin, spacing, shape))
+    V, T = _download_surface(obj, dl, nv, nt)
+    return (V, T, ns) if stats else (V, T)
+
+
+def export_isosurface(mesh, path, iso=0.0, lattice=None, band=None):
     """Extract {fine_sdf = iso} on the device(s) of `mesh` and write it to `path`: binary STL (.stl) or binary little-endian PLY (.ply).
-    lattice=(origin, spacing, shape): extract the continuous field's surface on that lattice instead, as isosurface_lattice does."""
+    lattice=(origin, spacing, shape): extract the continuous field's surface on that lattice instead, as isosurface_lattice does;
+    band=(origin, spacing, shape): the same mesh through isosurface_band (any cell count)."""
     fmt = _surface_format(path)
-    obj, _, _, _ = _extract(mesh, iso, lattice)
+    if lattice is not None and band is not None:
+        raise R2SError("export_isosurface: give lattice= or band=, not both")
+    obj, _, _, _, _ = _extract(mesh, iso, lattice, band)
     if mesh.multi is not None:
         obj.check(obj.lib.r2s_multi_export_isosurface(obj.h, str(path).encode(), fmt))
     else:

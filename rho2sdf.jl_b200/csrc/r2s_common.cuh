@@ -80,6 +80,8 @@ struct SurfLattice {
   float o[3], h[3]; int64_t dims[3]; float iso; i64 ka, kb, planes;
   std::vector<SurfSlabW> slabs;
   std::vector<i64> cnv, cnt;
+  bool band = false;      // r2s_isosurface_band: sample only the blocks that can hold the surface; nsampled = points evaluated by sweep 1
+  i64 nsampled = 0;
 };
 
 struct LocalGroup;      // in-process slab group (r2s_multi_*): r2s_comm.cu
@@ -158,7 +160,7 @@ struct r2s_ctx {
   double surf_origin[3] = {0, 0, 0}, surf_spacing[3] = {0, 0, 0};
   i64 surf_nv = 0, surf_nt = 0, surf_vglob = 0, surf_nv_all = 0, surf_nt_all = 0;
   // r2s_isosurface_lattice: the chunk of sampled lattice planes, the device copy of surf_lat.slabs
-  DevBuf surf_buf, surf_wtab;
+  DevBuf surf_buf, surf_wtab, surf_band;      // surf_band: block classes, the sampled block list and counters of one chunk (r2s_isosurface_band)
   SurfLattice surf_lat;
 };
 
@@ -241,7 +243,8 @@ int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);                  // pa
 int r2s_surf_download_slab(r2s_ctx *ctx, float *V, int32_t *T, i64 tglob, bool staging);   // this slab's part into the whole arrays
 int r2s_surf_write_file(const char *path, int format, const float *V, i64 nv, const int *T, i64 nt, std::string *err);
 // the surface of the continuous field on a lattice (r2s_isosurface_lattice): checks, then two sweeps over ctx->surf_lat's planes
-int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3]);
+int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3],
+                           bool band = false);      // band: any cell count (r2s_isosurface_band)
 int r2s_surf_lattice_count(r2s_ctx *ctx, i64 *nv, i64 *nt);                // sweep 1: chunk counts, this context's totals
 int r2s_surf_lattice_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total);          // sweep 2: emit + snap with this context's first global vertex id
 // r2s_sample.cu: the sampler of the continuous field, for r2s_rbf.cu (record) and r2s_multi.cu (one slab's share, no rank check)

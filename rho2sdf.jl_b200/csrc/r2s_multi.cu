@@ -302,14 +302,18 @@ int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th) {
 // -- with the weights of the slab owning the point's floor plane, through peer memory (plain pointers on a shared device).  The weights
 // are settled when the call starts and nothing writes them during it, so no exchange is ordered.  The host scans the slab counts in plane
 // order, as r2s_multi_isosurface does in slab order.
-int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
-                                 int64_t *n_triangles) {
+// band: r2s_multi_isosurface_band (blocks whose points read two slabs' weights are always sampled, r2s_surf.cu)
+static int multi_lattice_surface(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                                 int64_t *n_triangles, bool band, int64_t *n_sampled) {
   if (!m) return 1;
   if (!m->has_grid) { m->err = "r2s_multi_set_grid has not been called"; return 1; }
   m->have_surface = false;
   if (m->n == 1) {
     int64_t a = 0, b = 0;
-    if (r2s_isosurface_lattice(m->ctx[0], origin, spacing, dims, iso, &a, &b)) { m->err = m->ctx[0]->err; return 1; }
+    if (band ? r2s_isosurface_band(m->ctx[0], origin, spacing, dims, iso, &a, &b, n_sampled) : r2s_isosurface_lattice(m->ctx[0], origin, spacing, dims, iso, &a, &b)) {
+      m->err = m->ctx[0]->err;
+      return 1;
+    }
     m->surf_vb.assign({0, a}); m->surf_tb.assign({0, b});
     m->have_surface = true;
     if (n_vertices) *n_vertices = a;
@@ -320,7 +324,7 @@ int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const dou
   float o[3], h[3];
   SampleGrid G;
   if (multi_sample_ready(m, &G)) return 1;
-  if (r2s_surf_lattice_check(m->ctx[0], origin, spacing, dims, iso, o, h)) { m->err = m->ctx[0]->err; return 1; }
+  if (r2s_surf_lattice_check(m->ctx[0], origin, spacing, dims, iso, o, h, band)) { m->err = m->ctx[0]->err; return 1; }
   std::vector<i64> ka((size_t)m->n, 0), kb((size_t)m->n, 0);
   std::vector<bool> seen((size_t)m->n, false);
   int prev = -1;
@@ -338,10 +342,11 @@ int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const dou
   for (int r = 0; r < m->n; r++) {
     SurfLattice &L = m->ctx[(size_t)r]->surf_lat;
     for (int d = 0; d < 3; d++) { L.o[d] = o[d]; L.h[d] = h[d]; L.dims[d] = dims[d]; }
-    L.iso = iso; L.ka = ka[(size_t)r]; L.kb = kb[(size_t)r]; L.slabs = slabs;
+    L.iso = iso; L.ka = ka[(size_t)r]; L.kb = kb[(size_t)r]; L.slabs = slabs; L.band = band; L.nsampled = 0;
   }
+  auto release = [&]() { for (int r = 0; r < m->n; r++) { cudaSetDevice(m->ctx[(size_t)r]->device); m->ctx[(size_t)r]->surf_band.release(); } };
   std::vector<i64> nv((size_t)m->n, 0), nt((size_t)m->n, 0);
-  if (run_all(m, [&](int r) { return r2s_surf_lattice_count(m->ctx[(size_t)r], &nv[(size_t)r], &nt[(size_t)r]); })) return 1;
+  if (run_all(m, [&](int r) { return r2s_surf_lattice_count(m->ctx[(size_t)r], &nv[(size_t)r], &nt[(size_t)r]); })) { release(); return 1; }
   // global bases in plane order (slab order unless the lattice runs downwards in z)
   std::vector<int> order((size_t)m->n);
   for (int r = 0; r < m->n; r++) order[(size_t)r] = r;
@@ -355,12 +360,27 @@ int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const dou
         if (r2s_surf_lattice_emit(c, m->surf_vb[(size_t)r], v)) return 1;
         c->surf_part = true;
         return 0;
-      }))
+      })) {
+    release();
     return 1;
+  }
+  release();
   m->have_surface = true;
   if (n_vertices) *n_vertices = v;
   if (n_triangles) *n_triangles = t;
+  if (n_sampled) {
+    *n_sampled = 0;
+    for (int r = 0; r < m->n; r++) *n_sampled += m->ctx[(size_t)r]->surf_lat.nsampled;
+  }
   return 0;
+}
+int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                                 int64_t *n_triangles) {
+  return multi_lattice_surface(m, origin, spacing, dims, iso, n_vertices, n_triangles, false, nullptr);
+}
+int r2s_multi_isosurface_band(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                              int64_t *n_triangles, int64_t *n_sampled) {
+  return multi_lattice_surface(m, origin, spacing, dims, iso, n_vertices, n_triangles, true, n_sampled);
 }
 
 int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format) {

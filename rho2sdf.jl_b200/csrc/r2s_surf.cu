@@ -28,6 +28,7 @@
 #include "r2s_mc.cuh"
 #include "r2s_sample.cuh"
 #include "r2s_snap.cuh"
+#include "r2s_band.cuh"
 
 __constant__ uint8_t c_mc[256][16];      // per case: triangle count, then 3 cube edges per triangle (mc_build_case)
 __constant__ uint8_t c_mc_edge[12];      // per cube edge: start corner | axis << 4
@@ -230,6 +231,97 @@ __global__ void __launch_bounds__(128) k_surf_snap(SampleGrid G, SnapArgs s) {
   s.V[3 * t] = ax == 0 ? x : px; s.V[3 * t + 1] = ax == 1 ? x : py; s.V[3 * t + 2] = ax == 2 ? x : pz;
 }
 
+// ---- r2s_isosurface_band: sample only the lattice blocks that can hold the surface (r2s_band.cuh) -------------------------------------
+// Block (bx, by, bz) covers the lattice cells [b B, min(b B + B, dims - 1)) per axis and classifies the closed box of their points.  A point
+// belongs to the closed boxes of at most two blocks per axis: its owner min(i / B, nb - 1), and owner - 1 when i is a multiple of B inside
+// the lattice.  The chunk's points whose owner is skipped receive a fill value on the proven side (iso, or the float below iso); then every
+// point that some sampled block holds is evaluated once, by the last sampled block (in (bz, by, bx) order) holding it, with the sampler's
+// arithmetic.  A value marching cubes or the snap reads is therefore exact wherever it matters: every crossing edge lies in the closed box
+// of its lower point's owner, which is sampled, and a fill value sits on its point's true side.
+struct BandArgs {
+  float o[3], h[3], iso, below;          // below: the float below iso (the fill of an outside block)
+  i64 n[3], nb[3];                       // lattice points and blocks per axis
+  i64 ka, kb, lz0, nblk;                 // chunk planes [ka, kb) written to out (plane ka first); block layers from lz0 on, nblk blocks
+  i64 kown;                              // planes below kown are this context's: only their evaluations are counted
+  int nslab;
+  const SurfSlabW *tab;
+  uint8_t *cls;                          // per block of the chunk's layers: 0 sampled, 1 inside, 2 outside
+  i64 *list, *cnt;                       // the sampled blocks; cnt[0] = their number, cnt[1] += points evaluated
+  float *out;
+};
+
+__device__ __forceinline__ int band_slab(const SampleGrid &G, const BandArgs &A, float z) {
+  const int c = smp_floor(G.C[2], G.n[2], G.c0[2], G.inv[2], z);
+  int r = 0;
+  while (r + 1 < A.nslab && c >= A.tab[r].k1) r++;
+  return r;
+}
+
+// one thread per block of the chunk's layers: classify, and list the sampled ones (in any order: the values do not depend on it)
+__global__ void __launch_bounds__(128) k_band_classify(SampleGrid G, BandArgs A) {
+  const i64 t = blockIdx.x * (i64)blockDim.x + threadIdx.x;
+  if (t >= A.nblk) return;
+  const i64 b[3] = {t % A.nb[0], (t / A.nb[0]) % A.nb[1], A.lz0 + t / (A.nb[0] * A.nb[1])};
+  i64 lo[3], hi[3];
+  for (int d = 0; d < 3; d++) { lo[d] = b[d] * R2S_BAND_B; hi[d] = lo[d] + R2S_BAND_B < A.n[d] - 1 ? lo[d] + R2S_BAND_B : A.n[d] - 1; }
+  // a block whose points read two slabs' weights is sampled; otherwise every evaluation in it reads slab r's
+  const int r = band_slab(G, A, smp_add(A.o[2], smp_mul((float)lo[2], A.h[2])));
+  int c = 0;
+  if (r == band_slab(G, A, smp_add(A.o[2], smp_mul((float)hi[2], A.h[2])))) {
+    G.w = A.tab[r].w; G.px = A.tab[r].px;
+    c = band_classify(G, A.o, A.h, lo, hi, A.iso, band_margin());
+    if (c == 2 && !(A.below > -INFINITY)) c = 0;
+  }
+  A.cls[t] = (uint8_t)c;
+  if (!c) A.list[atomicAdd((unsigned long long *)A.cnt, 1ull)] = t;
+}
+
+__device__ __forceinline__ i64 band_owner(i64 i, i64 nb) { return i / R2S_BAND_B < nb - 1 ? i / R2S_BAND_B : nb - 1; }
+
+// one thread per point of planes [ka, kb): the fill value of a point whose owner is skipped
+__global__ void __launch_bounds__(256) k_band_fill(BandArgs A) {
+  const i64 t = blockIdx.x * (i64)blockDim.x + threadIdx.x, pl = A.n[0] * A.n[1];
+  if (t >= (A.kb - A.ka) * pl) return;
+  const i64 i = t % A.n[0], j = (t / A.n[0]) % A.n[1], k = A.ka + t / pl;
+  const uint8_t c = A.cls[band_owner(i, A.nb[0]) + A.nb[0] * (band_owner(j, A.nb[1]) + A.nb[1] * (band_owner(k, A.nb[2]) - A.lz0))];
+  if (c) A.out[t] = c == 1 ? A.iso : A.below;
+}
+
+// one CTA per sampled block: its closed box's points within planes [ka, kb) that it is the last sampled holder of
+__global__ void __launch_bounds__(256) k_band_sample(SampleGrid G, BandArgs A) {
+  constexpr int P = R2S_BAND_B + 1;
+  const i64 me = A.list[blockIdx.x];
+  const i64 b[3] = {me % A.nb[0], (me / A.nb[0]) % A.nb[1], A.lz0 + me / (A.nb[0] * A.nb[1])};
+  unsigned long long n = 0;
+  for (int q = threadIdx.x; q < P * P * P; q += blockDim.x) {
+    const i64 p[3] = {b[0] * R2S_BAND_B + q % P, b[1] * R2S_BAND_B + (q / P) % P, b[2] * R2S_BAND_B + q / (P * P)};
+    if (p[0] >= A.n[0] || p[1] >= A.n[1] || p[2] < A.ka || p[2] >= A.kb) continue;
+    // the blocks holding p, owner first per axis; the first sampled one in descending (z, y, x) order evaluates p
+    i64 c[3][2];
+    int nc[3];
+    for (int d = 0; d < 3; d++) {
+      c[d][0] = band_owner(p[d], A.nb[d]); nc[d] = 1;
+      if (p[d] % R2S_BAND_B == 0 && p[d] / R2S_BAND_B >= 1 && p[d] / R2S_BAND_B <= A.nb[d] - 1) c[d][nc[d]++] = p[d] / R2S_BAND_B - 1;
+    }
+    i64 first = -1;
+    for (int z = 0; z < nc[2] && first < 0; z++)
+      for (int y = 0; y < nc[1] && first < 0; y++)
+        for (int x = 0; x < nc[0] && first < 0; x++) {
+          const i64 id = c[0][x] + A.nb[0] * (c[1][y] + A.nb[1] * (c[2][z] - A.lz0));
+          if (!A.cls[id]) first = id;
+        }
+    if (first != me) continue;
+    const float x = smp_add(A.o[0], smp_mul((float)p[0], A.h[0])), y = smp_add(A.o[1], smp_mul((float)p[1], A.h[1]));
+    const float z = smp_add(A.o[2], smp_mul((float)p[2], A.h[2]));
+    SampleGrid g = G;
+    if (A.nslab > 1) { const int r = band_slab(G, A, z); g.w = A.tab[r].w; g.px = A.tab[r].px; }
+    A.out[((p[2] - A.ka) * A.n[1] + p[1]) * A.n[0] + p[0]] = sample_point<false>(g, x, y, z, nullptr);
+    n += p[2] < A.kown;
+  }
+  n = __reduce_add_sync(0xffffffffu, (unsigned)n);
+  if ((threadIdx.x & 31) == 0 && n) atomicAdd((unsigned long long *)A.cnt + 1, n);
+}
+
 __global__ void k_surf_totals(const i64 *vcnt, const i64 *tcnt, const i64 *vbase, const i64 *tbase, i64 nrows, i64 nown, const unsigned *bad, i64 *out) {
   out[0] = nown < nrows ? vbase[nown] : vbase[nrows - 1] + vcnt[nrows - 1];      // vertices of the owned rows
   out[1] = tbase[nrows - 1] + tcnt[nrows - 1];
@@ -331,13 +423,41 @@ int r2s_surf_emit(r2s_ctx *ctx, i64 vglob, i64 nv_total) {
 // planes above a chunk are the next chunk's first two: they move to the front of the buffer instead of being sampled again.
 #define SURF_LAT_BUDGET (1ll << 30)      // bytes of lattice values per chunk when R2S_SURF_PLANES is not set
 
-int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3]) {
+int r2s_surf_lattice_check(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, float o[3], float h[3],
+                           bool band) {
   if (!isfinite(iso)) FAIL("isosurface: iso must be finite");
   if (r2s_sample_lattice_check(ctx, origin, spacing, dims, o, h)) return 1;
   if (dims[0] < 2 || dims[1] < 2 || dims[2] < 2) FAIL("isosurface: the field needs at least 2 points per axis");
-  if ((dims[0] - 1) * (dims[1] - 1) * (dims[2] - 1) >= (1ll << 31)) FAIL("isosurface: 2^31 or more cells");
+  if (!band && (dims[0] - 1) * (dims[1] - 1) * (dims[2] - 1) >= (1ll << 31)) FAIL("isosurface: 2^31 or more cells");
   SampleGrid G;
   return r2s_sample_grid(ctx, &G, false);
+}
+
+// r2s_isosurface_band: the lattice planes [ka, kb) into out (plane ka first) -- classify the blocks of the layers holding them, fill the
+// points of skipped owners, evaluate the points the sampled blocks hold.  cnt[1] of ctx->surf_band counts the evaluations.
+static int band_planes(r2s_ctx *ctx, const SampleGrid &G, const SurfLattice &L, i64 ka, i64 kb, float *out) {
+  BandArgs A;
+  for (int d = 0; d < 3; d++) { A.o[d] = L.o[d]; A.h[d] = L.h[d]; A.n[d] = L.dims[d]; A.nb[d] = (L.dims[d] - 2) / R2S_BAND_B + 1; }
+  A.iso = L.iso; A.below = nextafterf(L.iso, -INFINITY);
+  A.ka = ka; A.kb = kb; A.kown = L.kb;
+  A.lz0 = std::min((ka > 0 ? ka - 1 : 0) / R2S_BAND_B, A.nb[2] - 1);      // plane ka also lies in the layer below when ka is a multiple of B
+  A.nblk = (std::min((kb - 1) / R2S_BAND_B, A.nb[2] - 1) - A.lz0 + 1) * A.nb[0] * A.nb[1];
+  A.nslab = (int)L.slabs.size(); A.tab = ctx->surf_wtab.as<SurfSlabW>();
+  A.cnt = ctx->surf_band.as<i64>(); A.list = A.cnt + 2; A.cls = (uint8_t *)(A.list + A.nblk);
+  A.out = out;
+  CK(cudaMemsetAsync(A.cnt, 0, sizeof(i64), ctx->stream));
+  k_band_classify<<<cdiv(A.nblk, 128), 128, 0, ctx->stream>>>(G, A);
+  LAUNCH_CHECK();
+  const i64 np = (kb - ka) * A.n[0] * A.n[1];
+  k_band_fill<<<cdiv(np, 256), 256, 0, ctx->stream>>>(A);
+  LAUNCH_CHECK();
+  i64 nact = 0;
+  if (r2s_readback(ctx, &nact, A.cnt, sizeof(i64))) return 1;
+  if (nact > 0) {
+    k_band_sample<<<(unsigned)nact, 256, 0, ctx->stream>>>(G, A);
+    LAUNCH_CHECK();
+  }
+  return 0;
 }
 
 static int lattice_sweep(r2s_ctx *ctx, bool emit, i64 vglob) {
@@ -359,20 +479,30 @@ static int lattice_sweep(r2s_ctx *ctx, bool emit, i64 vglob) {
     return r;
   };
   if (!emit) { L.cnv.clear(); L.cnt.clear(); }
+  if (L.band) {      // per chunk: its block layers' classes, list and two counters
+    const i64 nb = ((nx - 2) / R2S_BAND_B + 1) * ((ny - 2) / R2S_BAND_B + 1) * ((P + 2) / R2S_BAND_B + 2);
+    CK(ctx->surf_band.reserve(sizeof(i64) * (size_t)(nb + 2) + (size_t)nb));
+    CK(cudaMemsetAsync(ctx->surf_band.p, 0, 2 * sizeof(i64), ctx->stream));
+  }
   i64 have = L.ka, vb = 0, tb = 0;
   for (i64 c0 = L.ka, ci = 0; c0 < L.kb; c0 += P, ci++) {
     const i64 c1 = std::min(c0 + P, L.kb), need = std::min(c1 + 2, nz);
     // planes [c0, have) are the previous chunk's top planes, at buffer positions P + (k - c0): one plane per copy (no overlap for P = 1)
     for (i64 k = c0; k < have; k++)
       CK(cudaMemcpyAsync(buf + (k - c0) * pl, buf + (P + k - c0) * pl, sizeof(float) * (size_t)pl, cudaMemcpyDeviceToDevice, ctx->stream));
-    for (i64 k = std::max(have, c0); k < need;) {      // runs of planes read with the same slab's weights
-      const int r = slab_of(k);
-      i64 e = k + 1;
-      while (e < need && slab_of(e) == r) e++;
-      SampleGrid Gr = G;
-      Gr.w = L.slabs[(size_t)r].w; Gr.px = L.slabs[(size_t)r].px;
-      if (r2s_sample_lattice_dev(ctx, Gr, L.o, L.h, L.dims, k, e, buf + (k - c0) * pl)) return 1;
-      k = e;
+    const i64 k0 = std::max(have, c0);
+    if (L.band) {
+      if (k0 < need && band_planes(ctx, G, L, k0, need, buf + (k0 - c0) * pl)) return 1;
+    } else {
+      for (i64 k = k0; k < need;) {      // runs of planes read with the same slab's weights
+        const int r = slab_of(k);
+        i64 e = k + 1;
+        while (e < need && slab_of(e) == r) e++;
+        SampleGrid Gr = G;
+        Gr.w = L.slabs[(size_t)r].w; Gr.px = L.slabs[(size_t)r].px;
+        if (r2s_sample_lattice_dev(ctx, Gr, L.o, L.h, L.dims, k, e, buf + (k - c0) * pl)) return 1;
+        k = e;
+      }
     }
     have = need;
     const float *f = buf - c0 * pl;      // plane k of the chunk at f + k * pl (only planes [c0, need) are read)
@@ -400,6 +530,7 @@ static int lattice_sweep(r2s_ctx *ctx, bool emit, i64 vglob) {
   }
   CK(cudaStreamSynchronize(ctx->stream));
   if (!emit) { ctx->surf_nv = vb; ctx->surf_nt = tb; }
+  if (!emit && L.band && r2s_readback(ctx, &L.nsampled, ctx->surf_band.as<i64>() + 1, sizeof(i64))) return 1;
   return 0;
 }
 
@@ -591,13 +722,35 @@ int r2s_isosurface_lattice(r2s_ctx *ctx, const double origin[3], const double sp
   SurfLattice &L = ctx->surf_lat;
   if (r2s_surf_lattice_check(ctx, origin, spacing, dims, iso, L.o, L.h)) return 1;
   for (int d = 0; d < 3; d++) L.dims[d] = dims[d];
-  L.iso = iso; L.ka = 0; L.kb = dims[2];
+  L.iso = iso; L.ka = 0; L.kb = dims[2]; L.band = false;
   L.slabs.assign(1, SurfSlabW{INT64_MAX, ctx->rbf_w, (long long)ctx->rbf_px});
   i64 nv, nt;
   if (r2s_surf_lattice_count(ctx, &nv, &nt) || r2s_surf_lattice_emit(ctx, 0, nv)) return 1;
   ctx->surf_nv_all = nv; ctx->surf_nt_all = nt; ctx->surf_part = false;
   if (n_vertices) *n_vertices = nv;
   if (n_triangles) *n_triangles = nt;
+  return 0;
+}
+
+int r2s_isosurface_band(r2s_ctx *ctx, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
+                        int64_t *n_triangles, int64_t *n_sampled) {
+  if (!ctx) return 1;
+  ctx->have_surface = false;
+  if (ctx->nranks > 1)
+    FAIL(ctx->lg ? "r2s_isosurface_band: this context is one slab of an r2s_multi group; use r2s_multi_isosurface_band"
+                 : "r2s_isosurface_band: not available on a slab rank of the NCCL communicator (one process per GPU); extract on one context or with r2s_multi");
+  SurfLattice &L = ctx->surf_lat;
+  if (r2s_surf_lattice_check(ctx, origin, spacing, dims, iso, L.o, L.h, true)) return 1;
+  for (int d = 0; d < 3; d++) L.dims[d] = dims[d];
+  L.iso = iso; L.ka = 0; L.kb = dims[2]; L.band = true; L.nsampled = 0;
+  L.slabs.assign(1, SurfSlabW{INT64_MAX, ctx->rbf_w, (long long)ctx->rbf_px});
+  i64 nv, nt;
+  if (r2s_surf_lattice_count(ctx, &nv, &nt) || r2s_surf_lattice_emit(ctx, 0, nv)) { ctx->surf_band.release(); return 1; }
+  ctx->surf_band.release();
+  ctx->surf_nv_all = nv; ctx->surf_nt_all = nt; ctx->surf_part = false;
+  if (n_vertices) *n_vertices = nv;
+  if (n_triangles) *n_triangles = nt;
+  if (n_sampled) *n_sampled = L.nsampled;
   return 0;
 }
 

@@ -11,7 +11,7 @@ using Rho2sdf.MeshGrid: Mesh, Grid, generateGridPoints
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
-       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, isosurface_lattice, sample_sdf, sample_sdf_lattice, rbf_weights
+       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, isosurface_lattice, isosurface_band, sample_sdf, sample_sdf_lattice, rbf_weights
 
 const LIB = get(ENV, "R2S_LIBRARY", joinpath(@__DIR__, "..", "libr2s.so"))
 
@@ -249,6 +249,23 @@ function isosurface_lattice(m::MultiContext, origin::AbstractVector{<:Real}, spa
   V = Matrix{Float32}(undef, 3, nv[]); T = Matrix{Int32}(undef, 3, nt[])
   mcheck(m, ccall((:r2s_multi_download_isosurface, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Int32}), m.h, V, T))
   return V, T .+ Int32(1)
+end
+"""the mesh of isosurface_lattice, bit for bit, on lattices of any cell count, sampling only the lattice blocks that can hold the surface
+(include/r2s.h); returns (V, T, n_sampled), n_sampled the lattice points evaluated per sweep"""
+function isosurface_band(mesh::Mesh, origin::AbstractVector{<:Real}, spacing::AbstractVector{<:Real}, dims::NTuple{3,Int}; iso::Float32=0f0)
+  c = context(mesh); nv = Ref{Int64}(0); nt = Ref{Int64}(0); ns = Ref{Int64}(0)
+  check(c, ccall((:r2s_isosurface_band, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Cfloat, Ref{Int64}, Ref{Int64}, Ref{Int64}),
+                 c.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], iso, nv, nt, ns))
+  V, T = download_surface(c, nv[], nt[])
+  return V, T, ns[]
+end
+function isosurface_band(m::MultiContext, origin::AbstractVector{<:Real}, spacing::AbstractVector{<:Real}, dims::NTuple{3,Int}; iso::Float32=0f0)
+  nv = Ref{Int64}(0); nt = Ref{Int64}(0); ns = Ref{Int64}(0)
+  mcheck(m, ccall((:r2s_multi_isosurface_band, LIB), Cint, (Ptr{Cvoid}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Cfloat, Ref{Int64}, Ref{Int64}, Ref{Int64}),
+                  m.h, Vector{Float64}(origin), Vector{Float64}(spacing), Int64[dims...], iso, nv, nt, ns))
+  V = Matrix{Float32}(undef, 3, nv[]); T = Matrix{Int32}(undef, 3, nt[])
+  mcheck(m, ccall((:r2s_multi_download_isosurface, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Int32}), m.h, V, T))
+  return V, T .+ Int32(1), ns[]
 end
 "(weights on the coarse grid of `grid`, th): the definition of the continuous field"
 function rbf_weights(mesh::Mesh, grid)
