@@ -316,6 +316,35 @@ int r2s_isosurface_band(r2s_ctx *ctx, const double origin[3], const double spaci
 int r2s_multi_isosurface_band(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso,
                               int64_t *n_vertices, int64_t *n_triangles, int64_t *n_sampled);
 
+/* ---- the smoothed geometry on the FE mesh: per-element solid volume fractions (csrc/r2s_elemfrac.cu, r2s_elemfrac.cuh) -------------- */
+/* calculate_isocontour_volume's rule (Isocontour_volume.jl:1-75) -- a Heaviside at the Gauss points of an element, weighted by |det J| --
+ * applied to the continuous field f above (the field r2s_sample_sdf evaluates) on every element of the mesh of r2s_set_mesh.  Element e,
+ * quadrature order q = quad_order (1..32; 15 is the reference's order for crossing elements), nodes g and weights w of
+ * gauss_legendre(q), Gauss point t = (k q + j) q + i, i.e. ascending (k, j, i):
+ *   HEX8 (any trilinear element): x = sum_a N_a(g_i, g_j, g_k) X_a in double, W = ((w_i w_j) w_k) |det J|, with the shape functions and the
+ *     operation order of calculate_mesh_volume (r2s_mesh_volume), every operation rounded (no contraction).
+ *   TET4: the collapsed cube of calculate_mesh_volume, xi = (g_i + 1) / 2, eta = (g_j + 1) / 2 (1 - xi), zeta = (g_k + 1) / 2 (1 - xi - eta),
+ *     x = xi X_0 + eta X_1 + zeta X_2 + (1 - xi - eta - zeta) X_3, W = w_i w_j w_k |det J| (1 - xi) (1 - xi - eta) / 8 -- the geometrically
+ *     correct Duffy factor (sum W = |det J| / 6), NOT the reference's (1 - xi)^2 (1 - xi - eta) / 8 (MeshVolume.jl:107, 3/4 of the volume),
+ *     which would bias the ratio below.  So these V_e sum to the mesh volume, while r2s_mesh_volume's TET4 V_domain is 3/4 of it.
+ *   each point: p = float(x) per coordinate (sampler rule 1), f(p) by rules 2-5; the point is inside iff f >= iso (the corner rule of the
+ *     surface calls); a NaN value is outside.
+ *   each element: V_e = sum W and S_e = sum (inside ? W : +0) in one fixed order: 32 partials, partial l summing the points t = l mod 32 in
+ *     ascending t from +0, combined by p[l] += p[l + o] for o = 16, 8, 4, 2, 1 (l < o), the result p[0].  An element whose points are all
+ *     inside has S_e == V_e bit for bit, fraction exactly 1.  fractions[e] = S_e / V_e, and 0 when V_e == 0.
+ *   skipping: an element is never sampled when the block classifier of r2s_isosurface_band proves every Float32 value of its box on one
+ *     side of iso.  The box holds every p of the element's Gauss points: per axis [down(min_a X_a - s), up(max_a X_a + s)], s = 2^-40
+ *     max_a |X_a|, widened by one Float32 step (csrc/r2s_elemfrac.cuh gives the argument).  A skipped element's V_e is computed from the
+ *     geometry in the same order, and its fraction is exactly 1 or 0 -- the bits full evaluation gives; the results do not depend on it.
+ *   several slabs: the elements are split across the slabs; every Gauss point reads the weights of the slab owning its floor plane
+ *     (peer memory), so any split gives the bits of one context with the same weights.  An element whose box reaches the floor planes of
+ *     two slabs is always sampled.  Every slab writes its elements into the whole-mesh arrays.
+ * volumes (NULL or nel): V_e; n_evaluated (NULL or): the elements sampled (the others were skipped).  Needs a mesh and a smoothed field on the
+ * device; sdf_dists, fine_sdf, the weights, th and any surface are untouched.  Rejected with an error: quad_order outside 1..32, a non-finite
+ * iso, a NULL fractions, no mesh, no smoothed field; the single-context call fails on a slab rank of the NCCL communicator (use r2s_multi). */
+int r2s_element_volume_fractions(r2s_ctx *ctx, float iso, int quad_order, double *fractions, double *volumes, int64_t *n_evaluated);
+int r2s_multi_element_volume_fractions(r2s_multi *m, float iso, int quad_order, double *fractions, double *volumes, int64_t *n_evaluated);
+
 /* ---- measurement helper (bench.py): FMA-pipe peak of the device in TFLOP/s, fp64 != 0 -> double, else float -------- */
 int r2s_measure_fma_peak(r2s_ctx *ctx, int fp64, double *tflops);
 

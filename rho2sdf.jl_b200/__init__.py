@@ -30,7 +30,7 @@ __all__ = ["HEX8", "TET4", "Rho2sdfOptions", "Mesh", "Grid", "getMesh_AABB", "ge
            "remove_sdf_artifacts", "RBFs_smoothing", "calculate_volume_from_sdf", "rho2sdf", "rho2sdf_hex8", "rho2sdf_tet4",
            "exportSdfToVTI", "export_device_result_to_vti", "read_vti", "read_pvti",
            "isosurface", "isosurface_from_sdf", "isosurface_lattice", "isosurface_band", "export_isosurface", "read_stl", "read_ply",
-           "sample_sdf", "sample_sdf_lattice", "rbf_weights", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
+           "sample_sdf", "sample_sdf_lattice", "rbf_weights", "element_volume_fractions", "MultiContext", "FineGrid", "R2SError", "slab_partition", "init_slab_comm", "broadcast_unique_id", "load_library", "library_path", "Params", "Report", "Context"]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -149,6 +149,7 @@ def load_library():
     L.r2s_isosurface_band.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip, ip]
     L.r2s_multi_isosurface_band.argtypes = [vp, vp, vp, vp, C.c_float, ip, ip, ip]
     for pre in ("r2s_", "r2s_multi_"):
+        getattr(L, pre + "element_volume_fractions").argtypes = [vp, C.c_float, C.c_int, vp, vp, ip]
         getattr(L, pre + "sample_sdf").argtypes = [vp, vp, C.c_int64, vp, vp]
         getattr(L, pre + "sample_sdf_lattice").argtypes = [vp, vp, vp, vp, vp]
         getattr(L, pre + "download_rbf_weights").argtypes = [vp, vp, fp]
@@ -819,6 +820,22 @@ def rbf_weights(mesh):
     th = C.c_float()
     obj.check(getattr(obj.lib, pre + "download_rbf_weights")(obj.h, _ptr(w), C.byref(th)))
     return w, np.float32(th.value)
+
+
+def element_volume_fractions(mesh, iso=0.0, quad_order=15, return_volumes=False, stats=False):
+    """The solid volume fraction of every element of `mesh` in the continuous field of the last pipeline / smoothing call (what sample_sdf
+    evaluates): calculate_isocontour_volume's rule -- a Gauss point is solid iff f >= iso, weighted by |det J| -- at quad_order^3 points
+    per element (1..32), on the GPU.  Elements whose box the band classifier proves one-sided are not sampled; their fractions are exactly
+    1.0 or 0.0, the values full evaluation gives (include/r2s.h states the rule).  Returns fractions (nel,) float64; with return_volumes
+    also V_e (nel,), the element volumes of the same quadrature; with stats also the number of elements sampled."""
+    obj, pre = _sampler(mesh)
+    frac = np.empty(mesh.nel, dtype=np.float64)
+    vol = np.empty(mesh.nel, dtype=np.float64) if return_volumes else None
+    ne = C.c_int64()
+    obj.check(getattr(obj.lib, pre + "element_volume_fractions")(obj.h, float(iso), int(quad_order), _ptr(frac), _ptr(vol) if return_volumes else None,
+                                                                  C.byref(ne)))
+    out = (frac,) + ((vol,) if return_volumes else ()) + ((ne.value,) if stats else ())
+    return out if len(out) > 1 else frac
 
 
 # ---------------------------------------------------------------------------------------------------------------------

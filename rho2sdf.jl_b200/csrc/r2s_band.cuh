@@ -39,15 +39,12 @@ R2S_HD float band_up(double x) {        // the smallest float >= x
   return f;
 }
 
-// 0: sample, 1: every value of the box is >= iso, 2: every value is < iso.  lo / hi: the box's end lattice indices per axis (lo <= hi);
-// G: the weights every point of the box reads (one slab's)
-R2S_HD int band_classify(const SampleGrid &G, const float o[3], const float h[3], const long long lo[3], const long long hi[3], float iso, BandMargin M) {
+// 0: sample, 1: every value of the Float32 box [a_d, b_d] (a_d <= b_d) is >= iso, 2: every value is < iso.  G: the weights every point of
+// the box reads (one slab's).  The box form serves any set of points known to lie in the box (r2s_elemfrac.cuh: an element's Gauss points).
+R2S_HD int band_classify_box(const SampleGrid &G, const float a[3], const float b[3], float iso, BandMargin M) {
   if (!(fabsf(G.th) <= 0x1p126f)) return 0;
-  float a[3], b[3];
   int rl[3], rh[3], sl[3], sh[3];
   for (int d = 0; d < 3; d++) {
-    const float pa = smp_add(o[d], smp_mul((float)lo[d], h[d])), pb = smp_add(o[d], smp_mul((float)hi[d], h[d]));
-    a[d] = pa < pb ? pa : pb; b[d] = pa < pb ? pb : pa;
     const int fa = smp_floor(G.C[d], G.n[d], G.c0[d], G.inv[d], a[d]), fb = smp_floor(G.C[d], G.n[d], G.c0[d], G.inv[d], b[d]);
     rl[d] = fa - 2 < 0 ? 0 : fa - 2; rh[d] = fb + 3 > G.n[d] - 1 ? G.n[d] - 1 : fb + 3;
     sl[d] = fb - 2; sh[d] = fa + 3;
@@ -79,4 +76,14 @@ R2S_HD int band_classify(const SampleGrid &G, const float o[3], const float h[3]
   if (!neg && (G.th >= iso || smp_add(band_down(s), G.th) >= iso)) return 1;
   if (!pos && (G.th < iso || smp_add(band_up(-s), G.th) < iso)) return 2;
   return 0;
+}
+
+// the lattice form: lo / hi are the box's end lattice indices per axis (lo <= hi) of the lattice o + float(i) h
+R2S_HD int band_classify(const SampleGrid &G, const float o[3], const float h[3], const long long lo[3], const long long hi[3], float iso, BandMargin M) {
+  float a[3], b[3];
+  for (int d = 0; d < 3; d++) {
+    const float pa = smp_add(o[d], smp_mul((float)lo[d], h[d])), pb = smp_add(o[d], smp_mul((float)hi[d], h[d]));
+    a[d] = pa < pb ? pa : pb; b[d] = pa < pb ? pb : pa;
+  }
+  return band_classify_box(G, a, b, iso, M);
 }

@@ -259,6 +259,10 @@ int r2s_sample_download_weights(r2s_ctx *ctx, float *w, float *th, i64 k0, i64 k
 // r2s_points.cu: evalDistances / Sign_Detection at n host points (rho_n on the host)
 int r2s_points_distances(r2s_ctx *ctx, const double *rho_n, double rho_t, double delta_factor, const double *pts, i64 n, double *dist, double *xp);
 int r2s_points_signs(r2s_ctx *ctx, const double *rho_n, double rho_t, const double *pts, i64 n, double *signs);
+// r2s_elemfrac.cu: per-element volume fractions of the continuous field; the checks of both entry points, and the elements [e0, e1) of one
+// context (every point reads the weights of the slab of slabs owning its floor plane) into host arrays indexed by e - e0
+int r2s_ef_check(r2s_ctx *ctx, float iso, int quad_order, const double *fractions);
+int r2s_ef_range(r2s_ctx *ctx, const std::vector<SurfSlabW> &slabs, i64 e0, i64 e1, float iso, int quad_order, double *frac, double *vol, i64 *nev);
 // in-process groups (r2s_multi.cu drives them): one context per slab, one host thread per context
 LocalGroup *r2s_local_group_create(r2s_ctx **ctxs, int n, std::string *err);
 void r2s_local_group_destroy(LocalGroup *g);

@@ -193,27 +193,6 @@ extern "C" int r2s_mesh_is_lattice(r2s_ctx *ctx, int *is_lattice) {
   return 0;
 }
 
-// ---------------------------------------------------------------------------------------------------------------
-// shape functions in the reference's form (ShapeFunctions/hex8_shape.jl:2-70); this TU is built with -fmad=false
-// ---------------------------------------------------------------------------------------------------------------
-__device__ inline void hex8_shape_d(const double xi[3], double N[8], double dN[8][3]) {
-  double m1 = xi[0] - 1, p1 = xi[0] + 1, m2 = xi[1] - 1, p2 = xi[1] + 1, m3 = xi[2] - 1, p3 = xi[2] + 1;
-  double t1 = m1 * m2, t2 = p1 * m2, t3 = p1 * p2, t4 = m1 * p2, c = 0.125;
-  N[0] = -c * t1 * m3; N[1] = c * t2 * m3; N[2] = -c * t3 * m3; N[3] = c * t4 * m3;
-  N[4] = c * t1 * p3;  N[5] = -c * t2 * p3; N[6] = c * t3 * p3; N[7] = -c * t4 * p3;
-  double d = c * m3, dp = c * p3;
-  dN[0][0] = -d * m2; dN[1][0] = d * m2; dN[2][0] = -d * p2; dN[3][0] = d * p2;
-  dN[4][0] = dp * m2; dN[5][0] = -dp * m2; dN[6][0] = dp * p2; dN[7][0] = -dp * p2;
-  dN[0][1] = -d * m1; dN[1][1] = d * p1; dN[2][1] = -d * p1; dN[3][1] = d * m1;
-  dN[4][1] = dp * m1; dN[5][1] = -dp * p1; dN[6][1] = dp * p1; dN[7][1] = -dp * m1;
-  dN[0][2] = -c * t1; dN[1][2] = c * t2; dN[2][2] = -c * t3; dN[3][2] = c * t4;
-  dN[4][2] = c * t1;  dN[5][2] = -c * t2; dN[6][2] = c * t3;  dN[7][2] = -c * t4;
-}
-__device__ inline double det3(const double J[3][3]) {
-  return J[0][0] * (J[1][1] * J[2][2] - J[1][2] * J[2][1]) - J[0][1] * (J[1][0] * J[2][2] - J[1][2] * J[2][0]) +
-         J[0][2] * (J[1][0] * J[2][1] - J[1][1] * J[2][0]);
-}
-
 // deterministic sum: per-block partials in a fixed slot, summed in slot order by one thread
 __global__ void k_sum_partials(const double *__restrict__ part, int n, int stride, double *__restrict__ out) {
   if (threadIdx.x == 0 && blockIdx.x == 0)

@@ -297,6 +297,15 @@ int r2s_multi_download_rbf_weights(r2s_multi *m, float *weights, float *th) {
   return run_all(m, [&](int r) { return r2s_sample_download_weights(m->ctx[(size_t)r], weights, r == 0 ? th : nullptr, m->cut[(size_t)r], m->cut[(size_t)r + 1]); });
 }
 
+// every slab's weights and the coarse planes below which they serve a point (its floor plane's owner), for the kernels that route each
+// evaluation to the weights r2s_multi_sample_sdf would use
+static std::vector<SurfSlabW> slab_weights(const r2s_multi *m) {
+  std::vector<SurfSlabW> slabs((size_t)m->n);
+  for (int q = 0; q < m->n; q++)
+    slabs[(size_t)q] = SurfSlabW{q + 1 < m->n ? m->cut[(size_t)q + 1] : (i64)INT64_MAX, m->ctx[(size_t)q]->rbf_w, (long long)m->ctx[(size_t)q]->rbf_px};
+  return slabs;
+}
+
 // Zero surface of the continuous field on a lattice (r2s_surf.cu): every slab extracts the lattice planes r2s_multi_sample_sdf_lattice
 // gives it (a contiguous run, since the plane z is monotone in k), reading the two planes above its run -- and every snapping evaluation
 // -- with the weights of the slab owning the point's floor plane, through peer memory (plain pointers on a shared device).  The weights
@@ -336,9 +345,7 @@ static int multi_lattice_surface(r2s_multi *m, const double origin[3], const dou
     }
     kb[(size_t)r] = k + 1; prev = r;
   }
-  std::vector<SurfSlabW> slabs((size_t)m->n);
-  for (int q = 0; q < m->n; q++)
-    slabs[(size_t)q] = SurfSlabW{q + 1 < m->n ? m->cut[(size_t)q + 1] : (i64)INT64_MAX, m->ctx[(size_t)q]->rbf_w, (long long)m->ctx[(size_t)q]->rbf_px};
+  const std::vector<SurfSlabW> slabs = slab_weights(m);
   for (int r = 0; r < m->n; r++) {
     SurfLattice &L = m->ctx[(size_t)r]->surf_lat;
     for (int d = 0; d < 3; d++) { L.o[d] = o[d]; L.h[d] = h[d]; L.dims[d] = dims[d]; }
@@ -381,6 +388,34 @@ int r2s_multi_isosurface_lattice(r2s_multi *m, const double origin[3], const dou
 int r2s_multi_isosurface_band(r2s_multi *m, const double origin[3], const double spacing[3], const int64_t dims[3], float iso, int64_t *n_vertices,
                               int64_t *n_triangles, int64_t *n_sampled) {
   return multi_lattice_surface(m, origin, spacing, dims, iso, n_vertices, n_triangles, true, n_sampled);
+}
+
+// Per-element volume fractions (r2s_elemfrac.cu): the elements are cut into n contiguous ranges, one per slab; every Gauss point reads the
+// weights of the slab owning its floor plane through peer memory, so the result does not depend on the cut.  Each slab writes its range of
+// the caller's whole-mesh arrays.
+int r2s_multi_element_volume_fractions(r2s_multi *m, float iso, int quad_order, double *fractions, double *volumes, int64_t *n_evaluated) {
+  if (!m) return 1;
+  if (m->n == 1) {
+    const int rc = r2s_element_volume_fractions(m->ctx[0], iso, quad_order, fractions, volumes, n_evaluated);
+    if (rc) m->err = m->ctx[0]->err;
+    return rc;
+  }
+  if (r2s_ef_check(m->ctx[0], iso, quad_order, fractions)) { m->err = m->ctx[0]->err; return 1; }
+  SampleGrid G;
+  if (multi_sample_ready(m, &G)) return 1;
+  const std::vector<SurfSlabW> slabs = slab_weights(m);
+  const i64 nel = m->ctx[0]->nel;
+  std::vector<i64> nev((size_t)m->n, 0);
+  if (run_all(m, [&](int r) {
+        const i64 e0 = nel * r / m->n, e1 = nel * (r + 1) / m->n;
+        return r2s_ef_range(m->ctx[(size_t)r], slabs, e0, e1, iso, quad_order, fractions + e0, volumes ? volumes + e0 : nullptr, &nev[(size_t)r]);
+      }))
+    return 1;
+  if (n_evaluated) {
+    *n_evaluated = 0;
+    for (int r = 0; r < m->n; r++) *n_evaluated += nev[(size_t)r];
+  }
+  return 0;
 }
 
 int r2s_multi_export_isosurface(r2s_multi *m, const char *path, int format) {

@@ -11,7 +11,8 @@ using Rho2sdf.MeshGrid: Mesh, Grid, generateGridPoints
 using Rho2sdf.ElementTypes: AbstractElement, HEX8, TET4
 
 export rho2sdf, rho2sdf_hex8, rho2sdf_tet4, evalDistances, Sign_Detection, remove_sdf_artifacts!, RBFs_smoothing,
-       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, isosurface_lattice, isosurface_band, sample_sdf, sample_sdf_lattice, rbf_weights
+       DenseInNodes, find_threshold_for_volume, calculate_volume_from_sdf, isosurface, export_isosurface, isosurface_lattice, isosurface_band, sample_sdf, sample_sdf_lattice, rbf_weights,
+       element_volume_fractions
 
 const LIB = get(ENV, "R2S_LIBRARY", joinpath(@__DIR__, "..", "libr2s.so"))
 
@@ -266,6 +267,20 @@ function isosurface_band(m::MultiContext, origin::AbstractVector{<:Real}, spacin
   V = Matrix{Float32}(undef, 3, nv[]); T = Matrix{Int32}(undef, 3, nt[])
   mcheck(m, ccall((:r2s_multi_download_isosurface, LIB), Cint, (Ptr{Cvoid}, Ptr{Cfloat}, Ptr{Int32}), m.h, V, T))
   return V, T .+ Int32(1), ns[]
+end
+"""solid volume fraction of every element of `mesh` in the continuous field (calculate_isocontour_volume's rule at quad_order^3 Gauss points
+per element, a point solid iff f >= iso; include/r2s.h): (fractions, volumes V_e, elements sampled); a MultiContext takes the element count"""
+function element_volume_fractions(mesh::Mesh; iso::Float32=0f0, quad_order::Int=15)
+  c = context(mesh); frac = Vector{Float64}(undef, mesh.nel); vol = Vector{Float64}(undef, mesh.nel); ne = Ref{Int64}(0)
+  check(c, ccall((:r2s_element_volume_fractions, LIB), Cint, (Ptr{Cvoid}, Cfloat, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Int64}),
+                 c.h, iso, quad_order, frac, vol, ne))
+  return frac, vol, ne[]
+end
+function element_volume_fractions(m::MultiContext, nel::Integer; iso::Float32=0f0, quad_order::Int=15)
+  frac = Vector{Float64}(undef, nel); vol = Vector{Float64}(undef, nel); ne = Ref{Int64}(0)
+  mcheck(m, ccall((:r2s_multi_element_volume_fractions, LIB), Cint, (Ptr{Cvoid}, Cfloat, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Int64}),
+                  m.h, iso, quad_order, frac, vol, ne))
+  return frac, vol, ne[]
 end
 "(weights on the coarse grid of `grid`, th): the definition of the continuous field"
 function rbf_weights(mesh::Mesh, grid)
